@@ -12,6 +12,10 @@ arrays and one 200-epoch call beside it), i.e. H2D of ratings + factors, layout,
 of the factors inside the timed region.  At N > 1 the line's value is STRONG scaling (the same
 100M-rating problem cut into N user slices, with a parity block against the one-GPU run); the
 weak-scaling run is the secondary key ``weak``.  One JSON line on stdout (rank 0).
+``--dump-outputs DIR`` also writes what the last timed step returned as ``.npy`` files (the model
+after the last epoch; with ``--workload topn`` the last call's items and scores); the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.  It needs
+``--gpus 1``: the ring at N > 1 leaves the model spread over the ranks and is not dumped.
 """
 import argparse
 import functools
@@ -318,6 +322,8 @@ def run_native(args):
     ms_per_step = ms / args.steps
     value = nnz * args.steps / (ms * 1e-3)
     rmse_curve = torch.sqrt(se / nnz).cpu().numpy().tolist()
+    if args.dump_outputs:
+        dump_model(args.dump_outputs, M, se[-1].item())
 
     peak, peak_src = measured_peaks()
     bpu = algorithmic_bytes_per_update(k)
@@ -460,6 +466,34 @@ def run_native(args):
            "gpu_launches": int(launches_timed), "clocks": clk,
            "rmse_per_epoch": rmse_curve, "setup_s": time.time() - t_setup}
     return out
+
+
+DUMP_BYTES = 60 << 20   # all .npy files of one --dump-outputs together (under 64 MB)
+
+
+def dump_ids(n, bytes_per_id, budget):
+    """Ids 0 .. n-1, or a fixed, seeded, sorted sample of them when n ids would exceed the budget."""
+    cap = budget // bytes_per_id
+    return np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+
+
+def write_dump(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
+def dump_model(out_dir, M, sq_err_last):
+    """--dump-outputs: what a caller of the timed path receives after its last step, i.e. the model
+    as mfrec_model_read returns it (item / user factors [k, n] and biases) and the sum of squared
+    errors of that epoch.  A side with more columns than half the budget holds is written as a
+    sample of columns; <side>_ids holds the column ids written, sampled or not."""
+    u, v, ib, ub = M.read()
+    arrays = {"sq_err": np.array([sq_err_last])}
+    for side, f, b in (("item", u, ib), ("user", v, ub)):
+        ids = dump_ids(f.shape[1], (f.shape[0] + 2) * 8, DUMP_BYTES // 2)
+        arrays.update({side + "_factors": f[:, ids], side + "_bias": b[ids], side + "_ids": ids})
+    write_dump(out_dir, arrays)
 
 
 def ctx_sm_count(ctx):
@@ -688,6 +722,11 @@ def run_topn(args, ctx=None):
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
         clocks.end()
+    if getattr(args, "dump_outputs", None):
+        # the last call's result (items -1 padded, scores, counts) for a sample of users
+        ids = dump_ids(nu, (2 * N + 2) * 8, DUMP_BYTES)
+        write_dump(args.dump_outputs, {"topn_items": out[0][ids], "topn_scores": out[1][ids],
+                                       "topn_counts": out[2][ids], "topn_user_ids": ids})
     flops = 2.0 * nu * ni * k
     sm = float(np.mean(sweep_ms))
     peaks = {}
@@ -840,7 +879,15 @@ def main():
                          "weak = one tile per GPU (secondary key); both = strong line + `weak` key")
     ap.add_argument("--emulate-slabs", type=int, default=1,
                     help="debug: run one rank's share of a G-GPU ring on one GPU (no exchange)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step returned (the model and its squared-error "
+                         "sum; top-N: items and scores) as DIR/<name>.npy (float64, < 64 MB: large outputs as a "
+                         "seeded sample); --gpus 1 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.gpus != 1):
+        ap.error("--dump-outputs needs the native path on one GPU (--gpus 1)")
     # exactly ONE line on stdout: libraries print banners there (e.g. "NCCL version ..." at the
     # first communicator), so everything but the final JSON line is sent to stderr
     sys.stdout.flush()

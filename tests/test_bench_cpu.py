@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -21,6 +23,16 @@ def test_reference_arm_prints_the_contract_line():
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] == 1
     assert d["e2e"] == {"value": d["value"], "unit": "updates/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and "model" not in d["config"]
+
+
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "DIR"],
+                                   ["--gpus", "2", "--dump-outputs", "DIR"]])
+def test_arguments_the_bench_cannot_honour_are_refused(extra, tmp_path):
+    extra = [str(tmp_path / "dump") if a == "DIR" else a for a in extra]
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, stdout=subprocess.PIPE,
+                         stderr=subprocess.PIPE, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode == 2 and "error:" in out.stderr and out.stdout == "", out.stderr[-500:]
+    assert not (tmp_path / "dump").exists()
 
 
 def test_reference_arm_other_ranks_exit_quietly():

@@ -155,6 +155,63 @@ __device__ __forceinline__ int mfrec_window_levels(int user, int item, bool live
     lmax = __reduce_max_sync(full, live ? level : 0);
     return level;
 }
+
+// ---- PTX helpers: mbarrier + bulk async copy (TMA, non-tensor form) -------------------------------
+__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count)
+{
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
+}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
+{
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
+{
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "WAIT_%=:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
+        "@p bra DONE_%=;\n"
+        "bra WAIT_%=;\n"
+        "DONE_%=:\n"
+        "}\n" ::"r"(smem_u32(bar)),
+        "r"(parity)
+        : "memory");
+}
+__device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes, uint64_t *bar)
+{
+    asm volatile(
+        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
+        "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
+        : "memory");
+}
+
+// ---- hand-over counters between CTAs of one device (release / acquire at gpu scope) ----------------
+__device__ __forceinline__ int ld_acquire_gpu(const int32_t *p)
+{
+    int v;
+    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_release_gpu(int32_t *p, int v)
+{
+    asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+
+// ---- score order key of the top-N paths (topn.cu, topn_tc.cu) ---------------------------------------
+// monotone map float -> uint32 (larger float -> larger uint) and its inverse
+__device__ __forceinline__ uint32_t order_bits(float x)
+{
+    const uint32_t b = __float_as_uint(x);
+    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+__device__ __forceinline__ float unorder_bits(uint32_t k)
+{
+    const uint32_t b = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
+    return __uint_as_float(b);
+}
 #endif
 
 // ---- error plumbing -------------------------------------------------------------------

@@ -73,17 +73,6 @@ struct FunkParams {
     int update_users, update_items;
 };
 
-__device__ __forceinline__ int funk_ld_acquire(const int32_t *p)
-{
-    int v;
-    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void funk_st_release(int32_t *p, int v)
-{
-    asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
 // One launch = sub-epochs [s_begin, s_end) of one training pass.  With `ticks` the launch is
 // persistent and cooperative (all B sub-epochs): column blocks pass from CTA to CTA through
 // release / acquire counters exactly as in sgd.cu, instead of one kernel boundary per sub-epoch,
@@ -98,10 +87,7 @@ __device__ __forceinline__ void funk_st_release(int32_t *p, int v)
 // (Round 2, profiles/r02m_funk_full.md: replaying the 32 ratings of a batch one after the other,
 // every lane computing the same scalar update, was 57 warp instructions and ~360 cycles per
 // rating: 5.3 ms per 20 M-rating pass.)
-#ifndef MFREC_FUNK_DEEP_DIV
-#define MFREC_FUNK_DEEP_DIV 2
-#endif
-constexpr int kDeepDiv = MFREC_FUNK_DEEP_DIV;   // a batch with more than cnt / kDeepDiv levels is replayed serially
+constexpr int kDeepDiv = 2;   // a batch with more than cnt / kDeepDiv levels is replayed serially
 
 struct FunkStage {          // one staged rating of a deep batch, 32 bytes
     int u, i;               // user / item index relative to the row block / column block
@@ -164,7 +150,7 @@ __global__ void __launch_bounds__(512) funk_train_kernel(const FunkParams prm)
             if (i < W * W) bcnt[i] = prm.bucket_cnt[bucket_base + i];
         }
         if (prm.ticks && threadIdx.x == 0)
-            while (funk_ld_acquire(prm.ticks + cbl) < s) __nanosleep(64);
+            while (ld_acquire_gpu(prm.ticks + cbl) < s) __nanosleep(64);
         __syncthreads();   // the column block is ours; descriptors (and, first time, vfs) visible
         // item scalars: L2 loads (another SM wrote them; L1 may hold a stale line)
         for (int i = threadIdx.x; i < nq; i += blockDim.x) {
@@ -331,7 +317,7 @@ __global__ void __launch_bounds__(512) funk_train_kernel(const FunkParams prm)
         if (prm.ticks) {
             __threadfence();
             __syncthreads();
-            if (threadIdx.x == 0) funk_st_release(prm.ticks + cbl, s + 1);
+            if (threadIdx.x == 0) st_release_gpu(prm.ticks + cbl, s + 1);
         } else {
             __syncthreads();
         }

@@ -10,8 +10,8 @@
 //   bucket(slab g, row block rb, column block cb, phase p, worker w) holds the ratings of
 //   row group (rb, w) x column group (cb, (w + p) mod W), sorted by (user, item) so that
 //   ratings of one user are adjacent (sgd.cu keeps that user's row in registers).  (A bucket is
-//   one warp's serial work, so any order inside it is legal; MFREC_PACK_ORDER=dealt is the
-//   experiment that deals item-sorted ratings over the quads instead, see below.)
+//   one warp's serial work, so any order inside it is legal; see the key layout below for the
+//   order that was measured against this one.)
 //   Buckets are stored in (g, rb, cb, w, p) order -- worker-major, so the W buckets one warp
 //   walks through are one contiguous stream -- each starting on a 16-byte boundary so the
 //   warp can pull the stream through shared memory with cp.async.bulk.
@@ -58,7 +58,6 @@ __global__ void degree_kernel(const int32_t *__restrict__ idx, int64_t nnz, int3
 struct KeyLayout {
     int bits_i, bits_u, bits_b;
     int W, B;
-    int dealt;   // 1: bucket order = (item, user)-sorted ratings dealt over the quads; 0: sorted by (user, item)
 };
 
 // which copy of a split item a user's rating trains (any fixed function of the user will do: the
@@ -95,9 +94,7 @@ __global__ void key_kernel(const int32_t *__restrict__ idx, int64_t nnz,
         const uint64_t bucket =
             ((((uint64_t)slab * kl.B + rb) * kl.B + cbl) * kl.W + wr) * kl.W + p;
         const uint64_t pu = (uint32_t)user_perm[ui.x], pi = (uint32_t)item_perm[ui.y];
-        keys[n] = (bucket << (kl.bits_u + kl.bits_i)) |
-                  (kl.dealt ? (pi << kl.bits_u) | pu     // bucket, then item, then user
-                            : (pu << kl.bits_i) | pi);   // bucket, then user, then item
+        keys[n] = (bucket << (kl.bits_u + kl.bits_i)) | (pu << kl.bits_i) | pi;   // bucket, then user, then item
         vals[n] = (uint32_t)n;
     }
 }
@@ -125,19 +122,6 @@ __global__ void pad_counts_kernel(const int32_t *__restrict__ cnt, int64_t nb,
     if ((threadIdx.x & 31) == 0 && c > 0) atomicMax(widest, c);
 }
 
-// Position of the rating with sorted rank l (by item, then user) inside its bucket of n ratings.
-// The bucket is one warp's serial work, so ANY order of its ratings is a legal SGD order; the
-// order that lets the kernel overlap the most is the one where neighbouring ratings share neither
-// user nor item (sgd.cu applies such an aligned group of four side by side).  The item-sorted
-// ratings are therefore dealt round-robin over the bucket's s = n / 4 full quads: rank l goes to
-// quad l mod s, so an item with up to s ratings in the bucket appears at most once per quad
-// (and its users are distinct anyway).  The n mod 4 leftovers close the bucket.
-__device__ __forceinline__ int64_t dealt_position(int64_t l, int64_t n)
-{
-    const int64_t s = n >> 2;
-    return l < 4 * s ? (l % s) * 4 + l / s : l;
-}
-
 constexpr int32_t kTmpFirst = 1 << 30;   // .u, only between gather_kernel and hint_kernel: first rating of its bucket
 
 template <typename RT>
@@ -153,12 +137,11 @@ __global__ void gather_kernel(const uint64_t *__restrict__ keys, const uint32_t 
         const uint64_t key = keys[s];
         const uint32_t src = vals[s];
         const uint64_t b = key >> (kl.bits_u + kl.bits_i);
-        const int64_t first = raw_off[b], n = raw_off[b + 1] - first;
-        const int64_t at = kl.dealt ? dealt_position(s - first, n) : s - first;
+        const int64_t at = s - raw_off[b];
         const int64_t dst = pad_off[b] + at;
         PackedRating pr;
-        pr.u = (int32_t)(kl.dealt ? key & mask_u : (key >> kl.bits_i) & mask_u) | (at == 0 ? kTmpFirst : 0);
-        pr.i = (int32_t)(kl.dealt ? (key >> kl.bits_u) & mask_i : key & mask_i);
+        pr.u = (int32_t)((key >> kl.bits_i) & mask_u) | (at == 0 ? kTmpFirst : 0);
+        pr.i = (int32_t)(key & mask_i);
         pr.r = (float)ratings[src];
         packed[dst] = pr;
         if (order) order[dst] = (int64_t)src;
@@ -492,9 +475,7 @@ extern "C" int mfrec_ratings_pack(mfrec_ctx *ctx, const int32_t *ratings_index, 
         const int64_t min_copy = (opts && opts->split_min_copy > 0) ? opts->split_min_copy : 1024;
         double tot = 0.0;
         for (int32_t i = 0; i < ni; ++i) tot += (double)h_deg_i[i];
-        static double tau_frac = -1.0;   // MFREC_SPLIT_TAU: experiments with the threshold (fraction of a column group)
-        if (tau_frac < 0) tau_frac = getenv("MFREC_SPLIT_TAU") ? atof(getenv("MFREC_SPLIT_TAU")) : 0.5;
-        const double tau = std::max(1.0, tau_frac * tot / ((double)G * B * W));
+        const double tau = std::max(1.0, 0.5 * tot / ((double)G * B * W));   // half a column group's share
         for (int32_t i = 0; i < ni; ++i) {
             int64_t copies = 1;
             if (split != MFREC_SPLIT_OFF && (double)h_deg_i[i] > tau) {
@@ -562,16 +543,10 @@ extern "C" int mfrec_ratings_pack(mfrec_ctx *ctx, const int32_t *ratings_index, 
     kl.bits_b = bits_for(R->n_buckets);
     kl.W = W;
     kl.B = B;
-    {
-        // Order inside a bucket.  Sorted by (user, item): a user's ratings are adjacent and its row
-        // stays in registers.  "Dealt" (MFREC_PACK_ORDER=dealt): item-sorted ratings dealt round-robin
-        // over the quads -- more independent quads, but a user with several ratings in the bucket
-        // then recurs inside the prefetch window and takes the slow (re-read) path; measured slower
-        // on skewed data (21.4 vs 15.7 ms per epoch at Netflix shape).
-        static int dealt_env = -1;
-        if (dealt_env < 0) dealt_env = (getenv("MFREC_PACK_ORDER") && !strcmp(getenv("MFREC_PACK_ORDER"), "dealt")) ? 1 : 0;
-        kl.dealt = dealt_env;
-    }
+    // Order inside a bucket: sorted by (user, item), so a user's ratings are adjacent and its row
+    // stays in registers.  Item-sorted ratings dealt round-robin over the quads give more
+    // independent quads but were slower, because a user then recurs inside the prefetch window
+    // (21.4 vs 15.8 ms per epoch at Netflix shape, profiles/r02h_pack_order_dealt.log).
     if (kl.bits_i + kl.bits_u + kl.bits_b > 64)
         return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED,
                                "mfrec_ratings_pack: sort key needs %d bits", kl.bits_i + kl.bits_u + kl.bits_b);

@@ -50,14 +50,8 @@
 namespace {
 
 constexpr int kChunk = 64;    // ratings per TMA chunk
-#ifndef MF_KSTAGES
-#define MF_KSTAGES 4
-#endif
-#ifndef MF_KDEPTH
-#define MF_KDEPTH 16
-#endif
-constexpr int kStages = MF_KSTAGES;   // chunks in flight per warp (ring of kStages * kChunk ratings)
-constexpr int kDepth = MF_KDEPTH;     // P rows in flight per warp (cp.async ring), in stream positions
+constexpr int kStages = 4;    // chunks in flight per warp (ring of kStages * kChunk ratings)
+constexpr int kDepth = 16;    // P rows in flight per warp (cp.async ring), in stream positions
 constexpr int kQuadsAhead = kDepth / 4;
 constexpr int kRing = kChunk * kStages;
 static_assert(kChunk % 4 == 0, "chunks must be 16-byte multiples");
@@ -94,49 +88,10 @@ struct SgdParams {
     float lr, Ku, Ki, Kb;
     int update_users, update_items;
     float fx_scale, fx_inv;       // fixed-point scale of the warp reduction (power of two)
-    unsigned long long *timing;   // debug (MFREC_SGD_TIMING=1): [B][W][8] cycle counters, or null
-    int exp;                      // debug (MFREC_SGD_EXP, timing build only): knock-out experiments, results are WRONG
     unsigned long long wait_ns;   // ring: give up a hand-over wait after this long (0 = never)
 };
 
-// ---- PTX helpers: mbarrier + bulk async copy (TMA, non-tensor form) + cp.async ------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p)
-{
-    return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)),
-                 "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes,
-                                         uint64_t *bar)
-{
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-            smem_u32(dst_smem)),
-        "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-        : "memory");
-}
+// ---- PTX helpers: cp.async (mbarrier and bulk-copy helpers: common.cuh) -------------------
 template <int BYTES>
 __device__ __forceinline__ void cp_async(void *dst_smem, const void *src_gmem)
 {
@@ -206,16 +161,6 @@ __device__ __forceinline__ void frag_store_lane(const Frag<E> &f, float *p)
         else
             *p = f.x[0];
     }
-}
-
-// asynchronous global -> shared copy of one row, same lane <-> column mapping as frag_load
-template <int E>
-__device__ __forceinline__ void row_cp_async(float *dst_row, const float *src_row, int lane)
-{
-    constexpr int V = Frag<E>::V, NV = Frag<E>::NV;
-#pragma unroll
-    for (int c = 0; c < NV; ++c)
-        cp_async<V * 4>(dst_row + (c * 32 + lane) * V, src_row + (c * 32 + lane) * V);
 }
 
 // base + idx * stride as ONE 64-bit multiply-add (the compiler otherwise splits the masked id into
@@ -317,24 +262,8 @@ __device__ __forceinline__ unsigned long long fma2(unsigned long long a, unsigne
     return r;
 }
 
-__device__ __forceinline__ float warp_sum(float v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
-__device__ __forceinline__ int ld_acquire_gpu(const int32_t *p)
-{
-    int v;
-    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release_gpu(int32_t *p, int v)
-{
-    asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
 // system scope: the counter (and the data it guards) was written by / is read by another GPU
+// (the gpu-scope pair is in common.cuh)
 __device__ __forceinline__ int ld_acquire_sys(const int32_t *p)
 {
     int v;
@@ -385,7 +314,7 @@ __device__ __forceinline__ unsigned long long global_ns()
 // takes the generic path, which picks each row's source (registers / prefetch ring / global
 // memory) with warp-uniform branches.
 // ------------------------------------------------------------------------------------------
-template <int E, int KERNEL, bool TIMING, int MAXT, bool GATED, bool RING, typename PT = float>
+template <int E, int KERNEL, int MAXT, bool GATED, bool RING, typename PT = float>
 // MAXT: 256 (W <= 8: 255 registers per thread), 384 or 512; GATED: honour update_users /
 // update_items (else both on); RING: slabs move between ranks (DSGD), counters and hand-over at
 // system scope; PT: storage type of the user-factor rows in HBM (float, __half, __nv_bfloat16)
@@ -448,18 +377,6 @@ sgd_block_kernel(const SgdParams prm)
     uint32_t chunk_seq = 0;   // chunks this warp has pulled so far (ring stage + mbarrier parity)
     uint32_t tile_seq = 0;    // Q tiles this CTA has pulled so far (mbarrier parity)
     bool chunks_issued = false;   // the first chunks of the coming sub-epoch are already on their way
-    // opt-in section timer (cycles per warp): 0 bookkeeping + prefetch issue, 1 cp.async wait,
-    // 2 quad load, 3 updates, 4 phase hand-over wait, 5 sub-epoch set-up (ticket + tile), 6 tail
-    unsigned long long tsec[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    long long tmark = 0;
-    if constexpr (TIMING) tmark = clock64();
-    auto lap = [&](int k) {
-        if constexpr (TIMING) {
-            const long long now = clock64();
-            tsec[k] += (unsigned long long)(now - tmark);
-            tmark = now;
-        }
-    };
 
     // it = (epoch * G + slab step t) * B + sub-epoch s; the slab of a step is (rank + t) mod G.
     // (epoch, t, s) are carried along instead of being decoded from `it`: a 64-bit division per
@@ -601,7 +518,6 @@ sgd_block_kernel(const SgdParams prm)
         // item biases of the block: L2 loads (another SM wrote them; L1 may hold a stale line)
         for (int i = threadIdx.x; i < nq; i += blockDim.x) ibs[i] = __ldcg(R.ib + cs + i);
         __syncthreads();   // tile + biases in place
-        lap(5);
 
         Frag<E> cp, cq;        // current user row / item row (post-update values)
 #pragma unroll
@@ -613,10 +529,7 @@ sgd_block_kernel(const SgdParams prm)
         // deterministic warp reduction in 32-bit fixed point: one REDUX instead of a 5-level
         // shuffle butterfly; integer addition is associative, so the result does not depend on
         // lane order.  fx_scale is a power of two chosen from max |rating| (see sgd_epoch).
-        auto warp_sum_fx = [&](int v) {
-            if constexpr (TIMING) { if (prm.exp & 4) return v; }
-            return __reduce_add_sync(FULL, v);
-        };
+        auto warp_sum_fx = [&](int v) { return __reduce_add_sync(FULL, v); };
         auto dot_fx = [&](const Frag<E> &pu, const Frag<E> &q) {
             float part;
             if constexpr (E >= 2) {
@@ -634,7 +547,6 @@ sgd_block_kernel(const SgdParams prm)
             return __float2int_rn(part * fx_scale);
         };
         auto apply = [&](int isum, float r, Frag<E> &pu, float &bu, Frag<E> &q, float &bi) {
-            if constexpr (TIMING) { if (prm.exp & 16) { se_f += (float)isum; return; } }
             const float pred = fmaf((float)isum, fx_inv, bi + bu);
             float err, grad;
             if constexpr (KERNEL == MFREC_KERNEL_LINEAR) {
@@ -665,11 +577,9 @@ sgd_block_kernel(const SgdParams prm)
             }
         };
         auto store_p_row = [&](int u, const Frag<E> &pu) {
-            if constexpr (TIMING) { if (prm.exp & 1) return; }
             pfrag_store_lane<E, PT>(pu, row_ptr(P_lane, (uint32_t)u, kRowBytes), rng);
         };
         auto store_p = [&](int u, const Frag<E> &pu, float bu) {
-            if constexpr (TIMING) { if (prm.exp & 1) return; }
             store_p_row(u, pu);
             if (lane == 0) *row_ptr(ub_g, (uint32_t)u, 4) = bu;
         };
@@ -677,14 +587,12 @@ sgd_block_kernel(const SgdParams prm)
         // user id comes straight from the record).  keep bit t clear = rating t + 1 is the same
         // user and writes the newer value.
         auto store_bias_quad = [&](const int (&u4)[4], const float (&b4)[4], uint32_t keep) {
-            if constexpr (TIMING) { if (prm.exp & 1) return; }
             const bool lo = (lane & 2) == 0, even = (lane & 1) == 0;
             const int ul = lo ? (even ? u4[0] : u4[1]) : (even ? u4[2] : u4[3]);
             const float v = lo ? (even ? b4[0] : b4[1]) : (even ? b4[2] : b4[3]);
             if (lane < 4 && ((keep >> lane) & 1u)) *row_ptr(ub_g, (uint32_t)ul, 4) = v;
         };
         auto store_q = [&](int it, const Frag<E> &q, float bi) {
-            if constexpr (TIMING) { if (prm.exp & 2) return; }
             frag_store<E>(q, Qs + (size_t)(it - cs) * KPAD, lane);
             if (lane == 0) ibs[it - cs] = bi;
         };
@@ -846,7 +754,6 @@ sgd_block_kernel(const SgdParams prm)
                     __threadfence_block();
                 }
                 __syncwarp();
-                lap(4);
             }
             se_f = 0.f;
 #pragma unroll 1
@@ -872,16 +779,13 @@ sgd_block_kernel(const SgdParams prm)
                 const uint32_t fslot0 = (fx & (kQuadsAhead - 1)) * 4;
                 PT *const fdst = prow_lane + fslot0 * KPAD;
                 auto fetch_row = [&](int t) {
-                    if constexpr (TIMING) { if (prm.exp & 8) return; }
                     const PT *gsrc = row_ptr(P_lane, fu[t], kRowBytes);
 #pragma unroll
                     for (int c = 0; c < Frag<E>::NV; ++c)
                         cp_async<Frag<E>::V * sizeof(PT)>(fdst + t * KPAD + c * 32 * Frag<E>::V, gsrc + c * 32 * Frag<E>::V);
                 };
-                lap(0);
                 cp_async_wait<kQuadsAhead - 2>();   // the four rows of this quad have landed
                 __syncwarp();                       // ... and the bias copies / lane 0's stores are visible
-                lap(1);
                 // this quad's record was read one iteration ago (its decode would otherwise sit in
                 // front of everything else with a shared-memory latency); read the next one now
                 const int4 a = na, b = nb, c2 = nc;
@@ -889,7 +793,6 @@ sgd_block_kernel(const SgdParams prm)
                     const int4 *nsrc = reinterpret_cast<const int4 *>(quad_rec(x + 1));
                     na = nsrc[0]; nb = nsrc[1]; nc = nsrc[2];
                 }
-                lap(2);
                 const uint32_t slot0 = (x & (kQuadsAhead - 1)) * 4;
                 const int u4[4] = {a.x & kIdMask, a.w & kIdMask, b.z & kIdMask, c2.y & kIdMask};
                 const int f4[4] = {a.y, b.x, b.w, c2.z};   // item ids with the packer's hint bits
@@ -899,10 +802,7 @@ sgd_block_kernel(const SgdParams prm)
                 if (qtype == kQuadIndep) {
                     indep_quad(slot0, u4, i4, r4, fetch_row);
                 } else if (qtype == kQuadChain) {
-                    bool skip = false;
-                    if constexpr (TIMING) skip = (prm.exp & 32) != 0;   // experiment: chains cost nothing
-                    if (skip) { fetch_row(0); fetch_row(1); fetch_row(2); fetch_row(3); }
-                    else chain_quad(slot0, u4, i4[0], r4, fetch_row);
+                    chain_quad(slot0, u4, i4[0], r4, fetch_row);
                 } else if (qtype == kQuadClean) {
                     clean_quad(slot0, u4, i4, f4, r4, fetch_row);
                 } else {
@@ -920,7 +820,6 @@ sgd_block_kernel(const SgdParams prm)
                     if (lane < 4) cp_async<4>(pbias + fslot0 + lane, row_ptr(ub_g, ul, 4));
                 }
                 cp_async_commit();
-                lap(3);
             }
             se += (double)se_f;
             prev_i = -1;       // the column group changes hands: never forward Q across a phase
@@ -964,7 +863,6 @@ sgd_block_kernel(const SgdParams prm)
             chunks_issued = true;
         }
         __syncthreads();   // every warp is done with the tile
-        lap(4);
         // write the Q tile back and pass the column block on.  Around a ring the last sub-epoch of
         // a step leaves the block in the NEXT rank's copy of Q (peer memory, over NVLink): that
         // rank finds it in its own HBM when the counter arrives.
@@ -1025,11 +923,6 @@ sgd_block_kernel(const SgdParams prm)
         if (ns == 0 && nt == 0) epoch_rel += 1;
         s = ns;
         t_slab = nt;
-        lap(6);
-    }
-    if constexpr (TIMING) {
-        if (prm.timing && lane == 0)
-            for (int k2 = 0; k2 < 8; ++k2) prm.timing[((size_t)rb * W + warp) * 8 + k2] = tsec[k2];
     }
     if constexpr (RING) {
         // timed out: every epoch this launch still owed reports NaN
@@ -1253,7 +1146,7 @@ size_t mfrec_sgd_smem_bytes(int tile_rows, int kpad, int W, int p_elem_bytes)
 
 namespace {
 
-template <int E, bool TIMING>
+template <int E>
 int launch_sgd(mfrec_ctx *ctx, int kernel, SgdParams &prm, size_t smem, bool cooperative, int grid, bool ring,
                int p_kind)
 {
@@ -1264,21 +1157,21 @@ int launch_sgd(mfrec_ctx *ctx, int kernel, SgdParams &prm, size_t smem, bool coo
     void (*fn)(const SgdParams) = nullptr;
     // 9..12 warps: 384 threads leave 170 registers per thread (the kernel needs ~165: no spills);
     // 13..16 warps run the 512-thread build (128 registers, spills)
-    const bool mid = prm.W > 8 && prm.W <= 12 && !gated && !TIMING;
+    const bool mid = prm.W > 8 && prm.W <= 12 && !gated;
 #define MF_PICK(K)                                                                                     \
-    fn = mid ? sgd_block_kernel<E, K, false, 384, false, false>                                         \
-       : wide ? (gated ? sgd_block_kernel<E, K, TIMING, 512, true, false> : sgd_block_kernel<E, K, TIMING, 512, false, false>) \
-              : (gated ? sgd_block_kernel<E, K, TIMING, 256, true, false> : sgd_block_kernel<E, K, TIMING, 256, false, false>)
+    fn = mid ? sgd_block_kernel<E, K, 384, false, false>                                                \
+       : wide ? (gated ? sgd_block_kernel<E, K, 512, true, false> : sgd_block_kernel<E, K, 512, false, false>) \
+              : (gated ? sgd_block_kernel<E, K, 256, true, false> : sgd_block_kernel<E, K, 256, false, false>)
 #define MF_PICK_RING(K) \
-    fn = mid ? sgd_block_kernel<E, K, false, 384, false, true>                                           \
-       : wide ? sgd_block_kernel<E, K, false, 512, false, true> : sgd_block_kernel<E, K, false, 256, false, true>
+    fn = mid ? sgd_block_kernel<E, K, 384, false, true>                                                  \
+       : wide ? sgd_block_kernel<E, K, 512, false, true> : sgd_block_kernel<E, K, 256, false, true>
     if (p_kind != MFREC_STORAGE_F32) {
         // 16-bit user-factor rows: the training build only (both sides updated, <= 12 warps, one device)
-        if constexpr (E >= 2 && !TIMING) {
+        if constexpr (E >= 2) {
             if (ring || gated || prm.W > 12)
                 return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED,
                                        "fp16 / bf16 user-factor storage: single device, both sides updated, at most 12 warps per CTA");
-#define MF_PICK16(K, T) fn = prm.W > 8 ? sgd_block_kernel<E, K, false, 384, false, false, T> : sgd_block_kernel<E, K, false, 256, false, false, T>
+#define MF_PICK16(K, T) fn = prm.W > 8 ? sgd_block_kernel<E, K, 384, false, false, T> : sgd_block_kernel<E, K, 256, false, false, T>
             if (kernel == MFREC_KERNEL_LINEAR) {
                 if (p_kind == MFREC_STORAGE_F16) { MF_PICK16(MFREC_KERNEL_LINEAR, __half); } else { MF_PICK16(MFREC_KERNEL_LINEAR, __nv_bfloat16); }
             } else {
@@ -1286,11 +1179,11 @@ int launch_sgd(mfrec_ctx *ctx, int kernel, SgdParams &prm, size_t smem, bool coo
             }
 #undef MF_PICK16
         } else {
-            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "fp16 / bf16 user-factor storage needs k > 32 (and has no timing build)");
+            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "fp16 / bf16 user-factor storage needs k > 32");
         }
     } else if (ring) {
-        if (gated || TIMING)
-            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "ring launches train both sides and have no timing build");
+        if (gated)
+            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "ring launches train both sides");
         if (kernel == MFREC_KERNEL_LINEAR) { MF_PICK_RING(MFREC_KERNEL_LINEAR); } else { MF_PICK_RING(MFREC_KERNEL_LOGISTIC); }
     } else {
         if (kernel == MFREC_KERNEL_LINEAR) { MF_PICK(MFREC_KERNEL_LINEAR); } else { MF_PICK(MFREC_KERNEL_LOGISTIC); }
@@ -1312,16 +1205,15 @@ int launch_sgd(mfrec_ctx *ctx, int kernel, SgdParams &prm, size_t smem, bool coo
     return MFREC_OK;
 }
 
-template <bool TIMING>
 int launch_sgd_kpad(mfrec_ctx *ctx, int kpad, int kernel, SgdParams &prm, size_t smem, bool cooperative,
                     int grid = 0, bool ring = false, int p_kind = MFREC_STORAGE_F32)
 {
     if (grid == 0) grid = prm.B;
     switch (kpad) {
-    case 32: return launch_sgd<1, TIMING>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
-    case 64: return launch_sgd<2, TIMING>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
-    case 128: return launch_sgd<4, TIMING>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
-    case 256: return launch_sgd<8, TIMING>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
+    case 32: return launch_sgd<1>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
+    case 64: return launch_sgd<2>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
+    case 128: return launch_sgd<4>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
+    case 256: return launch_sgd<8>(ctx, kernel, prm, smem, cooperative, grid, ring, p_kind);
     default: return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "kpad=%d", kpad);
     }
 }
@@ -1356,8 +1248,6 @@ void fill_hyper(SgdParams &prm, const mfrec_ratings *r, double learning_rate, do
     frexpf(range, &ex);              // range <= 2^ex
     prm.fx_scale = ldexpf(1.f, 30 - ex);
     prm.fx_inv = ldexpf(1.f, ex - 30);
-    prm.timing = nullptr;
-    prm.exp = 0;
     prm.wait_ns = 0;
     prm.ranks = nullptr;
 }
@@ -1440,15 +1330,6 @@ extern "C" int mfrec_sgd_epoch(mfrec_ctx *ctx, const mfrec_ratings *r, mfrec_mod
     prm.tile_rows = r->max_cb_items;
     prm.e_base = 0;
     prm.se_stride = r->B;
-    // debug: MFREC_SGD_TIMING=1 prints per-section cycle counts of the first launches to stderr
-    static int timing_env = -1;
-    if (timing_env < 0) timing_env = getenv("MFREC_SGD_TIMING") ? std::max(3, atoi(getenv("MFREC_SGD_TIMING"))) : 0;
-    DevBuf<unsigned long long> d_timing;
-    prm.exp = getenv("MFREC_SGD_EXP") ? atoi(getenv("MFREC_SGD_EXP")) : 0;
-    if (timing_env) {
-        MF_CUDA(ctx, d_timing.alloc((size_t)r->B * r->W * 8, ctx->stream));
-        prm.timing = d_timing.p;
-    }
     int64_t part = 0;
     for (int64_t it = 0; it < n_it; it += persistent ? n_it : 1) {
         prm.it_begin = it;
@@ -1457,31 +1338,7 @@ extern "C" int mfrec_sgd_epoch(mfrec_ctx *ctx, const mfrec_ratings *r, mfrec_mod
         prm.self.se_part = ctx->se_scratch + part;
         part += r->B;
         if (persistent) MF_CUDA(ctx, cudaMemsetAsync(ctx->ticks, 0, (size_t)r->G * r->B * 4, ctx->stream));
-        if (timing_env) {
-            MF_CUDA(ctx, cudaMemsetAsync(d_timing.p, 0, (size_t)r->B * r->W * 64, ctx->stream));
-            MF_TRY(launch_sgd_kpad<true>(ctx, m->kpad, kernel, prm, smem, persistent, 0, false, m->p_kind));
-            std::vector<unsigned long long> h((size_t)r->B * r->W * 8);
-            MF_CUDA(ctx, cudaMemcpyAsync(h.data(), d_timing.p, h.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
-            MF_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            double avg[8] = {0};
-            double worst_tot = 0; int worst = 0;
-            for (int c = 0; c < r->B * r->W; ++c) {
-                double busy = 0;
-                for (int k2 = 0; k2 < 8; ++k2) avg[k2] += (double)h[(size_t)c * 8 + k2];
-                for (int k2 = 0; k2 < 4; ++k2) busy += (double)h[(size_t)c * 8 + k2];
-                if (busy > worst_tot) { worst_tot = busy; worst = c; }
-            }
-            fprintf(stderr, "[sgd timing] iterations [%lld,%lld): avg cycles/warp by section "
-                            "(issue, cp.async wait, quad load, update, hand-over wait, set-up, tail):",
-                    (long long)prm.it_begin, (long long)prm.it_end);
-            for (int k2 = 0; k2 < 7; ++k2) fprintf(stderr, " %.0f", avg[k2] / (r->B * r->W));
-            fprintf(stderr, " | busiest warp (cta %d warp %d):", worst / r->W, worst % r->W);
-            for (int k2 = 0; k2 < 7; ++k2) fprintf(stderr, " %llu", h[(size_t)worst * 8 + k2]);
-            fprintf(stderr, "\n");
-            if (--timing_env == 0) prm.timing = nullptr;
-        } else {
-            MF_TRY(launch_sgd_kpad<false>(ctx, m->kpad, kernel, prm, smem, persistent, 0, false, m->p_kind));
-        }
+        MF_TRY(launch_sgd_kpad(ctx, m->kpad, kernel, prm, smem, persistent, 0, false, m->p_kind));
     }
     if (sq_err_out) {
         se_reduce_kernel<<<1, 1024, 0, ctx->stream>>>(ctx->se_scratch, nparts, sq_err_out);
@@ -1728,7 +1585,7 @@ int ring_launch(mfrec_ring *const *rings, int n_ranks, int kernel, double learni
         prm.e_base = e_first;          // sums of epoch e go to se_part[(e - e_first) * grid ...]
         prm.se_stride = grid;
         prm.wait_ns = ring_wait_ns();
-        MF_TRY(launch_sgd_kpad<false>(ctx, g0->m->kpad, kernel, prm, smem, true, grid, true));
+        MF_TRY(launch_sgd_kpad(ctx, g0->m->kpad, kernel, prm, smem, true, grid, true));
         for (int i = 0; i < n_ranks; ++i) rings[i]->epochs_done += per_launch;
         if (hot) {
             for (int i = 0; i < n_ranks; ++i) {

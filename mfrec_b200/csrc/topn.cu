@@ -20,18 +20,6 @@
 
 namespace {
 
-__device__ __forceinline__ uint32_t order_bits(float x)
-{
-    // monotone map float -> uint32 (larger float -> larger uint)
-    const uint32_t b = __float_as_uint(x);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float unorder_bits(uint32_t k)
-{
-    const uint32_t b = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
-    return __uint_as_float(b);
-}
-
 struct TopnParams {
     const float *P, *Q, *ib, *ub;
     const int32_t *users;   // [nub] user ids of this batch

@@ -36,40 +36,10 @@ constexpr int kCand = 1024;      // candidate slots per user
 constexpr int kEpiWarps = 8;
 constexpr int kSweepThreads = 64 + kEpiWarps * 32;   // warp 0 producer, warp 1 MMA, warps 2.. epilogue
 
-// ---- PTX helpers ------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
+// ---- PTX helpers (mbarrier init / expect_tx / wait and bulk copies: common.cuh) ----------------
 __device__ __forceinline__ void mbar_arrive(uint64_t *bar)
 {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes, uint64_t *bar)
-{
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
-        "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-        : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
@@ -445,16 +415,6 @@ struct FinishParams {
     int32_t *fallback;           // [n_users] 1 = not certified
 };
 
-__device__ __forceinline__ uint32_t order_bits_tc(float x)
-{
-    const uint32_t b = __float_as_uint(x);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float order_bits_inv(uint32_t key)
-{
-    return __uint_as_float((key & 0x80000000u) ? (key & 0x7fffffffu) : ~key);
-}
-
 // One CTA per user: exact fp32 score of every candidate, masks, then the top N of them in order.
 //   dots    a warp per candidate, EIGHT candidates in flight: the 32 lanes read an item row with one
 //           coalesced 512-byte request (a thread per candidate would touch 32 different rows per load
@@ -589,7 +549,7 @@ __global__ void __launch_bounds__(128, MFREC_FINISH_CTAS) topn_finish_kernel(con
                 ok = !(lo < rbnd && p.rated_items[lo] == it);
             }
         }
-        keys[c] = ok ? order_bits_tc(sc) : 0u;
+        keys[c] = ok ? order_bits(sc) : 0u;
         xs[c] = p.has_bias ? dot + bi : dot;
         if (ok && fabsf(sc) <= 3.0e38f) {   // (an infinite score keeps its key; it only stays out of the bin range)
             valid += 1;
@@ -617,7 +577,7 @@ __global__ void __launch_bounds__(128, MFREC_FINISH_CTAS) topn_finish_kernel(con
     auto bin_of = [&](float sc) { return min(255, max(0, (int)((fminf(fmaxf(sc, smin), smax) - smin) * scale))); };
     if (nvalid > p.N) {   // (block-uniform)
         for (int c = threadIdx.x; c < nn; c += 128)
-            if (keys[c]) atomicAdd(&hist[bin_of(order_bits_inv(keys[c]))], 1);
+            if (keys[c]) atomicAdd(&hist[bin_of(unorder_bits(keys[c]))], 1);
         __syncthreads();
         if (warp == 0) {
             int h[8], s = 0;
@@ -648,7 +608,7 @@ __global__ void __launch_bounds__(128, MFREC_FINISH_CTAS) topn_finish_kernel(con
     int mine = 0;
     for (int base = c_lo; base < c_hi; base += 32) {
         const int c = base + lane;
-        const bool in = c < c_hi && keys[c] && bin_of(order_bits_inv(keys[c])) >= bin_min;
+        const bool in = c < c_hi && keys[c] && bin_of(unorder_bits(keys[c])) >= bin_min;
         mine += __popc(__ballot_sync(0xffffffffu, in));
     }
     __syncthreads();   // (w_cnt was read above by every thread)
@@ -659,7 +619,7 @@ __global__ void __launch_bounds__(128, MFREC_FINISH_CTAS) topn_finish_kernel(con
     const int n_surv_all = w_cnt[0] + w_cnt[1] + w_cnt[2] + w_cnt[3];
     for (int base = c_lo; base < c_hi; base += 32) {
         const int c = base + lane;
-        const bool in = c < c_hi && keys[c] && bin_of(order_bits_inv(keys[c])) >= bin_min;
+        const bool in = c < c_hi && keys[c] && bin_of(unorder_bits(keys[c])) >= bin_min;
         const uint32_t bal = __ballot_sync(0xffffffffu, in);
         const int at = off + __popc(bal & ((1u << lane) - 1u));
         if (in && at < kSurv) { skeys[at] = keys[c]; spos[at] = (int16_t)c; }
@@ -692,7 +652,7 @@ __global__ void __launch_bounds__(128, MFREC_FINISH_CTAS) topn_finish_kernel(con
         if (rank < p.N) {
             const int src = spos[c];
             p.out_items[(size_t)row * p.N + rank] = cand_s[src];
-            p.out_scores[(size_t)row * p.N + rank] = (double)order_bits_inv(key);
+            p.out_scores[(size_t)row * p.N + rank] = (double)unorder_bits(key);
             if (rank == p.N - 1) x_nth = xs[src];
         }
     }
@@ -852,8 +812,8 @@ extern "C" int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *M, int 
     // finish kernel's time is proportional to the candidates (it is bound by the L2 -> SM traffic
     // of their item rows, ~6 TB/s), a user with fewer than N of them is redone by the exact path:
     // measured at Netflix shape, budget 2.5 -> 12.3 ms / 0 redone, 2.1 -> 10.0 ms / 0, 1.8 ->
-    // 8.5 ms / 151 users, 1.5 -> 7.2 ms / 60,785 users.  MFREC_TOPN_BUDGET overrides (experiments).
-    static double budget = getenv("MFREC_TOPN_BUDGET") ? atof(getenv("MFREC_TOPN_BUDGET")) : 2.2;
+    // 8.5 ms / 151 users, 1.5 -> 7.2 ms / 60,785 users.
+    constexpr double budget = 2.2;
     const float z = (float)inv_norm_cdf(1.0 - std::min(0.45, budget * N / (double)nc));
     tr.lap("upload + moments + pack V");
 

@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define MFREC_B200_ABI_VERSION 3
+#define MFREC_B200_ABI_VERSION 4
 
 typedef enum mfrec_status {
     MFREC_OK = 0,
@@ -136,6 +136,28 @@ int mfrec_train_kmf(mfrec_ctx *ctx, int kernel, int nbr_epochs, int k, double le
                     int32_t ni, int32_t nu, double *items_bias, double *users_bias,
                     int update_users, int update_items, const mfrec_opts *opts,
                     double *rmse_per_epoch);
+
+/* Batched fold-in: the calls KMFRecommender.retrain_user / retrain_item / add_user make
+ * (kmf.py:120-172), for many rows at once.  side: which side the listed rows belong to. */
+enum { MFREC_FOLD_USERS = 0,   /* rows are users, items frozen: update_users = 1, update_items = 0 */
+       MFREC_FOLD_ITEMS = 1    /* rows are items, users frozen: update_users = 0, update_items = 1 */ };
+/* n_rows fold-ins in one call.  Result = calling mfrec_train_kmf(schedule = SEQUENTIAL) once per
+ * listed row, in list order, with that row's ratings (the entries of ratings_index naming it, in
+ * input order) and the update flags of `side`; bit-identical to that loop.  Ratings naming no
+ * listed row are ignored.  rows must be distinct (MFREC_ERR_BAD_ARG otherwise); a row or a rating
+ * index of a listed row outside its side's range is MFREC_ERR_INDEX.  Everything is validated
+ * before anything is written.  Only the listed rows and their ratings' frozen rows are copied to the
+ * device, and only the listed rows (and, for the linear kernel, the frozen side's biases, which the
+ * reference updates unconditionally) are written back.  Each row is one GPU lane; with the linear
+ * kernel, rows that share a frozen row run one after the other in list order (a row's level = 1 +
+ * the highest level of an earlier listed row sharing a frozen row with it; one launch per level),
+ * with the logistic kernel all rows run at once.  rmse: nullable, [n_rows][nbr_epochs], row p
+ * receives what mfrec_train_kmf's rmse_per_epoch would for row p (NaN for a row without ratings). */
+int mfrec_fold_in_kmf(mfrec_ctx *ctx, int kernel, int side, int nbr_epochs, int k, double learning_rate,
+                      double K_users, double K_items, double K_bias, double *u, double *v,
+                      const int32_t *ratings_index, const double *ratings, int64_t nnz,
+                      int32_t ni, int32_t nu, double *items_bias, double *users_bias,
+                      const int32_t *rows, int32_t n_rows, double *rmse);
 
 /* mfrec_train_kmf over SEVERAL GPUs driven by this process (devices: n_dev distinct CUDA device
  * ids): the users are cut into n_dev slices of equal rating count, every device packs and trains

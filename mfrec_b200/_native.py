@@ -19,6 +19,7 @@ ERR_BAD_ARG, ERR_INDEX, ERR_OOM, ERR_CUDA, ERR_UNSUPPORTED = -1, -2, -3, -4, -5
 KERNEL_LINEAR, KERNEL_LOGISTIC = 0, 1
 FUNK_WITHOUT_BIAS, FUNK_WITH_BIAS, FUNK_WITH_BIAS_DEV = 0, 1, 2
 SCHED_STRATIFIED, SCHED_SEQUENTIAL = 0, 1
+FOLD_USERS, FOLD_ITEMS = 0, 1
 
 PREDICTORS = {
     "predict_rating": 0,
@@ -42,7 +43,7 @@ EXPORTS = (
     "mfrec_ring_create", "mfrec_ring_destroy", "mfrec_ring_handle", "mfrec_ring_connect",
     "mfrec_ring_connect_local", "mfrec_ring_epochs", "mfrec_ring_epochs_one_device", "mfrec_ring_wait",
     "mfrec_ring_sync_model", "mfrec_model_topn", "mfrec_model_topn_sweep", "mfrec_ratings_copies",
-    "mfrec_train_kmf_multi",
+    "mfrec_train_kmf_multi", "mfrec_fold_in_kmf",
 )
 
 
@@ -179,6 +180,23 @@ def train_kmf(kernel, nbr_epochs, k, lr, K_users, K_items, K_bias, u, v, ratings
         C.c_int32(v.shape[1]), _ptr(items_bias), _ptr(users_bias), C.c_int(update_users),
         C.c_int(update_items), C.byref(o), _ptr(rm)), ctx.handle)
     return rm[:max(int(nbr_epochs), 0)]
+
+
+def fold_in_kmf(kernel, side, nbr_epochs, k, lr, K_users, K_items, K_bias, u, v, ratings_index, ratings,
+                items_bias, users_bias, rows, ctx=None):
+    """Many fold-ins in one call, in place (``mfrec_fold_in_kmf``): the same result as one
+    sequential-schedule ``train_kmf`` per listed row, in list order, on that row's ratings.
+    ``side`` = FOLD_USERS (rows are users) or FOLD_ITEMS.  Returns rmse [n_rows, nbr_epochs]."""
+    ctx = ctx or default_context()
+    rows = np.ascontiguousarray(rows, dtype=np.int32).reshape(-1)
+    rm = np.zeros((rows.shape[0], max(int(nbr_epochs), 0)), dtype=np.float64)
+    _check(lib().mfrec_fold_in_kmf(
+        ctx.handle, C.c_int(kernel), C.c_int(side), C.c_int(nbr_epochs), C.c_int(k), C.c_double(lr),
+        C.c_double(K_users), C.c_double(K_items), C.c_double(K_bias), _ptr(u), _ptr(v),
+        _ptr(ratings_index), _ptr(ratings), C.c_int64(ratings.shape[0]), C.c_int32(u.shape[1]),
+        C.c_int32(v.shape[1]), _ptr(items_bias), _ptr(users_bias), _ptr(rows), C.c_int32(rows.shape[0]),
+        _ptr(rm) if rm.size else None), ctx.handle)
+    return rm
 
 
 def train_kmf_multi(devices, kernel, nbr_epochs, k, lr, K_users, K_items, K_bias, u, v, ratings_index, ratings,

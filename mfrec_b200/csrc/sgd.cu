@@ -1018,6 +1018,104 @@ merge_copies_kernel(float *__restrict__ Q, float *__restrict__ ib, int kpad, con
 // ------------------------------------------------------------------------------------------
 constexpr int kSeqRegs = 32;   // features of a row pair kept in registers by the sequential kernel
 
+// A float64 factor row: feature f at p[f * stride].  RO rows are read through the read-only path
+// and never written (the frozen side of a batched fold-in).
+template <bool RO>
+struct KmfRow {
+    double *p;
+    int64_t stride;
+    __device__ __forceinline__ double ld(int f) const
+    {
+        if constexpr (RO) return __ldg(p + (int64_t)f * stride);
+        else return p[(int64_t)f * stride];
+    }
+    __device__ __forceinline__ void st(int f, double x) const
+    {
+        if constexpr (!RO) p[(int64_t)f * stride] = x;
+    }
+};
+
+// One rating of the reference loop (kmf_train.pyx:241-273 linear, :150-185 logistic): the prediction
+// summed over f in order, the error, the bias updates, then the feature updates -- every multiply and
+// add rounded on its own.  Every schedule that must reproduce the reference calls this one function,
+// so their results agree by construction.  bi / bu: the item / user bias (a register or the array
+// element itself), replaced by its updated value where the reference updates it (the linear kernel
+// updates both unconditionally).
+// Returns the squared error.
+template <class IRow, class URow>
+__device__ __forceinline__ double kmf_rating(int kernel, int dim, double lr, double K_users, double K_items,
+                                             double K_bias, double r, const IRow &ui_, const URow &vu_,
+                                             double &bi, double &bu, int update_users, int update_items)
+{
+    const double bi0 = bi, bu0 = bu;
+    double s = __dadd_rn(__dadd_rn(0.0, bi0), bu0);
+    double e2 = 0.0;
+    auto err_grad = [&](double &err, double &grad) {
+        if (kernel == MFREC_KERNEL_LINEAR) {
+            err = __dadd_rn(r, -s);
+            grad = err;
+        } else {
+            const double sig = 1.0 / __dadd_rn(1.0, exp(-s));
+            const double p = __dadd_rn(1.0, __dmul_rn(sig, 4.0));
+            err = __dadd_rn(r, -p);
+            grad = __dmul_rn(__dmul_rn(__dmul_rn(err, sig), __dadd_rn(1.0, -sig)), 4.0);
+        }
+        e2 = __dmul_rn(err, err);
+        if (kernel == MFREC_KERNEL_LINEAR || update_users)
+            bu = __dadd_rn(bu0, __dmul_rn(lr, __dadd_rn(grad, -__dmul_rn(K_bias, bu0))));
+        if (kernel == MFREC_KERNEL_LINEAR || update_items)
+            bi = __dadd_rn(bi0, __dmul_rn(lr, __dadd_rn(grad, -__dmul_rn(K_bias, bi0))));
+    };
+    double err, grad;
+    if (dim <= kSeqRegs) {
+        // both rows fit in registers: every load of the rating is in flight at once, the
+        // sum runs over f in order, the update reuses the registers
+        double mf[kSeqRegs], cf[kSeqRegs];
+#pragma unroll
+        for (int f = 0; f < kSeqRegs; ++f)
+            if (f < dim) { mf[f] = ui_.ld(f); cf[f] = vu_.ld(f); }
+#pragma unroll
+        for (int f = 0; f < kSeqRegs; ++f)
+            if (f < dim) s = __dadd_rn(s, __dmul_rn(mf[f], cf[f]));
+        err_grad(err, grad);
+#pragma unroll
+        for (int f = 0; f < kSeqRegs; ++f) {
+            if (f >= dim) continue;
+            if (update_items)
+                ui_.st(f, __dadd_rn(mf[f], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, cf[f]), -__dmul_rn(K_items, mf[f])))));
+            if (update_users)
+                vu_.st(f, __dadd_rn(cf[f], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, mf[f]), -__dmul_rn(K_users, cf[f])))));
+        }
+    } else {
+        // rows are read eight features at a time (independent loads in flight together)
+        for (int f0 = 0; f0 < dim; f0 += 8) {
+            double a[8], b[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                if (f0 + j < dim) { a[j] = ui_.ld(f0 + j); b[j] = vu_.ld(f0 + j); }
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                if (f0 + j < dim) s = __dadd_rn(s, __dmul_rn(a[j], b[j]));
+        }
+        err_grad(err, grad);
+        for (int f0 = 0; f0 < dim; f0 += 8) {
+            double mf[8], cf[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                if (f0 + j < dim) { mf[j] = ui_.ld(f0 + j); cf[j] = vu_.ld(f0 + j); }
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                if (f0 + j >= dim) continue;
+                if (update_items)
+                    ui_.st(f0 + j, __dadd_rn(mf[j], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, cf[j]), -__dmul_rn(K_items, mf[j])))));
+                if (update_users)
+                    vu_.st(f0 + j, __dadd_rn(cf[j], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, mf[j]), -__dmul_rn(K_users, cf[j])))));
+            }
+        }
+    }
+    return e2;
+}
+
 __global__ void __launch_bounds__(32)
 kmf_sequential_kernel(int kernel, int nbr_epochs, int dim, double lr, double K_users,
                       double K_items, double K_bias, double *u, double *v,
@@ -1047,76 +1145,8 @@ kmf_sequential_kernel(int kernel, int nbr_epochs, int dim, double lr, double K_u
             double e2 = 0.0;
             for (int L = 1; L <= lmax; ++L) {
                 if (live && level == L) {
-                    double *const ui_ = u + item, *const vu_ = v + user;
-                    const double bi0 = ib[item], bu0 = ub[user];
-                    double s = __dadd_rn(__dadd_rn(0.0, bi0), bu0);
-                    auto err_grad = [&](double &err, double &grad) {
-                        if (kernel == MFREC_KERNEL_LINEAR) {
-                            err = __dadd_rn(r, -s);
-                            grad = err;
-                        } else {
-                            const double sig = 1.0 / __dadd_rn(1.0, exp(-s));
-                            const double p = __dadd_rn(1.0, __dmul_rn(sig, 4.0));
-                            err = __dadd_rn(r, -p);
-                            grad = __dmul_rn(__dmul_rn(__dmul_rn(err, sig), __dadd_rn(1.0, -sig)), 4.0);
-                        }
-                        e2 = __dmul_rn(err, err);
-                        if (kernel == MFREC_KERNEL_LINEAR || update_users)
-                            ub[user] = __dadd_rn(bu0, __dmul_rn(lr, __dadd_rn(grad, -__dmul_rn(K_bias, bu0))));
-                        if (kernel == MFREC_KERNEL_LINEAR || update_items)
-                            ib[item] = __dadd_rn(bi0, __dmul_rn(lr, __dadd_rn(grad, -__dmul_rn(K_bias, bi0))));
-                    };
-                    double err, grad;
-                    if (dim <= kSeqRegs) {
-                        // both rows fit in registers: every load of the rating is in flight at once, the
-                        // sum runs over f in order, the update reuses the registers
-                        double mf[kSeqRegs], cf[kSeqRegs];
-#pragma unroll
-                        for (int f = 0; f < kSeqRegs; ++f)
-                            if (f < dim) { mf[f] = ui_[(int64_t)f * ni]; cf[f] = vu_[(int64_t)f * nu]; }
-#pragma unroll
-                        for (int f = 0; f < kSeqRegs; ++f)
-                            if (f < dim) s = __dadd_rn(s, __dmul_rn(mf[f], cf[f]));
-                        err_grad(err, grad);
-#pragma unroll
-                        for (int f = 0; f < kSeqRegs; ++f) {
-                            if (f >= dim) continue;
-                            if (update_items)
-                                ui_[(int64_t)f * ni] =
-                                    __dadd_rn(mf[f], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, cf[f]), -__dmul_rn(K_items, mf[f]))));
-                            if (update_users)
-                                vu_[(int64_t)f * nu] =
-                                    __dadd_rn(cf[f], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, mf[f]), -__dmul_rn(K_users, cf[f]))));
-                        }
-                    } else {
-                        // rows are read eight features at a time (independent loads in flight together)
-                        for (int f0 = 0; f0 < dim; f0 += 8) {
-                            double a[8], b[8];
-#pragma unroll
-                            for (int j = 0; j < 8; ++j)
-                                if (f0 + j < dim) { a[j] = ui_[(int64_t)(f0 + j) * ni]; b[j] = vu_[(int64_t)(f0 + j) * nu]; }
-#pragma unroll
-                            for (int j = 0; j < 8; ++j)
-                                if (f0 + j < dim) s = __dadd_rn(s, __dmul_rn(a[j], b[j]));
-                        }
-                        err_grad(err, grad);
-                        for (int f0 = 0; f0 < dim; f0 += 8) {
-                            double mf[8], cf[8];
-#pragma unroll
-                            for (int j = 0; j < 8; ++j)
-                                if (f0 + j < dim) { mf[j] = ui_[(int64_t)(f0 + j) * ni]; cf[j] = vu_[(int64_t)(f0 + j) * nu]; }
-#pragma unroll
-                            for (int j = 0; j < 8; ++j) {
-                                if (f0 + j >= dim) continue;
-                                if (update_items)
-                                    ui_[(int64_t)(f0 + j) * ni] =
-                                        __dadd_rn(mf[j], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, cf[j]), -__dmul_rn(K_items, mf[j]))));
-                                if (update_users)
-                                    vu_[(int64_t)(f0 + j) * nu] =
-                                        __dadd_rn(cf[j], __dmul_rn(lr, __dadd_rn(__dmul_rn(grad, mf[j]), -__dmul_rn(K_users, cf[j]))));
-                            }
-                        }
-                    }
+                    e2 = kmf_rating(kernel, dim, lr, K_users, K_items, K_bias, r, KmfRow<false>{u + item, ni},
+                                    KmfRow<false>{v + user, nu}, ib[item], ub[user], update_users, update_items);
                 }
                 __syncwarp();   // this level's stores are visible to the lanes of the next
             }
@@ -1125,6 +1155,63 @@ kmf_sequential_kernel(int kernel, int nbr_epochs, int dim, double lr, double K_u
         if (rmse_out && lane == 0) rmse_out[epoch] = sqrt(se / (double)nnz);
         __syncwarp();
     }
+}
+
+// ------------------------------------------------------------------------------------------
+// Batched fold-in (mfrec_fold_in_kmf): many fold-ins of the kind KMFRecommender.retrain_user /
+// retrain_item / add_user make (kmf.py:120-172), each ONE row trained on its own ratings against a
+// frozen other side.  All ratings of a fold-in share that row, so a fold-in is one serial chain:
+// ONE LANE PER ROW.  The lane walks its row's ratings in input order nbr_epochs times through
+// kmf_rating, the arithmetic of kmf_sequential_kernel, and sums the squared errors in the same
+// order: the result is the per-row call's bit for bit.
+//
+// The trained row stays on chip in a per-lane slice of shared memory, lane-interleaved (feature f of
+// lane t at slice[f * lanes + t]: no bank conflicts); only when not even one lane's row fits in
+// shared memory (k > ~29k) does it stay in its global row.  The frozen rows ([m][k], one contiguous
+// row per rating) go through the read-only path.  Jobs = rows with at least one rating, in launch
+// order; job j's ratings are [job_ptr[j], job_ptr[j+1]), its row is job_row[j] of trained / tbias.
+// Jobs of one launch share no written state: with the logistic kernel nothing of the frozen side
+// is written, with the linear kernel its biases are (the reference updates them unconditionally),
+// so the host launches one level of rows at a time (mfrec_fold_in_kmf).
+// ------------------------------------------------------------------------------------------
+template <bool SMEM, int SIDE>
+__global__ void __launch_bounds__(32)
+kmf_fold_in_kernel(int kernel, int nbr_epochs, int dim, double lr, double K_users, double K_items,
+                   double K_bias, double *__restrict__ trained, double *__restrict__ tbias,
+                   const double *__restrict__ frozen, double *fbias, const int32_t *__restrict__ job_row,
+                   const int64_t *__restrict__ job_ptr, const int32_t *__restrict__ fidx,
+                   const double *__restrict__ rv, int32_t n_jobs, double *__restrict__ rmse)
+{
+    extern __shared__ double slice[];
+    const int lanes = blockDim.x, t = threadIdx.x;
+    const int32_t j = blockIdx.x * lanes + t;
+    if (j >= n_jobs) return;
+    const int32_t row = job_row[j];
+    double *const grow = trained + (size_t)row * dim;
+    const KmfRow<false> mine{SMEM ? slice + t : grow, SMEM ? lanes : 1};
+    if (SMEM)
+        for (int f = 0; f < dim; ++f) mine.st(f, grow[f]);
+    double b = tbias[row];
+    const int64_t a = job_ptr[j], e = job_ptr[j + 1];
+    const bool linear = kernel == MFREC_KERNEL_LINEAR;
+    for (int epoch = 0; epoch < nbr_epochs; ++epoch) {
+        double se = 0.0;
+        for (int64_t n = a; n < e; ++n) {
+            const int32_t c = fidx[n];
+            const double r = rv[n];
+            const KmfRow<true> other{const_cast<double *>(frozen) + (size_t)c * dim, 1};
+            double fb = linear ? fbias[c] : __ldg(fbias + c);
+            const double e2 = SIDE == MFREC_FOLD_USERS
+                ? kmf_rating(kernel, dim, lr, K_users, K_items, K_bias, r, other, mine, fb, b, 1, 0)
+                : kmf_rating(kernel, dim, lr, K_users, K_items, K_bias, r, mine, other, b, fb, 0, 1);
+            if (linear) fbias[c] = fb;
+            se = __dadd_rn(se, e2);
+        }
+        rmse[(size_t)j * nbr_epochs + epoch] = sqrt(se / (double)(e - a));
+    }
+    if (SMEM)
+        for (int f = 0; f < dim; ++f) grow[f] = mine.ld(f);
+    tbias[row] = b;
 }
 
 }  // namespace
@@ -1657,6 +1744,64 @@ extern "C" int mfrec_ring_sync_model(mfrec_ring *g)
     return MFREC_OK;
 }
 
+// The rows a fold-in's ratings name, copied out of the caller's full arrays into compact ones and
+// back (KMFRecommender.retrain_user / retrain_item / add_user, kmf.py:120-172, name a handful of
+// rows: only those move, so the untouched rest of u / v / the biases stays bit-identical like in the
+// reference).  users / items: the distinct ids the ratings name, sorted; idx: ratings_index
+// renumbered into them.  Compact factors are [k][m] like the caller's, or [m][k] with row_major.
+struct FoldRows {
+    int k = 0;
+    bool row_major = false;
+    std::vector<int32_t> users, items, idx;
+    std::vector<double> u, v, ib, ub;
+
+    static std::vector<int32_t> distinct(const int32_t *ratings_index, int64_t nnz, int col)
+    {
+        std::vector<int32_t> ids(nnz);
+        for (int64_t n = 0; n < nnz; ++n) ids[n] = ratings_index[2 * n + col];
+        std::sort(ids.begin(), ids.end());
+        ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
+        return ids;
+    }
+    size_t at(size_t m, size_t a, int f) const { return row_major ? a * k + f : (size_t)f * m + a; }
+
+    void gather(int k_, bool row_major_, const double *u_, const double *v_, const double *ib_,
+                const double *ub_, int32_t ni, int32_t nu, const int32_t *ratings_index, int64_t nnz)
+    {
+        k = k_;
+        row_major = row_major_;
+        users = distinct(ratings_index, nnz, 0);
+        items = distinct(ratings_index, nnz, 1);
+        const size_t mu = users.size(), mi = items.size();
+        u.resize((size_t)k * mi);
+        v.resize((size_t)k * mu);
+        ib.resize(mi);
+        ub.resize(mu);
+        for (int f = 0; f < k; ++f) {
+            for (size_t a = 0; a < mi; ++a) u[at(mi, a, f)] = u_[(size_t)f * ni + items[a]];
+            for (size_t a = 0; a < mu; ++a) v[at(mu, a, f)] = v_[(size_t)f * nu + users[a]];
+        }
+        for (size_t a = 0; a < mi; ++a) ib[a] = ib_[items[a]];
+        for (size_t a = 0; a < mu; ++a) ub[a] = ub_[users[a]];
+        idx.resize((size_t)2 * nnz);
+        for (int64_t n = 0; n < nnz; ++n) {
+            idx[2 * n] = (int32_t)(std::lower_bound(users.begin(), users.end(), ratings_index[2 * n]) - users.begin());
+            idx[2 * n + 1] = (int32_t)(std::lower_bound(items.begin(), items.end(), ratings_index[2 * n + 1]) - items.begin());
+        }
+    }
+    // writes the compact rows back into every non-null array
+    void scatter(double *u_, double *v_, double *ib_, double *ub_, int32_t ni, int32_t nu) const
+    {
+        const size_t mu = users.size(), mi = items.size();
+        for (int f = 0; f < k; ++f) {
+            if (u_) for (size_t a = 0; a < mi; ++a) u_[(size_t)f * ni + items[a]] = u[at(mi, a, f)];
+            if (v_) for (size_t a = 0; a < mu; ++a) v_[(size_t)f * nu + users[a]] = v[at(mu, a, f)];
+        }
+        if (ib_) for (size_t a = 0; a < mi; ++a) ib_[items[a]] = ib[a];
+        if (ub_) for (size_t a = 0; a < mu; ++a) ub_[users[a]] = ub[a];
+    }
+};
+
 static int train_kmf_sequential(mfrec_ctx *ctx, int kernel, int nbr_epochs, int k, double lr,
                                 double K_users, double K_items, double K_bias, double *u, double *v,
                                 const int32_t *idx, const double *ratings, int64_t nnz, int32_t ni,
@@ -1724,37 +1869,15 @@ extern "C" int mfrec_train_kmf(mfrec_ctx *ctx, int kernel, int nbr_epochs, int k
                                        (long long)n, a, b);
         }
         // A fold-in (KMFRecommender.retrain_user / retrain_item / add_user, kmf.py:120-172) names a
-        // handful of rows: move only those.  The untouched rest of u / v / the biases is never
-        // copied, so it stays bit-identical like in the reference.
+        // handful of rows: move only those (FoldRows).
         if (nnz <= 65536 && (int64_t)ni + nu > 4 * nnz) {
-            std::vector<int32_t> uu(nnz), ii(nnz);
-            for (int64_t n = 0; n < nnz; ++n) { uu[n] = ratings_index[2 * n]; ii[n] = ratings_index[2 * n + 1]; }
-            std::sort(uu.begin(), uu.end());
-            uu.erase(std::unique(uu.begin(), uu.end()), uu.end());
-            std::sort(ii.begin(), ii.end());
-            ii.erase(std::unique(ii.begin(), ii.end()), ii.end());
-            const int32_t mu_ = (int32_t)uu.size(), mi_ = (int32_t)ii.size();
-            std::vector<double> cu((size_t)k * mi_), cv((size_t)k * mu_), cib(mi_), cub_(mu_);
-            std::vector<int32_t> cidx((size_t)2 * nnz);
-            for (int f = 0; f < k; ++f) {
-                for (int32_t a = 0; a < mi_; ++a) cu[(size_t)f * mi_ + a] = u[(size_t)f * ni + ii[a]];
-                for (int32_t a = 0; a < mu_; ++a) cv[(size_t)f * mu_ + a] = v[(size_t)f * nu + uu[a]];
-            }
-            for (int32_t a = 0; a < mi_; ++a) cib[a] = items_bias[ii[a]];
-            for (int32_t a = 0; a < mu_; ++a) cub_[a] = users_bias[uu[a]];
-            for (int64_t n = 0; n < nnz; ++n) {
-                cidx[2 * n] = (int32_t)(std::lower_bound(uu.begin(), uu.end(), ratings_index[2 * n]) - uu.begin());
-                cidx[2 * n + 1] = (int32_t)(std::lower_bound(ii.begin(), ii.end(), ratings_index[2 * n + 1]) - ii.begin());
-            }
+            FoldRows g;
+            g.gather(k, false, u, v, items_bias, users_bias, ni, nu, ratings_index, nnz);
             MF_TRY(train_kmf_sequential(ctx, kernel, nbr_epochs, k, learning_rate, K_users, K_items, K_bias,
-                                        cu.data(), cv.data(), cidx.data(), ratings, nnz, mi_, mu_, cib.data(),
-                                        cub_.data(), update_users, update_items, rmse_per_epoch));
-            for (int f = 0; f < k; ++f) {
-                for (int32_t a = 0; a < mi_; ++a) u[(size_t)f * ni + ii[a]] = cu[(size_t)f * mi_ + a];
-                for (int32_t a = 0; a < mu_; ++a) v[(size_t)f * nu + uu[a]] = cv[(size_t)f * mu_ + a];
-            }
-            for (int32_t a = 0; a < mi_; ++a) items_bias[ii[a]] = cib[a];
-            for (int32_t a = 0; a < mu_; ++a) users_bias[uu[a]] = cub_[a];
+                                        g.u.data(), g.v.data(), g.idx.data(), ratings, nnz, (int32_t)g.items.size(),
+                                        (int32_t)g.users.size(), g.ib.data(), g.ub.data(), update_users,
+                                        update_items, rmse_per_epoch));
+            g.scatter(u, v, items_bias, users_bias, ni, nu);
             return MFREC_OK;
         }
         return train_kmf_sequential(ctx, kernel, nbr_epochs, k, learning_rate, K_users, K_items, K_bias,
@@ -1880,4 +2003,173 @@ extern "C" int mfrec_train_kmf(mfrec_ctx *ctx, int kernel, int nbr_epochs, int k
     mfrec_ratings_destroy(R);
     tr.lap("free");
     return rc;
+}
+
+extern "C" int mfrec_fold_in_kmf(mfrec_ctx *ctx, int kernel, int side, int nbr_epochs, int k, double learning_rate,
+                                 double K_users, double K_items, double K_bias, double *u, double *v,
+                                 const int32_t *ratings_index, const double *ratings, int64_t nnz,
+                                 int32_t ni, int32_t nu, double *items_bias, double *users_bias,
+                                 const int32_t *rows, int32_t n_rows, double *rmse)
+{
+    if (!ctx) return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "mfrec_fold_in_kmf: NULL ctx");
+    if (!u || !v || !items_bias || !users_bias || (nnz > 0 && (!ratings_index || !ratings)) || (n_rows > 0 && !rows))
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_kmf: NULL array");
+    if (kernel != MFREC_KERNEL_LINEAR && kernel != MFREC_KERNEL_LOGISTIC)
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_kmf: kernel=%d", kernel);
+    if (side != MFREC_FOLD_USERS && side != MFREC_FOLD_ITEMS)
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_kmf: side=%d", side);
+    if (k <= 0 || ni <= 0 || nu <= 0 || nnz < 0 || nbr_epochs < 0 || n_rows < 0)
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_kmf: k=%d ni=%d nu=%d nnz=%lld epochs=%d rows=%d",
+                               k, ni, nu, (long long)nnz, nbr_epochs, n_rows);
+    const bool by_user = side == MFREC_FOLD_USERS, linear = kernel == MFREC_KERNEL_LINEAR;
+    const int tc = by_user ? 0 : 1;   // column of ratings_index naming the trained row; 1 - tc the frozen one
+    const int32_t n_side = by_user ? nu : ni, n_other = by_user ? ni : nu;
+
+    // list position of every trained-side row (-1: not listed)
+    std::vector<int32_t> pos(n_side, -1);
+    for (int32_t p = 0; p < n_rows; ++p) {
+        const int32_t r = rows[p];
+        if (r < 0 || r >= n_side)
+            return mfrec_set_error(ctx, MFREC_ERR_INDEX, "mfrec_fold_in_kmf: rows[%d] = %d outside [0, %d)", p, r, n_side);
+        if (pos[r] >= 0)
+            return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_kmf: row %d is listed twice (%d, %d)", r, pos[r], p);
+        pos[r] = p;
+    }
+    auto listed = [&](int64_t n) {
+        const int32_t t = ratings_index[2 * n + tc];
+        return t >= 0 && t < n_side ? pos[t] : -1;
+    };
+    // every listed row's ratings in input order: a stable counting sort by list position
+    std::vector<int64_t> rptr((size_t)n_rows + 1, 0);
+    for (int64_t n = 0; n < nnz; ++n) {
+        const int32_t p = listed(n);
+        if (p < 0) continue;
+        const int32_t o = ratings_index[2 * n + 1 - tc];
+        if (o < 0 || o >= n_other)
+            return mfrec_set_error(ctx, MFREC_ERR_INDEX, "mfrec_fold_in_kmf: rating %lld has (user,item)=(%d,%d)",
+                                   (long long)n, ratings_index[2 * n], ratings_index[2 * n + 1]);
+        ++rptr[p + 1];
+    }
+    for (int32_t p = 0; p < n_rows; ++p) rptr[p + 1] += rptr[p];
+    const int64_t nsel = rptr[n_rows];
+    MF_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (nbr_epochs == 0) return MFREC_OK;
+    if (rmse)   // a row without ratings: the reference divides 0/0 and leaves the model untouched
+        for (int32_t p = 0; p < n_rows; ++p)
+            if (rptr[p + 1] == rptr[p])
+                for (int e = 0; e < nbr_epochs; ++e) rmse[(size_t)p * nbr_epochs + e] = NAN;
+    if (nsel == 0) return MFREC_OK;
+    std::vector<int32_t> sidx((size_t)2 * nsel);
+    std::vector<double> sr(nsel);
+    {
+        std::vector<int64_t> cur(rptr.begin(), rptr.end() - 1);
+        for (int64_t n = 0; n < nnz; ++n) {
+            const int32_t p = listed(n);
+            if (p < 0) continue;
+            const int64_t s = cur[p]++;
+            sidx[2 * s] = ratings_index[2 * n];
+            sidx[2 * s + 1] = ratings_index[2 * n + 1];
+            sr[s] = ratings[n];
+        }
+    }
+    // the listed rows and the frozen rows their ratings name, row-major (a lane reads whole rows)
+    FoldRows g;
+    g.gather(k, true, u, v, items_bias, users_bias, ni, nu, sidx.data(), nsel);
+    std::vector<double> &tf = by_user ? g.v : g.u, &tb = by_user ? g.ub : g.ib, &fbv = by_user ? g.ib : g.ub;
+    const std::vector<double> &ff = by_user ? g.u : g.v;
+    const size_t n_frozen = by_user ? g.items.size() : g.users.size();
+
+    // Levels.  Logistic: rows share no written state, one level.  Linear: a row's ratings write the
+    // biases of its frozen rows, so a row runs after every earlier listed row that shares a frozen
+    // row with it: level = 1 + the highest level of such a row (one "last level" per frozen row).
+    struct Job { int32_t level, p; int64_t cnt; };
+    std::vector<Job> jobs;
+    jobs.reserve(n_rows);
+    std::vector<int32_t> last(linear ? n_frozen : 0, 0);
+    for (int32_t p = 0; p < n_rows; ++p) {
+        const int64_t a = rptr[p], b = rptr[p + 1];
+        if (a == b) continue;
+        int32_t level = 1;
+        if (linear) {
+            for (int64_t n = a; n < b; ++n) level = std::max(level, last[g.idx[2 * n + 1 - tc]] + 1);
+            for (int64_t n = a; n < b; ++n) last[g.idx[2 * n + 1 - tc]] = level;
+        }
+        jobs.push_back({level, p, b - a});
+    }
+    // levels in order; inside a level the longest rows first, so the lanes of a warp have similar trip counts
+    std::stable_sort(jobs.begin(), jobs.end(), [](const Job &x, const Job &y) {
+        return x.level != y.level ? x.level < y.level : x.cnt > y.cnt;
+    });
+    const int32_t n_jobs = (int32_t)jobs.size();
+    std::vector<int32_t> job_row(n_jobs), fidx(nsel), level_start;
+    std::vector<int64_t> job_ptr((size_t)n_jobs + 1, 0);
+    std::vector<double> rv(nsel);
+    for (int32_t j = 0; j < n_jobs; ++j) {
+        const Job &J = jobs[j];
+        if (j == 0 || J.level != jobs[j - 1].level) level_start.push_back(j);
+        const int64_t a = rptr[J.p];
+        job_row[j] = g.idx[2 * a + tc];
+        for (int64_t n = 0; n < J.cnt; ++n) {
+            fidx[job_ptr[j] + n] = g.idx[2 * (a + n) + 1 - tc];
+            rv[job_ptr[j] + n] = sr[a + n];
+        }
+        job_ptr[j + 1] = job_ptr[j] + J.cnt;
+    }
+    level_start.push_back(n_jobs);
+
+    // lanes per block: as many per-lane shared-memory rows as fit (up to a warp)
+    const size_t row_bytes = (size_t)k * 8;
+    const int lanes = (int)std::min<size_t>(32, ctx->smem_optin / row_bytes);
+    const bool smem = lanes > 0;
+    const int block = smem ? lanes : 32;
+    const size_t smem_bytes = smem ? (size_t)lanes * row_bytes : 0;
+    auto launch = by_user ? (smem ? kmf_fold_in_kernel<true, MFREC_FOLD_USERS> : kmf_fold_in_kernel<false, MFREC_FOLD_USERS>)
+                          : (smem ? kmf_fold_in_kernel<true, MFREC_FOLD_ITEMS> : kmf_fold_in_kernel<false, MFREC_FOLD_ITEMS>);
+    if (smem_bytes > 48 * 1024)
+        MF_CUDA(ctx, cudaFuncSetAttribute(launch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+
+    cudaStream_t st = ctx->stream;
+    DevBuf<double> d_tf, d_tb, d_ff, d_fb, d_rv, d_rm;
+    DevBuf<int32_t> d_row, d_fidx;
+    DevBuf<int64_t> d_ptr;
+    MF_CUDA(ctx, d_tf.alloc(tf.size(), st));
+    MF_CUDA(ctx, d_tb.alloc(tb.size(), st));
+    MF_CUDA(ctx, d_ff.alloc(ff.size(), st));
+    MF_CUDA(ctx, d_fb.alloc(fbv.size(), st));
+    MF_CUDA(ctx, d_rv.alloc(nsel, st));
+    MF_CUDA(ctx, d_fidx.alloc(nsel, st));
+    MF_CUDA(ctx, d_row.alloc(n_jobs, st));
+    MF_CUDA(ctx, d_ptr.alloc((size_t)n_jobs + 1, st));
+    MF_CUDA(ctx, d_rm.alloc((size_t)n_jobs * nbr_epochs, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_tf.p, tf.data(), tf.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_tb.p, tb.data(), tb.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_ff.p, ff.data(), ff.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_fb.p, fbv.data(), fbv.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_rv.p, rv.data(), (size_t)nsel * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_fidx.p, fidx.data(), (size_t)nsel * 4, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_row.p, job_row.data(), (size_t)n_jobs * 4, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_ptr.p, job_ptr.data(), ((size_t)n_jobs + 1) * 8, cudaMemcpyHostToDevice, st));
+    for (size_t L = 0; L + 1 < level_start.size(); ++L) {
+        const int32_t j0 = level_start[L], n = level_start[L + 1] - j0;
+        const int grid = (n + block - 1) / block;
+        launch<<<grid, block, smem_bytes, st>>>(kernel, nbr_epochs, k, learning_rate, K_users, K_items, K_bias,
+                                                d_tf.p, d_tb.p, d_ff.p, d_fb.p, d_row.p + j0, d_ptr.p + j0, d_fidx.p,
+                                                d_rv.p, n, d_rm.p + (size_t)j0 * nbr_epochs);
+        MF_LAUNCH_CHECK(ctx);
+    }
+    std::vector<double> h_rm((size_t)n_jobs * nbr_epochs);
+    MF_CUDA(ctx, cudaMemcpyAsync(tf.data(), d_tf.p, tf.size() * 8, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(tb.data(), d_tb.p, tb.size() * 8, cudaMemcpyDeviceToHost, st));
+    if (linear) MF_CUDA(ctx, cudaMemcpyAsync(fbv.data(), d_fb.p, fbv.size() * 8, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(h_rm.data(), d_rm.p, h_rm.size() * 8, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(ctx, cudaStreamSynchronize(st));
+    // only the trained side (and, linear, the frozen biases) goes back: the frozen rows and every
+    // unlisted row are never written
+    if (by_user) g.scatter(nullptr, v, linear ? items_bias : nullptr, users_bias, ni, nu);
+    else g.scatter(u, nullptr, items_bias, linear ? users_bias : nullptr, ni, nu);
+    if (rmse)
+        for (int32_t j = 0; j < n_jobs; ++j)
+            std::copy(h_rm.begin() + (size_t)j * nbr_epochs, h_rm.begin() + (size_t)(j + 1) * nbr_epochs,
+                      rmse + (size_t)jobs[j].p * nbr_epochs);
+    return MFREC_OK;
 }

@@ -5,12 +5,16 @@
 Cython module the reference imports (kmf.py:18, with its broken package path fixed)."""
 import numpy as np
 
+from mfrec_b200 import _native
 from mfrec_b200.lib import kmf_train
+from mfrec_b200.lib._buffers import buffer_arg
 from mfrec_b200.recommendation.base import Error
 from mfrec_b200.recommendation.mf import MFRecommender
 
 _KERNELS = {'train_logistic_kernel': kmf_train.train_logistic_kernel,
             'train_linear_kernel': kmf_train.train_linear_kernel}
+_KERNEL_IDS = {'train_logistic_kernel': _native.KERNEL_LOGISTIC,
+               'train_linear_kernel': _native.KERNEL_LINEAR}
 
 
 def _fold_in(kernel, *args):
@@ -129,3 +133,96 @@ class KMFRecommender(MFRecommender):
         ratings_index[:, 1] = users_ratings_index
         self.retrain_user(new_id, ratings_index, np.asarray(users_ratings, dtype=np.float64))
         return new_id
+
+    # ---- batched fold-in (not in the reference): one device call for many rows ----------------------
+    # Each leaves the recommender exactly as the loop of the single-row method over the same rows
+    # would: factors, biases, index / label maps and the numpy RNG (the new rows' initial features
+    # are drawn in list order before the one native call; training draws nothing).  Everything is
+    # validated before anything changes or is drawn.  Rows must be distinct and in range.
+    def retrain_users(self, user_indices, ratings_index, ratings, verbose=False, kernel='train_logistic_kernel'):
+        """``for u in user_indices: self.retrain_user(u, ratings_index, ratings, verbose, kernel)``."""
+        kernel_id = _KERNEL_IDS[kernel]
+        rows = _fold_rows(user_indices, self.nbr_users)
+        if rows.shape[0]:
+            idx, r = _fold_ratings(rows, 0, self.nbr_items, ratings_index, ratings)
+            self._fold_in_batch(_native.FOLD_USERS, rows, idx, r, verbose, kernel_id)
+
+    def retrain_items(self, item_indices, ratings_index, ratings, verbose=False, kernel='train_logistic_kernel'):
+        """``for i in item_indices: self.retrain_item(i, ratings_index, ratings, verbose, kernel)``."""
+        kernel_id = _KERNEL_IDS[kernel]
+        rows = _fold_rows(item_indices, self.nbr_items)
+        if rows.shape[0]:
+            idx, r = _fold_ratings(rows, 1, self.nbr_users, ratings_index, ratings)
+            self._fold_in_batch(_native.FOLD_ITEMS, rows, idx, r, verbose, kernel_id)
+
+    def add_users(self, user_labels, users_ratings_index_list, users_ratings_list, verbose=False,
+                  kernel='train_logistic_kernel'):
+        """``[self.add_user(l, i, r) for l, i, r in zip(...)]`` (add_user trains with the logistic
+        kernel, silently; ``kernel`` / ``verbose`` choose otherwise).  Returns the new user ids."""
+        kernel_id = _KERNEL_IDS[kernel]
+        labels, items_list, ratings_list = list(user_labels), list(users_ratings_index_list), list(users_ratings_list)
+        if not len(labels) == len(items_list) == len(ratings_list):
+            raise ValueError('user_labels, users_ratings_index_list and users_ratings_list differ in length')
+        first, n = self.nbr_users, len(labels)
+        if n == 0:
+            return []
+        idx, r = [], []
+        for j, (items, ratings) in enumerate(zip(items_list, ratings_list)):
+            items, ratings = np.asarray(items), np.asarray(ratings, dtype=np.float64)
+            if items.shape[0] != ratings.shape[0]:
+                raise Error('The index and the ratings array must be the same size')
+            ratings_index = np.zeros([ratings.shape[0], 2], dtype=np.int32)
+            ratings_index[:, 0] = first + j
+            ratings_index[:, 1] = items
+            idx.append(ratings_index)
+            r.append(ratings)
+        rows = np.arange(first, first + n)
+        idx, r = _fold_ratings(rows, 0, self.nbr_items, np.concatenate(idx), np.concatenate(r))
+        for label in labels:
+            new_id = self._get_new_user_id()
+            self.users_index[label] = new_id
+            self.users_label[new_id] = label
+        self.svd_v = np.ascontiguousarray(np.c_[self.svd_v, np.zeros((self.dimensionality, n))])
+        self.users_bias = np.r_[self.users_bias, np.zeros(n)]
+        self._fold_in_batch(_native.FOLD_USERS, rows, idx, r, verbose, kernel_id)
+        return [int(x) for x in rows]
+
+    def _fold_in_batch(self, side, rows, ratings_index, ratings, verbose, kernel_id):
+        init = self.init_user_features if side == _native.FOLD_USERS else self.init_item_features
+        for row in rows:
+            init(row)
+        kmf_train.fold_in(kernel_id, side, self.nbr_epochs, self.dimensionality, self.learning_rate,
+                          self.K_users, self.K_items, self.K_bias, self.svd_u, self.svd_v, ratings_index,
+                          ratings, self.items_bias, self.users_bias, rows, int(verbose))
+        self.invalidate_model()   # a few rows changed in place: the sampled fingerprint may miss them
+
+
+def _fold_rows(indices, n):
+    """The listed rows as int64: in [0, n) (IndexError) and distinct (ValueError)."""
+    rows = np.asarray(indices).reshape(-1)
+    if rows.shape[0] and not np.issubdtype(rows.dtype, np.integer):
+        raise IndexError('row indices must be integers, got %s' % rows.dtype)
+    rows = rows.astype(np.int64)
+    bad = (rows < 0) | (rows >= n)
+    if bad.any():
+        raise IndexError('row %d is outside [0, %d)' % (rows[bad][0], n))
+    if np.unique(rows).shape[0] != rows.shape[0]:
+        raise ValueError('a row is listed more than once')
+    return rows
+
+
+def _fold_ratings(rows, col, n_other, ratings_index, ratings):
+    """The ratings naming a listed row (column ``col``), in input order, checked like the single-row
+    calls check theirs: int32 / float64 buffers (ValueError), the other index in [0, n_other)
+    (IndexError)."""
+    ids = np.nonzero(np.isin(ratings_index[:, col], rows))[0]
+    idx = np.ascontiguousarray(ratings_index[ids, :])
+    r = np.ascontiguousarray(ratings[ids])
+    buffer_arg(idx, "ratings_index", np.int32, 2, writable=False)
+    buffer_arg(r, "ratings", np.float64, 1, writable=False)
+    other = idx[:, 1 - col]
+    bad = (other < 0) | (other >= n_other)
+    if bad.any():
+        raise IndexError('rating (user, item) = (%d, %d) names no %s' % (idx[bad][0, 0], idx[bad][0, 1],
+                                                                         'item' if col == 0 else 'user'))
+    return idx, r

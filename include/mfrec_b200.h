@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define MFREC_B200_ABI_VERSION 4
+#define MFREC_B200_ABI_VERSION 5
 
 typedef enum mfrec_status {
     MFREC_OK = 0,
@@ -184,6 +184,26 @@ int mfrec_train_funk(mfrec_ctx *ctx, int variant, int min_epochs, int max_epochs
                      int32_t ni, int32_t nu, const double *items_bias,
                      const double *users_bias, int update_users, int update_items,
                      const mfrec_opts *opts, int32_t *feature_epochs, double *feature_rmse);
+
+/* Batched Funk-SVD fold-in: the calls GDRecommender.retrain_user / retrain_item make
+ * (gradient_descent.py:879-905), for many rows at once.  side: MFREC_FOLD_USERS / MFREC_FOLD_ITEMS.
+ * Result = calling mfrec_train_funk(variant = MFREC_FUNK_WITH_BIAS_DEV, schedule = SEQUENTIAL) once
+ * per listed row, in list order, with that row's ratings (the entries of ratings_index naming it, in
+ * input order) and the update flags of `side`; bit-identical to that loop.  Ratings naming no listed
+ * row are ignored.  rows must be distinct (MFREC_ERR_BAD_ARG otherwise); a row or a rating index of a
+ * listed row outside its side's range is MFREC_ERR_INDEX; a listed row without ratings is
+ * MFREC_ERR_BAD_ARG (mfrec_train_funk refuses nnz = 0).  Everything is validated before anything is
+ * written.  Only the listed rows and their ratings' frozen rows are copied to the device, and only
+ * the listed rows are written back; the biases are read only.  The loop writes nothing two rows
+ * share, so every row is one GPU lane of one launch.  There is no max_epochs: the reference ignores
+ * it.  feature_epochs (nullable, int32 [n_rows][k]) and feature_rmse (nullable, [n_rows][k]): row p
+ * receives what mfrec_train_funk's feature_epochs / feature_rmse would for row p. */
+int mfrec_fold_in_funk(mfrec_ctx *ctx, int side, int min_epochs, double min_improvement, int k,
+                       double f_init, double learning_rate, double K, double overall_avg,
+                       double *u, double *v, const int32_t *ratings_index, const double *ratings,
+                       int64_t nnz, int32_t ni, int32_t nu, const double *items_bias,
+                       const double *users_bias, const int32_t *rows, int32_t n_rows,
+                       int32_t *feature_epochs, double *feature_rmse);
 
 /* ---- development variants of the Funk loop (SURVEY 8(a) A3; mfrec_b200/csrc/funk_dev.cu) ----
  * They run in the reference's own order (one device thread, float64, unfused) and are

@@ -43,7 +43,7 @@ EXPORTS = (
     "mfrec_ring_create", "mfrec_ring_destroy", "mfrec_ring_handle", "mfrec_ring_connect",
     "mfrec_ring_connect_local", "mfrec_ring_epochs", "mfrec_ring_epochs_one_device", "mfrec_ring_wait",
     "mfrec_ring_sync_model", "mfrec_model_topn", "mfrec_model_topn_sweep", "mfrec_ratings_copies",
-    "mfrec_train_kmf_multi", "mfrec_fold_in_kmf",
+    "mfrec_train_kmf_multi", "mfrec_fold_in_kmf", "mfrec_fold_in_funk",
 )
 
 
@@ -229,6 +229,25 @@ def train_funk(variant, min_epochs, max_epochs, min_improvement, k, f_init, lr, 
         C.c_int64(ratings.shape[0]), C.c_int32(u.shape[1]), C.c_int32(v.shape[1]),
         _ptr(items_bias), _ptr(users_bias), C.c_int(update_users), C.c_int(update_items),
         C.byref(o), _ptr(fe), _ptr(fr)), ctx.handle)
+    return fe, fr
+
+
+def fold_in_funk(side, min_epochs, min_improvement, k, f_init, lr, K, overall_avg, u, v, ratings_index,
+                 ratings, items_bias, users_bias, rows, ctx=None):
+    """Many Funk-SVD fold-ins in one call, in place (``mfrec_fold_in_funk``): the same result as one
+    sequential-schedule ``train_funk(FUNK_WITH_BIAS_DEV, ...)`` per listed row, in list order, on that
+    row's ratings.  ``side`` = FOLD_USERS (rows are users) or FOLD_ITEMS.  Returns (feature_epochs
+    int32 [n_rows, k], feature_rmse [n_rows, k])."""
+    ctx = ctx or default_context()
+    rows = np.ascontiguousarray(rows, dtype=np.int32).reshape(-1)
+    fe = np.zeros((rows.shape[0], k), dtype=np.int32)
+    fr = np.zeros((rows.shape[0], k), dtype=np.float64)
+    _check(lib().mfrec_fold_in_funk(
+        ctx.handle, C.c_int(side), C.c_int(min_epochs), C.c_double(min_improvement), C.c_int(k),
+        C.c_double(f_init), C.c_double(lr), C.c_double(K), C.c_double(overall_avg), _ptr(u), _ptr(v),
+        _ptr(ratings_index), _ptr(ratings), C.c_int64(ratings.shape[0]), C.c_int32(u.shape[1]),
+        C.c_int32(v.shape[1]), _ptr(items_bias), _ptr(users_bias), _ptr(rows), C.c_int32(rows.shape[0]),
+        _ptr(fe) if fe.size else None, _ptr(fr) if fr.size else None), ctx.handle)
     return fe, fr
 
 

@@ -24,8 +24,10 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <numeric>
 
 #include "common.cuh"
+#include "fold.h"
 
 namespace {
 
@@ -50,6 +52,24 @@ __device__ __forceinline__ double funk_estimate(double uf, double vf, double cac
         s = clamp15(s);
     }
     return s;
+}
+
+// One rating of the reference loop (gd_estimator.pyx:588-685): the prediction from the cached
+// partial prediction `cache` (or the baseline `base` while the cache is 0), the error, and the new
+// item scalar (from the OLD mf, cf) handed to set_mf, then the new user scalar to set_cf, each only
+// if its flag is set.  Returns the squared error.  funk_sequential_kernel and funk_fold_in_kernel
+// share it, so both run the same operations in the same order.
+template <class SetM, class SetC>
+__device__ __forceinline__ double funk_rating(double r, double cache, double base, double trail, double lr,
+                                              double K, double mf, double cf, int update_items,
+                                              int update_users, SetM set_mf, SetC set_cf)
+{
+    const double pr = funk_estimate(mf, cf, cache, base, trail, 1);
+    const double err = __dadd_rn(r, -pr);
+    const double e2 = __dmul_rn(err, err);
+    if (update_items) set_mf(__dadd_rn(mf, __dmul_rn(lr, __dadd_rn(__dmul_rn(err, cf), -__dmul_rn(K, mf)))));
+    if (update_users) set_cf(__dadd_rn(cf, __dmul_rn(lr, __dadd_rn(__dmul_rn(err, mf), -__dmul_rn(K, cf)))));
+    return e2;
 }
 
 struct FunkParams {
@@ -419,13 +439,8 @@ funk_sequential_kernel(int variant, int min_epochs, double min_improvement, int 
                 for (int L = 1; L <= lmax; ++L) {
                     if (live && level == L) {
                         const double cf = vf[user], mf = uf[item];
-                        const double pr = funk_estimate(mf, cf, cc, bb, trail, 1);
-                        const double err = __dadd_rn(r, -pr);
-                        e2 = __dmul_rn(err, err);
-                        if (update_items)
-                            uf[item] = __dadd_rn(mf, __dmul_rn(lr, __dadd_rn(__dmul_rn(err, cf), -__dmul_rn(K, mf))));
-                        if (update_users)
-                            vf[user] = __dadd_rn(cf, __dmul_rn(lr, __dadd_rn(__dmul_rn(err, mf), -__dmul_rn(K, cf))));
+                        e2 = funk_rating(r, cc, bb, trail, lr, K, mf, cf, update_items, update_users,
+                                         [&](double x) { uf[item] = x; }, [&](double x) { vf[user] = x; });
                     }
                     __syncwarp();   // this level's stores are visible to the lanes of the next
                 }
@@ -444,6 +459,111 @@ funk_sequential_kernel(int variant, int min_epochs, double min_improvement, int 
             cache[n] = funk_estimate(uf[item], vf[user], cache[n], bb, 0.0, 0);
         }
         __syncwarp();
+    }
+}
+
+// ---- batched fold-in (mfrec_fold_in_funk) -------------------------------------------------------
+// Many fold-ins of the kind GDRecommender.retrain_user / retrain_item make (gradient_descent.py:
+// 879-905): each trains ONE row on its own ratings with estimator_loop_with_bias_dev, the other side
+// frozen by the update flags.  That loop reads both bias arrays and the frozen side and writes
+// nothing but the row, so two fold-ins share no written state: all rows run in one launch, ONE LANE
+// PER ROW, in any order.
+//
+// A lane replays funk_sequential_kernel for its row.  Every rating names the row, so each one
+// depends on the one before it: the lane walks them in input order through funk_rating and sums the
+// squared errors in that order.  Within feature f the row's scalar t stays in a register, and what
+// else a rating's update reads is constant: the frozen scalar o and s0 = cache > 0 ? cache : base.
+// Both are staged once per feature (so[], ss[]) and loaded kAhead ratings ahead of the update that
+// needs them, so the chain is the ~13 dependent float64 operations of the update and no memory
+// round trip.  The cache refresh after a feature is folded into the next feature's staging.
+//
+// Jobs (rows) are sorted by rating count, longest first; block w holds jobs [32w, 32w + 32).  The
+// per-rating arrays are warp-interleaved: rating n of lane l of block w sits at
+// warp_off[w] + 32 n + l, so the lanes of a warp load consecutive addresses.  trained / frozen are
+// compact row-major [m][dim]; tbias / fbias their biases; fidx the frozen row of every rating.
+constexpr int kAhead = 8;   // ratings whose staged inputs are in flight ahead of the update
+
+template <int SIDE>
+__global__ void __launch_bounds__(32)
+funk_fold_in_kernel(int min_epochs, double min_improvement, int dim, double f_init, double lr, double K,
+                    double overall, double *__restrict__ trained, const double *__restrict__ tbias,
+                    const double *__restrict__ frozen, const double *__restrict__ fbias,
+                    const int32_t *__restrict__ job_row, const int32_t *__restrict__ job_cnt,
+                    const int64_t *__restrict__ warp_off, const int32_t *__restrict__ fidx,
+                    const double *__restrict__ rv, double *__restrict__ base, double *__restrict__ so,
+                    double *__restrict__ ss, int32_t n_jobs, int32_t *__restrict__ feature_epochs,
+                    double *__restrict__ feature_rmse)
+{
+    const int32_t j = blockIdx.x * 32 + threadIdx.x;
+    if (j >= n_jobs) return;
+    const int32_t row = job_row[j], cnt = job_cnt[j];
+    const int64_t p0 = warp_off[blockIdx.x] + threadIdx.x;
+    double *const grow = trained + (size_t)row * dim;
+    // the baseline of every rating: overall + b_item + b_user, in that order (gd_estimator.pyx:38-73)
+    const double tb = tbias[row];
+    for (int n = 0; n < cnt; ++n) {
+        const int64_t p = p0 + 32 * (int64_t)n;
+        const double fb = fbias[fidx[p]];
+        base[p] = SIDE == MFREC_FOLD_USERS ? __dadd_rn(__dadd_rn(overall, fb), tb)
+                                           : __dadd_rn(__dadd_rn(overall, tb), fb);
+    }
+    // rating n's staged inputs, or nothing past the row's end
+    auto load = [&](int n, double &o, double &s, double &r) {
+        if (n < cnt) {
+            const int64_t p = p0 + 32 * (int64_t)n;
+            o = so[p]; s = ss[p]; r = rv[p];
+        } else {
+            o = 0.0; s = 0.0; r = 0.0;
+        }
+    };
+    double rmse = 2.0, rmse_last = 0.0, t = 0.0;
+    for (int f = 0; f < dim; ++f) {
+        // stage feature f: the frozen scalars, and s0 from the cache feature f - 1 left behind
+        // (funk_sequential_kernel's refresh: funk_estimate(..., trailing = 0); the cache is 0 at f = 0)
+        for (int n = 0; n < cnt; ++n) {
+            const int64_t p = p0 + 32 * (int64_t)n;
+            double s0 = base[p];
+            if (f > 0) {
+                const double o = so[p], sp = ss[p];
+                const double c = SIDE == MFREC_FOLD_USERS ? funk_estimate(o, t, sp, sp, 0.0, 0)
+                                                          : funk_estimate(t, o, sp, sp, 0.0, 0);
+                s0 = c > 0 ? c : s0;
+            }
+            ss[p] = s0;
+            so[p] = frozen[(size_t)fidx[p] * dim + f];
+        }
+        t = grow[f];
+        const double trail = __dmul_rn(__dmul_rn((double)(dim - f - 1), f_init), f_init);
+        int epoch = 0;
+        while (epoch < min_epochs || rmse <= __dadd_rn(rmse_last, -min_improvement)) {
+            double se = 0.0;
+            rmse_last = rmse;
+            double o[kAhead], s[kAhead], r[kAhead];
+#pragma unroll
+            for (int i = 0; i < kAhead; ++i) load(i, o[i], s[i], r[i]);
+            for (int n0 = 0; n0 < cnt; n0 += kAhead) {
+                double on[kAhead], sn[kAhead], rn[kAhead];
+#pragma unroll
+                for (int i = 0; i < kAhead; ++i) load(n0 + kAhead + i, on[i], sn[i], rn[i]);
+#pragma unroll
+                for (int i = 0; i < kAhead; ++i) {
+                    if (n0 + i < cnt) {
+                        const auto set_t = [&](double x) { t = x; };
+                        const auto frozen_side = [](double) {};
+                        const double e2 = SIDE == MFREC_FOLD_USERS
+                            ? funk_rating(r[i], s[i], s[i], trail, lr, K, o[i], t, 0, 1, frozen_side, set_t)
+                            : funk_rating(r[i], s[i], s[i], trail, lr, K, t, o[i], 1, 0, set_t, frozen_side);
+                        se = __dadd_rn(se, e2);
+                    }
+                    o[i] = on[i]; s[i] = sn[i]; r[i] = rn[i];
+                }
+            }
+            rmse = sqrt(se / (double)cnt);
+            ++epoch;
+        }
+        grow[f] = t;
+        feature_epochs[(size_t)j * dim + f] = epoch;
+        feature_rmse[(size_t)j * dim + f] = rmse;
     }
 }
 
@@ -616,5 +736,117 @@ extern "C" int mfrec_train_funk(mfrec_ctx *ctx, int variant, int min_epochs, int
     MF_CUDA(ctx, cudaStreamSynchronize(st));
     if (feature_epochs) memcpy(feature_epochs, h_fe.data(), (size_t)k * 4);
     if (feature_rmse) memcpy(feature_rmse, h_fr.data(), (size_t)k * 8);
+    return MFREC_OK;
+}
+
+extern "C" int mfrec_fold_in_funk(mfrec_ctx *ctx, int side, int min_epochs, double min_improvement, int k,
+                                  double f_init, double learning_rate, double K, double overall_avg,
+                                  double *u, double *v, const int32_t *ratings_index, const double *ratings,
+                                  int64_t nnz, int32_t ni, int32_t nu, const double *items_bias,
+                                  const double *users_bias, const int32_t *rows, int32_t n_rows,
+                                  int32_t *feature_epochs, double *feature_rmse)
+{
+    if (!ctx) return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "mfrec_fold_in_funk: NULL ctx");
+    if (!u || !v || !items_bias || !users_bias || (nnz > 0 && (!ratings_index || !ratings)) || (n_rows > 0 && !rows))
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_funk: NULL array");
+    if (side != MFREC_FOLD_USERS && side != MFREC_FOLD_ITEMS)
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_funk: side=%d", side);
+    if (k <= 0 || ni <= 0 || nu <= 0 || nnz < 0 || n_rows < 0)
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_funk: k=%d ni=%d nu=%d nnz=%lld rows=%d",
+                               k, ni, nu, (long long)nnz, n_rows);
+    const bool by_user = side == MFREC_FOLD_USERS;
+    const int tc = by_user ? 0 : 1;   // column of ratings_index naming the trained row; 1 - tc the frozen one
+    FoldSelection sel;
+    MF_TRY(sel.count(ctx, "mfrec_fold_in_funk", side, ratings_index, nnz, ni, nu, rows, n_rows));
+    const std::vector<int64_t> &rptr = sel.rptr;
+    for (int32_t p = 0; p < n_rows; ++p)
+        if (rptr[p + 1] == rptr[p])   // mfrec_train_funk refuses nnz = 0 too
+            return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG,
+                                   "mfrec_fold_in_funk: row %d (rows[%d]) has no ratings (the reference loops forever on 0/0)",
+                                   rows[p], p);
+    MF_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (n_rows == 0) return MFREC_OK;
+    const int64_t nsel = sel.nsel();
+    sel.gather(ratings_index, ratings, nnz);
+    // the listed rows and the frozen rows their ratings name, row-major (a lane reads whole rows)
+    FoldRows g;
+    g.gather(k, true, u, v, items_bias, users_bias, ni, nu, sel.idx.data(), nsel);
+    std::vector<double> &tf = by_user ? g.v : g.u;
+    const std::vector<double> &tb = by_user ? g.ub : g.ib, &ff = by_user ? g.u : g.v, &fbv = by_user ? g.ib : g.ub;
+
+    // jobs: the longest rows first (list order among equal counts), 32 to a block; a block's
+    // per-rating arrays are 32 x (its first job's count) long, lane-interleaved
+    std::vector<int32_t> order(n_rows);
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](int32_t a, int32_t b) {
+        return rptr[a + 1] - rptr[a] > rptr[b + 1] - rptr[b];
+    });
+    const int32_t n_blocks = (n_rows + 31) / 32;
+    std::vector<int64_t> warp_off((size_t)n_blocks + 1, 0);
+    for (int32_t w = 0; w < n_blocks; ++w) {
+        const int32_t p = order[(size_t)w * 32];
+        warp_off[w + 1] = warp_off[w] + 32 * (rptr[p + 1] - rptr[p]);
+    }
+    const int64_t slots = warp_off[n_blocks];
+    std::vector<int32_t> job_row(n_rows), job_cnt(n_rows), fidx(slots, 0);
+    std::vector<double> rv(slots, 0.0);
+    for (int32_t j = 0; j < n_rows; ++j) {
+        const int32_t p = order[j];
+        const int64_t a = rptr[p], q0 = warp_off[j / 32] + (j % 32);
+        job_row[j] = g.idx[2 * a + tc];
+        job_cnt[j] = (int32_t)(rptr[p + 1] - a);
+        for (int64_t n = 0; n < job_cnt[j]; ++n) {
+            fidx[q0 + 32 * n] = g.idx[2 * (a + n) + 1 - tc];
+            rv[q0 + 32 * n] = sel.r[a + n];
+        }
+    }
+
+    cudaStream_t st = ctx->stream;
+    DevBuf<double> d_tf, d_tb, d_ff, d_fb, d_rv, d_base, d_so, d_ss, d_fr;
+    DevBuf<int32_t> d_row, d_cnt, d_fidx, d_fe;
+    DevBuf<int64_t> d_off;
+    MF_CUDA(ctx, d_tf.alloc(tf.size(), st));
+    MF_CUDA(ctx, d_tb.alloc(tb.size(), st));
+    MF_CUDA(ctx, d_ff.alloc(ff.size(), st));
+    MF_CUDA(ctx, d_fb.alloc(fbv.size(), st));
+    MF_CUDA(ctx, d_rv.alloc(slots, st));
+    MF_CUDA(ctx, d_base.alloc(slots, st));
+    MF_CUDA(ctx, d_so.alloc(slots, st));
+    MF_CUDA(ctx, d_ss.alloc(slots, st));
+    MF_CUDA(ctx, d_fidx.alloc(slots, st));
+    MF_CUDA(ctx, d_row.alloc(n_rows, st));
+    MF_CUDA(ctx, d_cnt.alloc(n_rows, st));
+    MF_CUDA(ctx, d_off.alloc((size_t)n_blocks + 1, st));
+    MF_CUDA(ctx, d_fe.alloc((size_t)n_rows * k, st));
+    MF_CUDA(ctx, d_fr.alloc((size_t)n_rows * k, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_tf.p, tf.data(), tf.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_tb.p, tb.data(), tb.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_ff.p, ff.data(), ff.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_fb.p, fbv.data(), fbv.size() * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_rv.p, rv.data(), (size_t)slots * 8, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_fidx.p, fidx.data(), (size_t)slots * 4, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_row.p, job_row.data(), (size_t)n_rows * 4, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_cnt.p, job_cnt.data(), (size_t)n_rows * 4, cudaMemcpyHostToDevice, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(d_off.p, warp_off.data(), ((size_t)n_blocks + 1) * 8, cudaMemcpyHostToDevice, st));
+    auto launch = by_user ? funk_fold_in_kernel<MFREC_FOLD_USERS> : funk_fold_in_kernel<MFREC_FOLD_ITEMS>;
+    launch<<<n_blocks, 32, 0, st>>>(min_epochs, min_improvement, k, f_init, learning_rate, K, overall_avg,
+                                    d_tf.p, d_tb.p, d_ff.p, d_fb.p, d_row.p, d_cnt.p, d_off.p, d_fidx.p, d_rv.p,
+                                    d_base.p, d_so.p, d_ss.p, n_rows, d_fe.p, d_fr.p);
+    MF_LAUNCH_CHECK(ctx);
+    std::vector<int32_t> h_fe((size_t)n_rows * k);
+    std::vector<double> h_fr((size_t)n_rows * k);
+    MF_CUDA(ctx, cudaMemcpyAsync(tf.data(), d_tf.p, tf.size() * 8, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(h_fe.data(), d_fe.p, h_fe.size() * 4, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(ctx, cudaMemcpyAsync(h_fr.data(), d_fr.p, h_fr.size() * 8, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(ctx, cudaStreamSynchronize(st));
+    // only the listed rows go back: the frozen side, both bias arrays and every unlisted row are
+    // never written
+    if (by_user) g.scatter(nullptr, v, nullptr, nullptr, ni, nu);
+    else g.scatter(u, nullptr, nullptr, nullptr, ni, nu);
+    for (int32_t j = 0; j < n_rows; ++j) {
+        const size_t p = order[j];
+        if (feature_epochs) std::copy(h_fe.begin() + (size_t)j * k, h_fe.begin() + (size_t)(j + 1) * k, feature_epochs + p * k);
+        if (feature_rmse) std::copy(h_fr.begin() + (size_t)j * k, h_fr.begin() + (size_t)(j + 1) * k, feature_rmse + p * k);
+    }
     return MFREC_OK;
 }

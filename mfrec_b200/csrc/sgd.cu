@@ -46,6 +46,7 @@
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "fold.h"
 
 namespace {
 
@@ -1744,64 +1745,6 @@ extern "C" int mfrec_ring_sync_model(mfrec_ring *g)
     return MFREC_OK;
 }
 
-// The rows a fold-in's ratings name, copied out of the caller's full arrays into compact ones and
-// back (KMFRecommender.retrain_user / retrain_item / add_user, kmf.py:120-172, name a handful of
-// rows: only those move, so the untouched rest of u / v / the biases stays bit-identical like in the
-// reference).  users / items: the distinct ids the ratings name, sorted; idx: ratings_index
-// renumbered into them.  Compact factors are [k][m] like the caller's, or [m][k] with row_major.
-struct FoldRows {
-    int k = 0;
-    bool row_major = false;
-    std::vector<int32_t> users, items, idx;
-    std::vector<double> u, v, ib, ub;
-
-    static std::vector<int32_t> distinct(const int32_t *ratings_index, int64_t nnz, int col)
-    {
-        std::vector<int32_t> ids(nnz);
-        for (int64_t n = 0; n < nnz; ++n) ids[n] = ratings_index[2 * n + col];
-        std::sort(ids.begin(), ids.end());
-        ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
-        return ids;
-    }
-    size_t at(size_t m, size_t a, int f) const { return row_major ? a * k + f : (size_t)f * m + a; }
-
-    void gather(int k_, bool row_major_, const double *u_, const double *v_, const double *ib_,
-                const double *ub_, int32_t ni, int32_t nu, const int32_t *ratings_index, int64_t nnz)
-    {
-        k = k_;
-        row_major = row_major_;
-        users = distinct(ratings_index, nnz, 0);
-        items = distinct(ratings_index, nnz, 1);
-        const size_t mu = users.size(), mi = items.size();
-        u.resize((size_t)k * mi);
-        v.resize((size_t)k * mu);
-        ib.resize(mi);
-        ub.resize(mu);
-        for (int f = 0; f < k; ++f) {
-            for (size_t a = 0; a < mi; ++a) u[at(mi, a, f)] = u_[(size_t)f * ni + items[a]];
-            for (size_t a = 0; a < mu; ++a) v[at(mu, a, f)] = v_[(size_t)f * nu + users[a]];
-        }
-        for (size_t a = 0; a < mi; ++a) ib[a] = ib_[items[a]];
-        for (size_t a = 0; a < mu; ++a) ub[a] = ub_[users[a]];
-        idx.resize((size_t)2 * nnz);
-        for (int64_t n = 0; n < nnz; ++n) {
-            idx[2 * n] = (int32_t)(std::lower_bound(users.begin(), users.end(), ratings_index[2 * n]) - users.begin());
-            idx[2 * n + 1] = (int32_t)(std::lower_bound(items.begin(), items.end(), ratings_index[2 * n + 1]) - items.begin());
-        }
-    }
-    // writes the compact rows back into every non-null array
-    void scatter(double *u_, double *v_, double *ib_, double *ub_, int32_t ni, int32_t nu) const
-    {
-        const size_t mu = users.size(), mi = items.size();
-        for (int f = 0; f < k; ++f) {
-            if (u_) for (size_t a = 0; a < mi; ++a) u_[(size_t)f * ni + items[a]] = u[at(mi, a, f)];
-            if (v_) for (size_t a = 0; a < mu; ++a) v_[(size_t)f * nu + users[a]] = v[at(mu, a, f)];
-        }
-        if (ib_) for (size_t a = 0; a < mi; ++a) ib_[items[a]] = ib[a];
-        if (ub_) for (size_t a = 0; a < mu; ++a) ub_[users[a]] = ub[a];
-    }
-};
-
 static int train_kmf_sequential(mfrec_ctx *ctx, int kernel, int nbr_epochs, int k, double lr,
                                 double K_users, double K_items, double K_bias, double *u, double *v,
                                 const int32_t *idx, const double *ratings, int64_t nnz, int32_t ni,
@@ -2023,35 +1966,10 @@ extern "C" int mfrec_fold_in_kmf(mfrec_ctx *ctx, int kernel, int side, int nbr_e
                                k, ni, nu, (long long)nnz, nbr_epochs, n_rows);
     const bool by_user = side == MFREC_FOLD_USERS, linear = kernel == MFREC_KERNEL_LINEAR;
     const int tc = by_user ? 0 : 1;   // column of ratings_index naming the trained row; 1 - tc the frozen one
-    const int32_t n_side = by_user ? nu : ni, n_other = by_user ? ni : nu;
-
-    // list position of every trained-side row (-1: not listed)
-    std::vector<int32_t> pos(n_side, -1);
-    for (int32_t p = 0; p < n_rows; ++p) {
-        const int32_t r = rows[p];
-        if (r < 0 || r >= n_side)
-            return mfrec_set_error(ctx, MFREC_ERR_INDEX, "mfrec_fold_in_kmf: rows[%d] = %d outside [0, %d)", p, r, n_side);
-        if (pos[r] >= 0)
-            return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_fold_in_kmf: row %d is listed twice (%d, %d)", r, pos[r], p);
-        pos[r] = p;
-    }
-    auto listed = [&](int64_t n) {
-        const int32_t t = ratings_index[2 * n + tc];
-        return t >= 0 && t < n_side ? pos[t] : -1;
-    };
-    // every listed row's ratings in input order: a stable counting sort by list position
-    std::vector<int64_t> rptr((size_t)n_rows + 1, 0);
-    for (int64_t n = 0; n < nnz; ++n) {
-        const int32_t p = listed(n);
-        if (p < 0) continue;
-        const int32_t o = ratings_index[2 * n + 1 - tc];
-        if (o < 0 || o >= n_other)
-            return mfrec_set_error(ctx, MFREC_ERR_INDEX, "mfrec_fold_in_kmf: rating %lld has (user,item)=(%d,%d)",
-                                   (long long)n, ratings_index[2 * n], ratings_index[2 * n + 1]);
-        ++rptr[p + 1];
-    }
-    for (int32_t p = 0; p < n_rows; ++p) rptr[p + 1] += rptr[p];
-    const int64_t nsel = rptr[n_rows];
+    FoldSelection sel;
+    MF_TRY(sel.count(ctx, "mfrec_fold_in_kmf", side, ratings_index, nnz, ni, nu, rows, n_rows));
+    const std::vector<int64_t> &rptr = sel.rptr;
+    const int64_t nsel = sel.nsel();
     MF_CUDA(ctx, cudaSetDevice(ctx->device));
     if (nbr_epochs == 0) return MFREC_OK;
     if (rmse)   // a row without ratings: the reference divides 0/0 and leaves the model untouched
@@ -2059,22 +1977,11 @@ extern "C" int mfrec_fold_in_kmf(mfrec_ctx *ctx, int kernel, int side, int nbr_e
             if (rptr[p + 1] == rptr[p])
                 for (int e = 0; e < nbr_epochs; ++e) rmse[(size_t)p * nbr_epochs + e] = NAN;
     if (nsel == 0) return MFREC_OK;
-    std::vector<int32_t> sidx((size_t)2 * nsel);
-    std::vector<double> sr(nsel);
-    {
-        std::vector<int64_t> cur(rptr.begin(), rptr.end() - 1);
-        for (int64_t n = 0; n < nnz; ++n) {
-            const int32_t p = listed(n);
-            if (p < 0) continue;
-            const int64_t s = cur[p]++;
-            sidx[2 * s] = ratings_index[2 * n];
-            sidx[2 * s + 1] = ratings_index[2 * n + 1];
-            sr[s] = ratings[n];
-        }
-    }
+    sel.gather(ratings_index, ratings, nnz);
+    const std::vector<double> &sr = sel.r;
     // the listed rows and the frozen rows their ratings name, row-major (a lane reads whole rows)
     FoldRows g;
-    g.gather(k, true, u, v, items_bias, users_bias, ni, nu, sidx.data(), nsel);
+    g.gather(k, true, u, v, items_bias, users_bias, ni, nu, sel.idx.data(), nsel);
     std::vector<double> &tf = by_user ? g.v : g.u, &tb = by_user ? g.ub : g.ib, &fbv = by_user ? g.ib : g.ub;
     const std::vector<double> &ff = by_user ? g.u : g.v;
     const size_t n_frozen = by_user ? g.items.size() : g.users.size();

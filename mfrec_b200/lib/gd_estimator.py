@@ -54,6 +54,44 @@ def _train(variant, min_epochs, max_epochs, min_improvement, dim, f_init, learni
     return None
 
 
+def fold_in(side, min_epochs, min_improvement, dim, f_init, learning_rate, K, overall_avg, u, v,
+            ratings_index, ratings, items_bias, users_bias, rows, verbose=0):
+    """Many fold-ins in one device call (not in the reference): the same result, bit for bit, as
+    calling ``estimator_loop_with_bias_dev`` once per listed row, in list order, on the ratings naming
+    that row, with ``update_users, update_items = 1, 0`` (``side`` = ``_native.FOLD_USERS``) or
+    ``0, 1`` (``_native.FOLD_ITEMS``) under the sequential schedule -- what
+    ``GDRecommender.retrain_user`` / ``retrain_item`` do.  The batch always runs the reference's order,
+    whatever ``options["schedule"]`` says.  Every listed row needs at least one rating.  ``verbose``
+    prints what those calls would, row by row, and ``last_feature_epochs`` / ``last_feature_rmse`` are
+    left as the last of them leaves them.  Returns (feature_epochs [n_rows, dim], feature_rmse
+    [n_rows, dim])."""
+    global last_feature_epochs, last_feature_rmse
+    dim = int(dim)
+    buffer_arg(u, "u", np.float64, 2)
+    buffer_arg(v, "v", np.float64, 2)
+    buffer_arg(ratings_index, "ratings_index", np.int32, 2, writable=False)
+    buffer_arg(ratings, "ratings", np.float64, 1, writable=False)
+    buffer_arg(items_bias, "items_bias", np.float64, 1, writable=False)
+    buffer_arg(users_bias, "users_bias", np.float64, 1, writable=False)
+    check_rating_arrays(u, v, ratings_index, ratings, items_bias, users_bias)
+    if dim > u.shape[0] or dim > v.shape[0] or dim < 0:
+        raise ValueError("dim=%d exceeds the factor arrays (%d, %d features)" % (dim, u.shape[0], v.shape[0]))
+    rows = np.ascontiguousarray(rows, dtype=np.int32).reshape(-1)
+    if rows.shape[0] == 0 or dim == 0:
+        return np.zeros((rows.shape[0], dim), dtype=np.int32), np.zeros((rows.shape[0], dim))
+    fe, fr = _native.fold_in_funk(
+        side, int(min_epochs), float(min_improvement), dim, float(f_init), float(learning_rate), float(K),
+        float(overall_avg), u[:dim], v[:dim], ratings_index, ratings, items_bias, users_bias, rows,
+        ctx=_native.default_context(options["device"]))
+    last_feature_epochs, last_feature_rmse = fe[-1].copy(), fr[-1].copy()
+    if verbose:
+        for p in range(rows.shape[0]):
+            for f in range(dim):
+                print("Training the feature " + str(f))
+                print("RMSE: " + str(fr[p, f]) + "\n")
+    return fe, fr
+
+
 def estimator_loop_without_bias(min_epochs, max_epochs, min_improvement, dim, f_init,
                                 learning_rate, K, u, v, ratings_index, ratings, nbr_users,
                                 nbr_items, verbose=0):

@@ -6,8 +6,9 @@
 reference's Cython module."""
 import numpy as np
 
+from mfrec_b200 import _native
 from mfrec_b200.lib import gd_estimator
-from mfrec_b200.recommendation.mf import MFRecommender
+from mfrec_b200.recommendation.mf import MFRecommender, _fold_ratings, _fold_rows
 
 
 class GDRecommender(MFRecommender):
@@ -180,3 +181,41 @@ class GDRecommender(MFRecommender):
         valid_ids = np.where(ratings_index[:, 1] == item_index)[0]
         self.init_item_features(item_index)
         self._retrain(valid_ids, ratings_index, ratings, 0, 1, verbose)
+
+    # ---- batched fold-in (not in the reference): one device call for many rows ----------------------
+    # Each leaves the recommender exactly as the loop of the single-row method over the same rows
+    # leaves it when gd_estimator.options["schedule"] is "sequential" -- the reference's own order:
+    # svd_u, svd_v, the untouched biases, the numpy RNG (the rows' initial features are drawn in list
+    # order before the one native call; training draws nothing), what verbose prints and
+    # gd_estimator.last_feature_epochs / last_feature_rmse.  The batch always runs that order; under
+    # the default stratified schedule the single-row calls order each row's ratings differently and
+    # agree with the batch to float tolerance only.  Everything is validated before anything changes
+    # or is drawn: rows must be distinct and in range, and every row needs at least one rating (the
+    # loop would train the rows before such a row and then raise; the batch raises up front).
+    def retrain_users(self, user_indices, ratings_index, ratings, verbose=False):
+        """``for u in user_indices: self.retrain_user(u, ratings_index, ratings, verbose)``."""
+        rows = _fold_rows(user_indices, self.nbr_users)
+        if rows.shape[0]:
+            idx, r = _fold_ratings(rows, 0, self.nbr_items, ratings_index, ratings)
+            self._fold_in_batch(_native.FOLD_USERS, rows, idx, r, verbose)
+
+    def retrain_items(self, item_indices, ratings_index, ratings, verbose=False):
+        """``for i in item_indices: self.retrain_item(i, ratings_index, ratings, verbose)``."""
+        rows = _fold_rows(item_indices, self.nbr_items)
+        if rows.shape[0]:
+            idx, r = _fold_ratings(rows, 1, self.nbr_users, ratings_index, ratings)
+            self._fold_in_batch(_native.FOLD_ITEMS, rows, idx, r, verbose)
+
+    def _fold_in_batch(self, side, rows, ratings_index, ratings, verbose):
+        col = 0 if side == _native.FOLD_USERS else 1
+        rated = np.isin(rows, ratings_index[:, col])
+        if not rated.all():
+            raise ValueError('%s %d has no ratings to train on' % ('user' if col == 0 else 'item', rows[~rated][0]))
+        init = self.init_user_features if side == _native.FOLD_USERS else self.init_item_features
+        for row in rows:
+            init(row)
+        gd_estimator.fold_in(side, self.min_epochs, self.min_improvement, self.dimensionality,
+                             self.feature_init, self.learning_rate, self.K, self.overall_bias, self.svd_u,
+                             self.svd_v, ratings_index, ratings, self.items_bias, self.users_bias, rows,
+                             int(verbose))
+        self.invalidate_model()   # a few rows changed in place: the sampled fingerprint may miss them

@@ -7,9 +7,8 @@ import numpy as np
 
 from mfrec_b200 import _native
 from mfrec_b200.lib import kmf_train
-from mfrec_b200.lib._buffers import buffer_arg
 from mfrec_b200.recommendation.base import Error
-from mfrec_b200.recommendation.mf import MFRecommender
+from mfrec_b200.recommendation.mf import MFRecommender, _fold_ratings, _fold_rows
 
 _KERNELS = {'train_logistic_kernel': kmf_train.train_logistic_kernel,
             'train_linear_kernel': kmf_train.train_linear_kernel}
@@ -196,33 +195,3 @@ class KMFRecommender(MFRecommender):
                           ratings, self.items_bias, self.users_bias, rows, int(verbose))
         self.invalidate_model()   # a few rows changed in place: the sampled fingerprint may miss them
 
-
-def _fold_rows(indices, n):
-    """The listed rows as int64: in [0, n) (IndexError) and distinct (ValueError)."""
-    rows = np.asarray(indices).reshape(-1)
-    if rows.shape[0] and not np.issubdtype(rows.dtype, np.integer):
-        raise IndexError('row indices must be integers, got %s' % rows.dtype)
-    rows = rows.astype(np.int64)
-    bad = (rows < 0) | (rows >= n)
-    if bad.any():
-        raise IndexError('row %d is outside [0, %d)' % (rows[bad][0], n))
-    if np.unique(rows).shape[0] != rows.shape[0]:
-        raise ValueError('a row is listed more than once')
-    return rows
-
-
-def _fold_ratings(rows, col, n_other, ratings_index, ratings):
-    """The ratings naming a listed row (column ``col``), in input order, checked like the single-row
-    calls check theirs: int32 / float64 buffers (ValueError), the other index in [0, n_other)
-    (IndexError)."""
-    ids = np.nonzero(np.isin(ratings_index[:, col], rows))[0]
-    idx = np.ascontiguousarray(ratings_index[ids, :])
-    r = np.ascontiguousarray(ratings[ids])
-    buffer_arg(idx, "ratings_index", np.int32, 2, writable=False)
-    buffer_arg(r, "ratings", np.float64, 1, writable=False)
-    other = idx[:, 1 - col]
-    bad = (other < 0) | (other >= n_other)
-    if bad.any():
-        raise IndexError('rating (user, item) = (%d, %d) names no %s' % (idx[bad][0, 0], idx[bad][0, 1],
-                                                                         'item' if col == 0 else 'user'))
-    return idx, r

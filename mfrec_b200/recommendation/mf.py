@@ -3,6 +3,7 @@
 import numpy as np
 
 from mfrec_b200 import _native
+from mfrec_b200.lib._buffers import buffer_arg
 from mfrec_b200.recommendation.base import BaseRecommender
 
 
@@ -241,3 +242,35 @@ class MFRecommender(BaseRecommender):
             if getattr(type(self), name, None) is target:
                 return name
         raise KeyError(predictor)
+
+
+# ---- batched fold-in: argument checks shared by KMFRecommender and GDRecommender ------------------
+def _fold_rows(indices, n):
+    """The listed rows as int64: in [0, n) (IndexError) and distinct (ValueError)."""
+    rows = np.asarray(indices).reshape(-1)
+    if rows.shape[0] and not np.issubdtype(rows.dtype, np.integer):
+        raise IndexError('row indices must be integers, got %s' % rows.dtype)
+    rows = rows.astype(np.int64)
+    bad = (rows < 0) | (rows >= n)
+    if bad.any():
+        raise IndexError('row %d is outside [0, %d)' % (rows[bad][0], n))
+    if np.unique(rows).shape[0] != rows.shape[0]:
+        raise ValueError('a row is listed more than once')
+    return rows
+
+
+def _fold_ratings(rows, col, n_other, ratings_index, ratings):
+    """The ratings naming a listed row (column ``col``), in input order, checked like the single-row
+    calls check theirs: int32 / float64 buffers (ValueError), the other index in [0, n_other)
+    (IndexError)."""
+    ids = np.nonzero(np.isin(ratings_index[:, col], rows))[0]
+    idx = np.ascontiguousarray(ratings_index[ids, :])
+    r = np.ascontiguousarray(ratings[ids])
+    buffer_arg(idx, "ratings_index", np.int32, 2, writable=False)
+    buffer_arg(r, "ratings", np.float64, 1, writable=False)
+    other = idx[:, 1 - col]
+    bad = (other < 0) | (other >= n_other)
+    if bad.any():
+        raise IndexError('rating (user, item) = (%d, %d) names no %s' % (idx[bad][0, 0], idx[bad][0, 1],
+                                                                         'item' if col == 0 else 'user'))
+    return idx, r

@@ -300,7 +300,11 @@ int mfrec_bias_stats(mfrec_ctx *ctx, const int32_t *ratings_index, const double 
  * implicit-feedback WRMF, float64, u [k][nbr_items] and v [k][nbr_users] updated in place.
  * users_row / items_row are the reference's own arrays (mfrec/lib/datasets.py:13-32):
  * [0, count_0, count_1, ...] with n_*_row entries, i.e. n_*_row - 1 active rows; *_col hold the
- * neighbour ids in row order.  c_pos and reg are the reference's c_pos and k arguments. */
+ * neighbour ids in row order.  c_pos and reg are the reference's c_pos and k arguments.
+ * k may be 1..256, the library-wide limit (as mfrec_model_create); k > 256 is
+ * MFREC_ERR_UNSUPPORTED.  Where a row's k x k system fits one CTA's shared memory (k <= 165 with
+ * 227 KB per block) one CTA solves it; above that a cluster of CTAs holds it in distributed shared
+ * memory.  The choice follows from k and the device alone; both are deterministic. */
 int mfrec_train_als_wrmf(mfrec_ctx *ctx, int nbr_epochs, int k, double *u, double *v,
                          const int32_t *users_row, int64_t n_users_row, const int32_t *users_col,
                          const int32_t *items_row, int64_t n_items_row, const int32_t *items_col,

@@ -10,7 +10,8 @@
 //               v_j = M^-1 b                        (als_implicit.pyx:257-306)
 //   item pass:  the same with the roles swapped, on the UPDATED V   (:308-352)
 // Inside a pass the rows are independent, so one CTA solves one row: M is assembled in shared
-// memory (k^2 doubles: k <= 160), factorised by Cholesky (M is symmetric positive definite:
+// memory (k^2 doubles: k <= 165 with 227 KB per block; above that, up to k = 256, a cluster of CTAs
+// shares M, see als_cluster_solve_kernel), factorised by Cholesky (M is symmetric positive definite:
 // Gram matrices plus reg > 0) and solved by two triangular sweeps.  The reference inverts M with
 // numpy.linalg.inv and multiplies; the two agree to float64 round-off for these well-conditioned
 // systems (tests compare at 1e-9).  Everything is float64: this is a dense small-matrix problem
@@ -210,6 +211,221 @@ als_solve_kernel(const double *__restrict__ X, const double *__restrict__ HH, co
     for (int f = tid; f < k; f += nt) Y[(int64_t)j * k + f] = b[f];
 }
 
+// ---- cluster row solver: k where one CTA's shared memory cannot hold M (k > 165 at 227 KB) ----------
+// One thread-block cluster of C CTAs per active row.  M lives in distributed shared memory, its rows
+// dealt row-cyclically (CTA `rank` owns rows rank, rank + C, ...), so that every CTA keeps a near-equal
+// share of the shrinking trailing update.  Each CTA
+//   1. assembles its own rows of M = HH + c_pos * sum x x^T + reg I (lower triangle and the
+//      diagonal 64-column block; nothing above is read) and its entries of b, staging every
+//      neighbour row itself;
+//   2. factorises M = L L^T right-looking with the forward solve L y = b riding along: for column c
+//      every CTA pushes the RAW entries M[r][c] of its rows r >= c (and the owner of row c pushes
+//      b[c]) into every CTA's column buffer, one cluster barrier, then every CTA derives
+//      d = sqrt(M[c][c]), L[:, c] = M[:, c] / d and y[c] = b[c] / d itself -- the same operations
+//      on the same operands everywhere -- and updates its own rows.  Column c + 1 of its rows is
+//      updated and pushed first (look-ahead), so that the barrier's round trip overlaps the rest
+//      of the trailing update.  Column buffers and the local copy of L's column alternate between
+//      two slots: a CTA can be at most one column ahead of the slowest;
+//   3. CTA 0 solves L^T x = y, copying L's rows out of the other CTAs' shared memory in blocks of
+//      kTile rows, and writes Y[j].
+// Neighbour rows are staged with coalesced loads, not bulk copies: a row is k * 8 bytes at k * 8-byte
+// offsets, which the bulk copy's 16-byte rule excludes for odd k.
+constexpr int kClusterThreads = 256;
+constexpr int kClusterMax = 8;   // portable cluster size
+
+__device__ __forceinline__ uint32_t cluster_ctarank()
+{
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
+__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
+// generic address of the same shared-memory location in CTA `rank` of the cluster
+__device__ __forceinline__ double *cluster_map(double *p, uint32_t rank)
+{
+    uint64_t q;
+    asm volatile("mapa.u64 %0, %1, %2;" : "=l"(q) : "l"(p), "r"(rank));
+    return reinterpret_cast<double *>(q);
+}
+
+// staged-row pitch: whole 64-column blocks of the Gram tiles (the padding is zero)
+__host__ __device__ inline int als_cluster_pitch(int k) { return ((k + 63) / 64) * 64; }
+// shared memory per CTA: own rows of M [nr][k], b [nr], column buffers [2][k + 1], L's column [2][k],
+// y [k], staged rows [kTile][pitch]
+__host__ __device__ inline size_t als_cluster_smem(int k, int C, int kTile)
+{
+    const size_t nr = (size_t)(k + C - 1) / C;
+    return (nr * k + nr + 2 * (size_t)(k + 1) + 2 * (size_t)k + k + (size_t)kTile * als_cluster_pitch(k)) * sizeof(double);
+}
+
+__global__ void __launch_bounds__(kClusterThreads, 1)
+als_cluster_solve_kernel(const double *__restrict__ X, const double *__restrict__ HH, const int64_t *__restrict__ off,
+                         const int32_t *__restrict__ col, int k, double c_pos, double reg, double *__restrict__ Y,
+                         int kTile, int C)
+{
+    extern __shared__ double sm[];
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const int warp = tid >> 5, lane = tid & 31, nwarp = nt >> 5;
+    const int rank = (int)cluster_ctarank();
+    const int nr = (k + C - 1) / C;
+    const int nloc = (k - rank + C - 1) / C;   // own rows: i = rank + C * li, li < nloc
+    const int kp = als_cluster_pitch(k);
+    double *Ml = sm;                       // [nr][k]
+    double *bl = Ml + (size_t)nr * k;      // [nr]
+    double *colb = bl + nr;                // [2][k + 1]: raw M[:, c] by global row, raw b[c] at [k]
+    double *lcol = colb + 2 * (k + 1);     // [2][k]: L[:, c]
+    double *yv = lcol + 2 * k;             // [k]: y, then x
+    double *xs = yv + k;                   // [kTile][kp]: staged neighbour rows; rows of L in step 3
+    const int64_t j = blockIdx.x / C;
+    cluster_arrive();   // (waited for before the first push: every CTA of the cluster is running)
+
+    // 1. assembly
+    for (int e = tid; e < nloc * k; e += nt) {
+        const int li = e / k, c = e - li * k, i = rank + C * li;
+        double h = HH[(size_t)i * k + c];
+        if (c == i) h += reg;
+        Ml[e] = h;
+    }
+    for (int li = tid; li < nr; li += nt) bl[li] = 0.0;
+    for (int e = tid; e < kTile * (kp - k); e += nt) xs[(e / (kp - k)) * kp + k + e % (kp - k)] = 0.0;
+    // register tile: 4 own rows x 8 columns (c0 + 8 jj) of one 64-column block; blocks right of the
+    // tile's last row are skipped
+    const int ngr = (nloc + 3) / 4, ncb = kp / 64, ntile = ngr * ncb * 8;
+    const int64_t a = off[j], z = off[j + 1];
+    for (int64_t t0 = a; t0 < z; t0 += kTile) {
+        const int nrow = (int)min((int64_t)kTile, z - t0);
+        __syncthreads();
+        for (int r = warp; r < nrow; r += nwarp) {
+            const double *src = X + (int64_t)col[t0 + r] * k;
+            for (int f = lane; f < k; f += 32) xs[r * kp + f] = src[f];
+        }
+        __syncthreads();
+        for (int w = tid; w < ntile; w += nt) {
+            const int p = w >> 3, g = p / ncb, cb = p - g * ncb;
+            if (64 * cb > rank + C * min(4 * g + 3, nloc - 1)) continue;
+            const int c0 = 64 * cb + (w & 7);
+            int ri[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) ri[q] = rank + C * min(4 * g + q, nloc - 1);   // (past nloc: read, ignored)
+            double acc[4][8];
+#pragma unroll
+            for (int q = 0; q < 4; ++q)
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) acc[q][jj] = 0.0;
+            const double *xr = xs;
+            for (int r = 0; r < nrow; ++r, xr += kp) {
+                double rv[4], cv[8];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) rv[q] = xr[ri[q]];
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) cv[jj] = xr[c0 + 8 * jj];
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+#pragma unroll
+                    for (int jj = 0; jj < 8; ++jj) acc[q][jj] += rv[q] * cv[jj];
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q)
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) {
+                    const int li = 4 * g + q, c = c0 + 8 * jj;
+                    if (li < nloc && c < k) Ml[li * k + c] += c_pos * acc[q][jj];
+                }
+        }
+        for (int li = tid; li < nloc; li += nt) {
+            const int i = rank + C * li;
+            double acc = 0.0;
+            for (int r = 0; r < nrow; ++r) acc += xs[r * kp + i];
+            bl[li] += (1.0 + c_pos) * acc;
+        }
+    }
+    __syncthreads();
+
+    // 2. factorisation + forward solve
+    cluster_wait();
+    for (int li = tid; li < nloc; li += nt) {   // raw column 0
+        const int i = rank + C * li;
+        for (int q = 0; q < C; ++q) {
+            double *dst = cluster_map(colb, q);
+            dst[i] = Ml[li * k];
+            if (i == 0) dst[k] = bl[li];
+        }
+    }
+    cluster_arrive();
+    const int tr = tid >> 4, tc = tid & 15;   // 16 x 16 grid of the trailing update
+    for (int c = 0; c < k; ++c) {
+        cluster_wait();
+        const double *cb = colb + (c & 1) * (k + 1);
+        double *lc = lcol + (c & 1) * k;
+        const double d = sqrt(cb[c]);
+        const double yc = cb[k] / d;
+        for (int r = c + 1 + tid; r < k; r += nt) {
+            const double v = cb[r] / d;
+            lc[r] = v;
+            if (r % C == rank) Ml[(r / C) * k + c] = v;
+        }
+        if (tid == 0) {
+            yv[c] = yc;
+            if (c % C == rank) Ml[(c / C) * k + c] = d;
+        }
+        __syncthreads();
+        const int lb = c + 1 <= rank ? 0 : (c + 1 - rank + C - 1) / C;   // first own row > c
+        if (c + 1 < k) {   // look-ahead: column c + 1 of the own rows, pushed to every CTA
+            double *nb = colb + ((c + 1) & 1) * (k + 1);
+            const double lnext = lc[c + 1];
+            for (int li = lb + tid; li < nloc; li += nt) {
+                const int i = rank + C * li;
+                const double v = Ml[li * k + c + 1] - lc[i] * lnext;
+                Ml[li * k + c + 1] = v;
+                double bv = 0.0;
+                if (i == c + 1) bl[li] = bv = bl[li] - lc[i] * yc;
+                for (int q = 0; q < C; ++q) {
+                    double *dst = cluster_map(nb, q);
+                    dst[i] = v;
+                    if (i == c + 1) dst[k] = bv;
+                }
+            }
+            cluster_arrive();
+        }
+        for (int li = lb + tr; li < nloc; li += 16) {   // the rest: columns c + 2 .. i, b of rows > c + 1
+            const int i = rank + C * li;
+            const double lr = lc[i];
+            for (int c2 = c + 2 + tc; c2 <= i; c2 += 16) Ml[li * k + c2] -= lr * lc[c2];
+            if (tc == 15 && i > c + 1) bl[li] -= lr * yc;
+        }
+    }
+    cluster_arrive();   // L complete in every CTA
+    cluster_wait();
+
+    // 3. back substitution L^T x = y on CTA 0, as in als_solve_kernel, kTile rows of L at a time
+    if (rank == 0) {
+        for (int r1 = k - 1; r1 >= 0; r1 -= kTile) {
+            const int r0 = max(0, r1 - kTile + 1);
+            for (int r = r0 + warp; r <= r1; r += nwarp) {
+                const double *src = cluster_map(Ml + (size_t)(r / C) * k, r % C);
+#pragma unroll 4
+                for (int f = lane; f <= r; f += 32) xs[(r - r0) * kp + f] = src[f];
+            }
+            __syncthreads();
+            if (tid < 32) {
+                for (int r = r1; r >= r0; --r) {
+                    const double *Lr = xs + (r - r0) * kp;
+                    const double x = yv[r] / Lr[r];
+                    for (int c = lane; c < r; c += 32) yv[c] -= Lr[c] * x;
+                    __syncwarp();
+                    if (lane == 0) yv[r] = x;
+                    __syncwarp();
+                }
+            }
+            __syncthreads();
+        }
+        for (int f = tid; f < k; f += nt) Y[j * k + f] = yv[f];
+    }
+    cluster_arrive();   // the other CTAs keep their shared memory until CTA 0 has read it
+    cluster_wait();
+}
+
 int gram(mfrec_ctx *ctx, const double *X, int64_t n, int k, double *part, int nblocks, double *HH)
 {
     const int64_t rpb = (n + nblocks - 1) / nblocks;
@@ -253,9 +469,24 @@ extern "C" int mfrec_train_als_wrmf(mfrec_ctx *ctx, int nbr_epochs, int k, doubl
     // hide it better, as long as four CTAs still fit an SM
     int kTile = kTileMax;
     while (kTile > kTileMin && ((size_t)k * k + 2 * k + (size_t)kTile * als_pitch(k)) * sizeof(double) * 4 > ctx->smem_per_sm) kTile /= 2;
-    const size_t smem = ((size_t)k * k + 2 * k + (size_t)kTile * als_pitch(k)) * sizeof(double);
-    if (smem > ctx->smem_optin)
-        return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "mfrec_train_als_wrmf: k=%d needs %zu B of shared memory", k, smem);
+    size_t smem = ((size_t)k * k + 2 * k + (size_t)kTile * als_pitch(k)) * sizeof(double);
+    // k where M does not fit one CTA: the cluster solver, on the fewest CTAs whose shares fit, with as
+    // many staged rows as then fit
+    int csize = 1;
+    if (smem > ctx->smem_optin) {
+        if (k > 256)
+            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "mfrec_train_als_wrmf: k=%d > 256, the library-wide limit (as mfrec_model_create)", k);
+        cudaFuncAttributes fa;
+        MF_CUDA(ctx, cudaFuncGetAttributes(&fa, als_cluster_solve_kernel));
+        const size_t budget = ctx->smem_optin > fa.sharedSizeBytes ? ctx->smem_optin - fa.sharedSizeBytes : 0;
+        csize = 2;
+        while (csize < kClusterMax && als_cluster_smem(k, csize, kTileMin) > budget) ++csize;
+        kTile = kTileMax;
+        while (kTile > kTileMin && als_cluster_smem(k, csize, kTile) > budget) kTile /= 2;
+        smem = als_cluster_smem(k, csize, kTile);
+        if (smem > budget)
+            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "mfrec_train_als_wrmf: k=%d needs %zu B of shared memory on each of %d CTAs", k, smem, csize);
+    }
     if (nbr_epochs == 0) return MFREC_OK;
     const std::vector<int64_t> uoff = offsets_from_counts(users_row, n_users_row);
     const std::vector<int64_t> ioff = offsets_from_counts(items_row, n_items_row);
@@ -300,18 +531,47 @@ extern "C" int mfrec_train_als_wrmf(mfrec_ctx *ctx, int nbr_epochs, int k, doubl
     MF_CUDA(ctx, cudaMemcpyAsync(d_stage.p, v, (size_t)k * nbr_users * 8, cudaMemcpyHostToDevice, st));
     to_rows_f64_kernel<<<dim3((unsigned)ceil_div64(nbr_users, 32), (k + 31) / 32), 256, 0, st>>>(d_stage.p, k, nbr_users, d_V.p);
     MF_LAUNCH_CHECK(ctx);
-    MF_CUDA(ctx, cudaFuncSetAttribute(als_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaLaunchConfig_t ccfg = {};
+    cudaLaunchAttribute cattr[1];
+    if (csize == 1) {
+        MF_CUDA(ctx, cudaFuncSetAttribute(als_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    } else {
+        MF_CUDA(ctx, cudaFuncSetAttribute(als_cluster_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        cattr[0].id = cudaLaunchAttributeClusterDimension;
+        cattr[0].val.clusterDim.x = csize;
+        cattr[0].val.clusterDim.y = 1;
+        cattr[0].val.clusterDim.z = 1;
+        ccfg.gridDim = dim3(csize, 1, 1);
+        ccfg.blockDim = dim3(kClusterThreads, 1, 1);
+        ccfg.dynamicSmemBytes = smem;
+        ccfg.stream = st;
+        ccfg.attrs = cattr;
+        ccfg.numAttrs = 1;
+        int nclusters = 0;
+        MF_CUDA(ctx, cudaOccupancyMaxActiveClusters(&nclusters, als_cluster_solve_kernel, &ccfg));
+        if (nclusters < 1)
+            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "mfrec_train_als_wrmf: k=%d: a cluster of %d CTAs with %zu B of shared memory each does not fit the device", k, csize, smem);
+    }
+    // one pass: every active row of Y solved against the fixed X (HH = X^T X already computed)
+    auto solve = [&](const double *X, const int64_t *doff, const int32_t *dcol, int64_t rows, double *Y) -> int {
+        if (rows == 0) return MFREC_OK;
+        if (csize == 1) {
+            als_solve_kernel<<<(unsigned)rows, 128, smem, st>>>(X, d_HH.p, doff, dcol, k, (double)c_pos, reg, Y, kTile);
+        } else {
+            if (rows * csize > INT32_MAX)
+                return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "mfrec_train_als_wrmf: %lld rows x %d CTAs exceed one grid", (long long)rows, csize);
+            ccfg.gridDim = dim3((unsigned)(rows * csize), 1, 1);
+            MF_CUDA(ctx, cudaLaunchKernelEx(&ccfg, als_cluster_solve_kernel, X, (const double *)d_HH.p, doff, dcol, k,
+                                            (double)c_pos, reg, Y, kTile, csize));
+        }
+        MF_LAUNCH_CHECK(ctx);
+        return MFREC_OK;
+    };
     for (int e = 0; e < nbr_epochs; ++e) {
         MF_TRY(gram(ctx, d_U.p, nbr_items, k, d_part.p, nblocks, d_HH.p));
-        if (nau > 0) {
-            als_solve_kernel<<<(unsigned)nau, 128, smem, st>>>(d_U.p, d_HH.p, d_uoff.p, d_ucol.p, k, (double)c_pos, reg, d_V.p, kTile);
-            MF_LAUNCH_CHECK(ctx);
-        }
+        MF_TRY(solve(d_U.p, d_uoff.p, d_ucol.p, nau, d_V.p));
         MF_TRY(gram(ctx, d_V.p, nbr_users, k, d_part.p, nblocks, d_HH.p));
-        if (nai > 0) {
-            als_solve_kernel<<<(unsigned)nai, 128, smem, st>>>(d_V.p, d_HH.p, d_ioff.p, d_icol.p, k, (double)c_pos, reg, d_U.p, kTile);
-            MF_LAUNCH_CHECK(ctx);
-        }
+        MF_TRY(solve(d_V.p, d_ioff.p, d_icol.p, nai, d_U.p));
     }
     from_rows_f64_kernel<<<dim3((unsigned)ceil_div64(nbr_users, 32), (k + 31) / 32), 256, 0, st>>>(d_V.p, k, nbr_users, d_stage.p);
     MF_LAUNCH_CHECK(ctx);

@@ -213,6 +213,53 @@ user_threshold_kernel(const float *__restrict__ P, int kpad, int k, int ka, cons
     }
 }
 
+// The same thresholds where the [ka][ka] covariance does not fit one CTA's shared memory (ka > 240
+// with 227 KB per block): the covariance is formed once in global memory, as float values equal to
+// user_threshold_kernel's, and read from there through L2.  The covariance is exactly symmetric
+// (gram is written symmetrically, the mean product commutes), so a lane reads entry [g][f] for its
+// row f: neighbouring lanes read neighbouring floats, in the same order of g as the shared-memory
+// kernel, which therefore gives the same tau and eps.
+__global__ void __launch_bounds__(256)
+item_cov_kernel(const double *__restrict__ sum, const double *__restrict__ gram, int ka, int32_t nc, float *__restrict__ cov)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= ka * ka) return;
+    const int f = j / ka, g = j % ka;
+    cov[j] = (float)(gram[j] / nc - (sum[f] / nc) * (sum[g] / nc));
+}
+
+__global__ void __launch_bounds__(256)
+user_threshold_l2_kernel(const float *__restrict__ P, int kpad, int k, int ka, const int32_t *__restrict__ users,
+                         int64_t u0, int32_t n_users, int32_t nu, const double *__restrict__ sum,
+                         const float *__restrict__ cov, const float *__restrict__ qmax2, int32_t nc, float z,
+                         float *__restrict__ tau, float *__restrict__ eps)
+{
+    const int lane = threadIdx.x & 31;
+    const int w = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (w >= n_users) return;
+    const int64_t uid = users ? users[u0 + w] : u0 + w;
+    if (uid < 0 || uid >= nu) { if (lane == 0) { tau[w] = INFINITY; eps[w] = 0.f; } return; }
+    const float *p = P + uid * kpad;
+    float m = 0.f, var = 0.f, n2 = 0.f;
+    for (int f = lane; f < ka; f += 32) {
+        const float pf = f < k ? p[f] : 1.f;
+        float row = 0.f;
+        for (int g = 0; g < ka; ++g) row = fmaf(cov[g * ka + f], g < k ? p[g] : 1.f, row);
+        var = fmaf(pf, row, var);
+        m = fmaf(pf, (float)(sum[f] / nc), m);
+        n2 = fmaf(pf, pf, n2);
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        m += __shfl_xor_sync(0xffffffffu, m, o);
+        var += __shfl_xor_sync(0xffffffffu, var, o);
+        n2 += __shfl_xor_sync(0xffffffffu, n2, o);
+    }
+    if (lane == 0) {
+        tau[w] = m + z * sqrtf(fmaxf(var, 0.f));
+        eps[w] = 0.0078125f * sqrtf(n2) * sqrtf(*qmax2);
+    }
+}
+
 // ---- 3. the sweep -------------------------------------------------------------------------------
 struct SweepParams {
     const __nv_bfloat16 *A;     // [groups * NA][KB][128][64]   user tiles of this batch
@@ -802,6 +849,15 @@ extern "C" int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *M, int 
     }
     item_moments_kernel<<<dim3(ka, ka), 256, 0, st>>>(M->Q, M->ib, kpad, ka, k, nc, d_sum.p, d_gram.p, d_qmax2.p);
     MF_LAUNCH_CHECK(ctx);
+    // the per-user thresholds hold the covariance in shared memory where it fits, else read it through L2
+    const size_t smem_thr = ((size_t)ka * (ka | 1) + ka) * 4;
+    const bool thr_in_l2 = smem_thr > ctx->smem_optin;
+    DevBuf<float> d_cov;
+    if (thr_in_l2) {
+        MF_CUDA(ctx, d_cov.alloc((size_t)ka * ka, ctx->stream));
+        item_cov_kernel<<<(ka * ka + 255) / 256, 256, 0, st>>>(d_sum.p, d_gram.p, ka, nc, d_cov.p);
+        MF_LAUNCH_CHECK(ctx);
+    }
     {
         const int64_t chunks = (int64_t)n_btiles * KB * kBN * 8;
         pack_operand_kernel<kBN><<<(unsigned)ceil_div64(chunks, 256), 256, 0, st>>>(
@@ -827,12 +883,17 @@ extern "C" int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *M, int 
         const int nub = (int)std::min<int64_t>(batch, n_users - first);
         const int n_groups = (nub + group - 1) / group;
         cudaEventRecord(ev[2], st);
-        const size_t smem_thr = ((size_t)ka * (ka | 1) + ka) * 4;
-        if (smem_thr > 48 * 1024)
-            cudaFuncSetAttribute(user_threshold_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_thr);
-        user_threshold_kernel<<<(nub + 7) / 8, 256, smem_thr, st>>>(M->P, kpad, k, ka, users ? d_users.p : nullptr, first,
-                                                                   nub, nu, d_sum.p, d_gram.p, d_qmax2.p, nc, z,
-                                                                   d_tau.p, d_eps.p);
+        if (thr_in_l2) {
+            user_threshold_l2_kernel<<<(nub + 7) / 8, 256, 0, st>>>(M->P, kpad, k, ka, users ? d_users.p : nullptr, first,
+                                                                    nub, nu, d_sum.p, d_cov.p, d_qmax2.p, nc, z,
+                                                                    d_tau.p, d_eps.p);
+        } else {
+            if (smem_thr > 48 * 1024)
+                cudaFuncSetAttribute(user_threshold_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_thr);
+            user_threshold_kernel<<<(nub + 7) / 8, 256, smem_thr, st>>>(M->P, kpad, k, ka, users ? d_users.p : nullptr, first,
+                                                                       nub, nu, d_sum.p, d_gram.p, d_qmax2.p, nc, z,
+                                                                       d_tau.p, d_eps.p);
+        }
         MF_LAUNCH_CHECK(ctx);
         {
             const int64_t chunks = (int64_t)n_groups * NA * KB * 128 * 8;

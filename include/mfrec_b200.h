@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define MFREC_B200_ABI_VERSION 5
+#define MFREC_B200_ABI_VERSION 6
 
 typedef enum mfrec_status {
     MFREC_OK = 0,
@@ -309,6 +309,31 @@ int mfrec_train_als_wrmf(mfrec_ctx *ctx, int nbr_epochs, int k, double *u, doubl
                          const int32_t *users_row, int64_t n_users_row, const int32_t *users_col,
                          const int32_t *items_row, int64_t n_items_row, const int32_t *items_col,
                          int32_t nbr_users, int32_t nbr_items, int c_pos, double reg);
+
+/* mfrec_train_als_wrmf over SEVERAL shards driven by this process, with the same arrays, checks and
+ * status codes; the result equals mfrec_train_als_wrmf on devices[0] bit for bit.  devices: one CUDA
+ * device id per shard, n_shards <= 16; ids may repeat (each entry is its own shard with its own
+ * context, stream and copies of u and v, also when it shares a device).  Users and items are cut,
+ * separately, into n_shards contiguous ranges of active rows of near-equal estimated cost
+ * (deg * k^2 + k^3 / 3 per row; a range may be empty).  Every half-pass each shard computes the full
+ * HH of the fixed side itself, with the solver layout and Gram block count of devices[0], solves its
+ * range and stores every solution into every shard's copy (directly addressed peer memory between
+ * devices); an event per shard orders the half-passes.  No context argument: errors are reported
+ * through mfrec_last_error(NULL).  An empty device list or an id that is not a device is
+ * MFREC_ERR_BAD_ARG; two devices that cannot address each other's memory, or a device that cannot
+ * run devices[0]'s solver layout, are MFREC_ERR_UNSUPPORTED, before any launch.  u and v cross the
+ * host link once, to the first shard; the other shards copy them device to device.  Peer access is
+ * enabled for the call and disabled again where the call enabled it.  Peer access is process-wide, so
+ * the call is not safe to run concurrently with another user of peer mappings between the same
+ * devices (a ring, or a second multi-shard call): a mapping that this call enabled is removed when
+ * it returns.  Debug only: with the environment variable MFREC_ALS_SHARD_TIMES set to a file name, a
+ * call appends one JSON line to that file, every shard's row ranges and its milliseconds per
+ * half-pass (Gram + solve, CUDA events). */
+int mfrec_train_als_wrmf_multi(const int32_t *devices, int n_shards, int nbr_epochs, int k,
+                               double *u, double *v,
+                               const int32_t *users_row, int64_t n_users_row, const int32_t *users_col,
+                               const int32_t *items_row, int64_t n_items_row, const int32_t *items_col,
+                               int32_t nbr_users, int32_t nbr_items, int c_pos, double reg);
 
 /* ---- resident objects (what the one-call drop-ins are made of) ------------------- */
 

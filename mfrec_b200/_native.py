@@ -43,7 +43,7 @@ EXPORTS = (
     "mfrec_ring_create", "mfrec_ring_destroy", "mfrec_ring_handle", "mfrec_ring_connect",
     "mfrec_ring_connect_local", "mfrec_ring_epochs", "mfrec_ring_epochs_one_device", "mfrec_ring_wait",
     "mfrec_ring_sync_model", "mfrec_model_topn", "mfrec_model_topn_sweep", "mfrec_ratings_copies",
-    "mfrec_train_kmf_multi", "mfrec_fold_in_kmf", "mfrec_fold_in_funk",
+    "mfrec_train_kmf_multi", "mfrec_fold_in_kmf", "mfrec_fold_in_funk", "mfrec_train_als_wrmf_multi",
 )
 
 
@@ -311,6 +311,18 @@ def train_als_wrmf(nbr_epochs, k, u, v, users_row, users_col, items_row, items_c
         C.c_int64(users_row.shape[0]), _ptr(users_col), _ptr(items_row),
         C.c_int64(items_row.shape[0]), _ptr(items_col), C.c_int32(nbr_users), C.c_int32(nbr_items),
         C.c_int(int(c_pos)), C.c_double(float(reg))), ctx.handle)
+
+
+def train_als_wrmf_multi(devices, nbr_epochs, k, u, v, users_row, users_col, items_row, items_col, nbr_users,
+                         nbr_items, c_pos=1, reg=0.015):
+    """train_als_wrmf over several shards, one per entry of ``devices`` (ids may repeat); in place,
+    bit-identical to train_als_wrmf on ``devices[0]``."""
+    dev = np.ascontiguousarray(devices, dtype=np.int32).reshape(-1)
+    _check(lib().mfrec_train_als_wrmf_multi(
+        _ptr(dev) if dev.size else None, C.c_int(dev.shape[0]), C.c_int(nbr_epochs), C.c_int(k), _ptr(u), _ptr(v),
+        _ptr(users_row), C.c_int64(users_row.shape[0]), _ptr(users_col), _ptr(items_row),
+        C.c_int64(items_row.shape[0]), _ptr(items_col), C.c_int32(nbr_users), C.c_int32(nbr_items),
+        C.c_int(int(c_pos)), C.c_double(float(reg))), None)
 
 
 def _as(a, dtype):

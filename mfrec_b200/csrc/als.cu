@@ -20,6 +20,10 @@
 // The CSR-like inputs are the reference's own (mfrec/lib/datasets.py:13-32): row = [0, count_0,
 // count_1, ...] (counts, NOT offsets; the kernel loop accumulates them, als_implicit.pyx:266-268),
 // col = neighbour ids in row order.
+#include <algorithm>
+#include <cstdio>
+#include <cstdlib>
+#include <utility>
 #include <vector>
 
 #include "common.cuh"
@@ -103,9 +107,12 @@ __global__ void validate_cols_kernel(const int32_t *__restrict__ col, int64_t n,
 // register tiles below never leave the row (the padding is zero).
 __host__ __device__ inline int als_pitch(int k) { return ((k + 7) / 8) * 8; }
 
-__global__ void __launch_bounds__(128)
-als_solve_kernel(const double *__restrict__ X, const double *__restrict__ HH, const int64_t *__restrict__ off,
-                 const int32_t *__restrict__ col, int k, double c_pos, double reg, double *__restrict__ Y, int kTile)
+// The solve of row j = blockIdx.x (offsets off[j], off[j + 1]); store(j, f, x) writes feature f of its
+// solution.  Both instantiations (als_solve_kernel, als_solve_multi_kernel) share this code up to the store.
+template <class Store>
+__device__ __forceinline__ void als_solve_row(const double *__restrict__ X, const double *__restrict__ HH,
+                                              const int64_t *__restrict__ off, const int32_t *__restrict__ col, int k,
+                                              double c_pos, double reg, int kTile, Store store)
 {
     extern __shared__ double sm[];
     const int kp = als_pitch(k);
@@ -208,7 +215,31 @@ als_solve_kernel(const double *__restrict__ X, const double *__restrict__ HH, co
         }
     }
     __syncthreads();
-    for (int f = tid; f < k; f += nt) Y[(int64_t)j * k + f] = b[f];
+    for (int f = tid; f < k; f += nt) store(j, f, b[f]);
+}
+
+// the solved side of a multi-shard call lives once per shard: a solution goes to every copy
+constexpr int kAlsMaxShards = 16;
+struct AlsDst {
+    double *p[kAlsMaxShards];
+    int n;
+};
+
+__global__ void __launch_bounds__(128)
+als_solve_kernel(const double *__restrict__ X, const double *__restrict__ HH, const int64_t *__restrict__ off,
+                 const int32_t *__restrict__ col, int k, double c_pos, double reg, double *__restrict__ Y, int kTile)
+{
+    als_solve_row(X, HH, off, col, k, c_pos, reg, kTile, [&](int j, int f, double x) { Y[(int64_t)j * k + f] = x; });
+}
+
+// rows r0 + blockIdx.x (off / col cover this launch's rows only), stored into every copy in dst
+__global__ void __launch_bounds__(128)
+als_solve_multi_kernel(const double *__restrict__ X, const double *__restrict__ HH, const int64_t *__restrict__ off,
+                       const int32_t *__restrict__ col, int k, double c_pos, double reg, AlsDst dst, int64_t r0, int kTile)
+{
+    als_solve_row(X, HH, off, col, k, c_pos, reg, kTile, [&](int j, int f, double x) {
+        for (int q = 0; q < dst.n; ++q) dst.p[q][(r0 + j) * k + f] = x;
+    });
 }
 
 // ---- cluster row solver: k where one CTA's shared memory cannot hold M (k > 165 at 227 KB) ----------
@@ -259,10 +290,11 @@ __host__ __device__ inline size_t als_cluster_smem(int k, int C, int kTile)
     return (nr * k + nr + 2 * (size_t)(k + 1) + 2 * (size_t)k + k + (size_t)kTile * als_cluster_pitch(k)) * sizeof(double);
 }
 
-__global__ void __launch_bounds__(kClusterThreads, 1)
-als_cluster_solve_kernel(const double *__restrict__ X, const double *__restrict__ HH, const int64_t *__restrict__ off,
-                         const int32_t *__restrict__ col, int k, double c_pos, double reg, double *__restrict__ Y,
-                         int kTile, int C)
+// the cluster's solve of row j = blockIdx.x / C; CTA 0 calls store(j, f, x) for every feature f of the solution
+template <class Store>
+__device__ __forceinline__ void als_cluster_solve_row(const double *__restrict__ X, const double *__restrict__ HH,
+                                                      const int64_t *__restrict__ off, const int32_t *__restrict__ col,
+                                                      int k, double c_pos, double reg, int kTile, int C, Store store)
 {
     extern __shared__ double sm[];
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -420,10 +452,29 @@ als_cluster_solve_kernel(const double *__restrict__ X, const double *__restrict_
             }
             __syncthreads();
         }
-        for (int f = tid; f < k; f += nt) Y[j * k + f] = yv[f];
+        for (int f = tid; f < k; f += nt) store(j, f, yv[f]);
     }
     cluster_arrive();   // the other CTAs keep their shared memory until CTA 0 has read it
     cluster_wait();
+}
+
+__global__ void __launch_bounds__(kClusterThreads, 1)
+als_cluster_solve_kernel(const double *__restrict__ X, const double *__restrict__ HH, const int64_t *__restrict__ off,
+                         const int32_t *__restrict__ col, int k, double c_pos, double reg, double *__restrict__ Y,
+                         int kTile, int C)
+{
+    als_cluster_solve_row(X, HH, off, col, k, c_pos, reg, kTile, C, [&](int64_t j, int f, double x) { Y[j * k + f] = x; });
+}
+
+// rows r0 + blockIdx.x / C (off / col cover this launch's rows only), stored into every copy in dst
+__global__ void __launch_bounds__(kClusterThreads, 1)
+als_cluster_solve_multi_kernel(const double *__restrict__ X, const double *__restrict__ HH, const int64_t *__restrict__ off,
+                               const int32_t *__restrict__ col, int k, double c_pos, double reg, AlsDst dst, int64_t r0,
+                               int kTile, int C)
+{
+    als_cluster_solve_row(X, HH, off, col, k, c_pos, reg, kTile, C, [&](int64_t j, int f, double x) {
+        for (int q = 0; q < dst.n; ++q) dst.p[q][(r0 + j) * k + f] = x;
+    });
 }
 
 int gram(mfrec_ctx *ctx, const double *X, int64_t n, int k, double *part, int nblocks, double *HH)
@@ -449,6 +500,44 @@ std::vector<int64_t> offsets_from_counts(const int32_t *row, int64_t n_row)
     return off;
 }
 
+// The row solver of one device: staged neighbour rows per step, CTAs per row (1: als_solve_kernel,
+// more: als_cluster_solve_kernel) and dynamic shared memory per CTA.  A function of k and the device.
+struct AlsLayout {
+    int kTile = kTileMax;
+    int csize = 1;
+    size_t smem = 0;
+};
+
+int als_layout(mfrec_ctx *ctx, int k, const char *who, AlsLayout &L)
+{
+    // neighbour rows per staging step: the loads of a step are one L2 round trip, so more rows per step
+    // hide it better, as long as four CTAs still fit an SM
+    int kTile = kTileMax;
+    while (kTile > kTileMin && ((size_t)k * k + 2 * k + (size_t)kTile * als_pitch(k)) * sizeof(double) * 4 > ctx->smem_per_sm) kTile /= 2;
+    size_t smem = ((size_t)k * k + 2 * k + (size_t)kTile * als_pitch(k)) * sizeof(double);
+    // k where M does not fit one CTA: the cluster solver, on the fewest CTAs whose shares fit, with as
+    // many staged rows as then fit
+    int csize = 1;
+    if (smem > ctx->smem_optin) {
+        if (k > 256)
+            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "%s: k=%d > 256, the library-wide limit (as mfrec_model_create)", who, k);
+        cudaFuncAttributes fa;
+        MF_CUDA(ctx, cudaFuncGetAttributes(&fa, als_cluster_solve_kernel));
+        const size_t budget = ctx->smem_optin > fa.sharedSizeBytes ? ctx->smem_optin - fa.sharedSizeBytes : 0;
+        csize = 2;
+        while (csize < kClusterMax && als_cluster_smem(k, csize, kTileMin) > budget) ++csize;
+        kTile = kTileMax;
+        while (kTile > kTileMin && als_cluster_smem(k, csize, kTile) > budget) kTile /= 2;
+        smem = als_cluster_smem(k, csize, kTile);
+        if (smem > budget)
+            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "%s: k=%d needs %zu B of shared memory on each of %d CTAs", who, k, smem, csize);
+    }
+    L.kTile = kTile;
+    L.csize = csize;
+    L.smem = smem;
+    return MFREC_OK;
+}
+
 }  // namespace
 
 extern "C" int mfrec_train_als_wrmf(mfrec_ctx *ctx, int nbr_epochs, int k, double *u, double *v,
@@ -465,28 +554,10 @@ extern "C" int mfrec_train_als_wrmf(mfrec_ctx *ctx, int nbr_epochs, int k, doubl
     if (nau > nbr_users || nai > nbr_items)
         return mfrec_set_error(ctx, MFREC_ERR_INDEX, "mfrec_train_als_wrmf: more rows in the sparse structure than users / items");
     MF_CUDA(ctx, cudaSetDevice(ctx->device));
-    // neighbour rows per staging step: the loads of a step are one L2 round trip, so more rows per step
-    // hide it better, as long as four CTAs still fit an SM
-    int kTile = kTileMax;
-    while (kTile > kTileMin && ((size_t)k * k + 2 * k + (size_t)kTile * als_pitch(k)) * sizeof(double) * 4 > ctx->smem_per_sm) kTile /= 2;
-    size_t smem = ((size_t)k * k + 2 * k + (size_t)kTile * als_pitch(k)) * sizeof(double);
-    // k where M does not fit one CTA: the cluster solver, on the fewest CTAs whose shares fit, with as
-    // many staged rows as then fit
-    int csize = 1;
-    if (smem > ctx->smem_optin) {
-        if (k > 256)
-            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "mfrec_train_als_wrmf: k=%d > 256, the library-wide limit (as mfrec_model_create)", k);
-        cudaFuncAttributes fa;
-        MF_CUDA(ctx, cudaFuncGetAttributes(&fa, als_cluster_solve_kernel));
-        const size_t budget = ctx->smem_optin > fa.sharedSizeBytes ? ctx->smem_optin - fa.sharedSizeBytes : 0;
-        csize = 2;
-        while (csize < kClusterMax && als_cluster_smem(k, csize, kTileMin) > budget) ++csize;
-        kTile = kTileMax;
-        while (kTile > kTileMin && als_cluster_smem(k, csize, kTile) > budget) kTile /= 2;
-        smem = als_cluster_smem(k, csize, kTile);
-        if (smem > budget)
-            return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "mfrec_train_als_wrmf: k=%d needs %zu B of shared memory on each of %d CTAs", k, smem, csize);
-    }
+    AlsLayout lay;
+    MF_TRY(als_layout(ctx, k, "mfrec_train_als_wrmf", lay));
+    const int kTile = lay.kTile, csize = lay.csize;
+    const size_t smem = lay.smem;
     if (nbr_epochs == 0) return MFREC_OK;
     const std::vector<int64_t> uoff = offsets_from_counts(users_row, n_users_row);
     const std::vector<int64_t> ioff = offsets_from_counts(items_row, n_items_row);
@@ -581,5 +652,341 @@ extern "C" int mfrec_train_als_wrmf(mfrec_ctx *ctx, int nbr_epochs, int k, doubl
     MF_LAUNCH_CHECK(ctx);
     MF_CUDA(ctx, cudaMemcpyAsync(u, d_stage.p, (size_t)k * nbr_items * 8, cudaMemcpyDeviceToHost, st));
     MF_CUDA(ctx, cudaStreamSynchronize(st));
+    return MFREC_OK;
+}
+
+// ---- mfrec_train_als_wrmf over several shards ------------------------------------------------------
+// Inside a half-pass every row's system is independent, and its only shared inputs are the fixed
+// side's factors and HH.  So every shard keeps a full copy of U and V, computes HH itself (the same
+// gram() with the same block count: the same sums in the same order), solves a contiguous range of
+// rows with the one-device code path, and stores each solution into every shard's copy of the solved
+// side (peer stores over NVLink, plain stores when the copy is on its own device).  An event per
+// shard separates the half-passes.  The result is the one-device result bit for bit.
+namespace {
+
+struct AlsShard {
+    int device = 0;
+    mfrec_ctx *ctx = nullptr;
+    cudaEvent_t done = nullptr;              // recorded after each of its solves
+    std::vector<cudaEvent_t> tev;            // MFREC_ALS_SHARD_TIMES: start / end of each half-pass
+    int64_t u0 = 0, u1 = 0, i0 = 0, i1 = 0;  // active users [u0, u1), items [i0, i1)
+    std::vector<int64_t> huoff, hioff;       // offsets of its rows, from 0
+    DevBuf<double> U, V;                     // plain cudaMalloc: other devices store into them
+    DevBuf<double> stage, part, HH;          // stage: shard 0 only (host layout in and out)
+    DevBuf<int64_t> uoff, ioff;
+    DevBuf<int32_t> ucol, icol, bad;
+    int32_t h_bad = 0;
+
+    void release()
+    {
+        if (!ctx) return;
+        cudaSetDevice(device);
+        U.release(); V.release(); stage.release(); part.release(); HH.release();
+        uoff.release(); ioff.release(); ucol.release(); icol.release(); bad.release();
+        if (done) cudaEventDestroy(done);
+        for (cudaEvent_t e : tev) if (e) cudaEventDestroy(e);
+        done = nullptr;
+        tev.clear();
+        mfrec_ctx_destroy(ctx);
+        ctx = nullptr;
+    }
+};
+
+// Owns the shards and the peer mappings this call enabled; on every exit it waits for all streams
+// (a shard's kernels store into the others' copies), then frees everything and disables those mappings.
+struct AlsShards {
+    std::vector<AlsShard> s;
+    std::vector<std::pair<int, int>> peers;   // (device, peer device)
+    int caller_device = -1;                   // current device on entry, current again on exit
+    explicit AlsShards(int n) : s(n)
+    {
+        if (cudaGetDevice(&caller_device) != cudaSuccess) caller_device = -1;
+    }
+    ~AlsShards()
+    {
+        for (AlsShard &x : s)
+            if (x.ctx) {
+                cudaSetDevice(x.device);
+                cudaStreamSynchronize(x.ctx->stream);
+            }
+        for (AlsShard &x : s) x.release();
+        for (const auto &p : peers) {
+            cudaSetDevice(p.first);
+            cudaDeviceDisablePeerAccess(p.second);
+        }
+        if (caller_device >= 0) cudaSetDevice(caller_device);
+    }
+};
+
+// Cuts active rows [0, n) into `parts` contiguous ranges of near-equal estimated solve cost, 3 deg k^2
+// + k^3 per row (the Gram update and the Cholesky, times 3): range s ends before the first row at
+// which the running cost reaches (s + 1) / parts of the total.  Ranges may be empty.
+std::vector<int64_t> split_rows(const std::vector<int64_t> &off, int64_t n, int k, int parts)
+{
+    const int64_t kk3 = 3 * (int64_t)k * k, kkk = (int64_t)k * k * k;
+    std::vector<int64_t> pre((size_t)n + 1, 0);
+    for (int64_t j = 0; j < n; ++j) pre[j + 1] = pre[j] + (off[j + 1] - off[j]) * kk3 + kkk;
+    std::vector<int64_t> cut((size_t)parts + 1, n);
+    cut[0] = 0;
+    for (int s = 1; s < parts; ++s) {
+        const int64_t target = pre[n] / parts * s + pre[n] % parts * s / parts;
+        const int64_t c = std::lower_bound(pre.begin(), pre.end(), target) - pre.begin();
+        cut[s] = std::max(cut[s - 1], std::min(c, n));
+    }
+    return cut;
+}
+
+}  // namespace
+
+extern "C" int mfrec_train_als_wrmf_multi(const int32_t *devices, int n_shards, int nbr_epochs, int k,
+                                          double *u, double *v,
+                                          const int32_t *users_row, int64_t n_users_row, const int32_t *users_col,
+                                          const int32_t *items_row, int64_t n_items_row, const int32_t *items_col,
+                                          int32_t nbr_users, int32_t nbr_items, int c_pos, double reg)
+{
+    const char *who = "mfrec_train_als_wrmf_multi";
+    if (!devices || n_shards < 1)
+        return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "%s: no devices", who);
+    if (!u || !v || !users_row || !items_row)
+        return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "%s: NULL argument", who);
+    if (k <= 0 || nbr_users <= 0 || nbr_items <= 0 || nbr_epochs < 0 || n_users_row < 1 || n_items_row < 1)
+        return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "%s: k=%d users=%d items=%d epochs=%d", who, k,
+                               nbr_users, nbr_items, nbr_epochs);
+    const int64_t nau = n_users_row - 1, nai = n_items_row - 1;
+    if (nau > nbr_users || nai > nbr_items)
+        return mfrec_set_error(nullptr, MFREC_ERR_INDEX, "%s: more rows in the sparse structure than users / items", who);
+    if (n_shards > kAlsMaxShards)
+        return mfrec_set_error(nullptr, MFREC_ERR_UNSUPPORTED, "%s: %d shards, at most %d", who, n_shards, kAlsMaxShards);
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) {
+        cudaGetLastError();
+        return mfrec_set_error(nullptr, MFREC_ERR_CUDA, "%s: no CUDA device; this library has no CPU path", who);
+    }
+    for (int d = 0; d < n_shards; ++d)
+        if (devices[d] < 0 || devices[d] >= count)
+            return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "%s: device %d of %d", who, devices[d], count);
+    AlsShards G(n_shards);
+    std::vector<AlsShard> &S = G.s;
+    for (int d = 0; d < n_shards; ++d) {
+        S[d].device = devices[d];
+        MF_TRY(mfrec_ctx_create(devices[d], &S[d].ctx));
+    }
+    // distinct devices, and every ordered pair of them must reach the other's memory
+    std::vector<int> devs;
+    for (int d = 0; d < n_shards; ++d)
+        if (std::find(devs.begin(), devs.end(), devices[d]) == devs.end()) devs.push_back(devices[d]);
+    for (int a : devs)
+        for (int b : devs) {
+            if (a == b) continue;
+            int can = 0;
+            MF_CUDA(nullptr, cudaDeviceCanAccessPeer(&can, a, b));
+            if (!can) return mfrec_set_error(nullptr, MFREC_ERR_UNSUPPORTED, "%s: device %d cannot address device %d", who, a, b);
+        }
+    // one solver layout and one Gram block count for all shards, those of the first shard's device (and
+    // of a one-device call there): bit-identity needs the same partition of every sum
+    AlsLayout lay;
+    MF_TRY(als_layout(S[0].ctx, k, who, lay));
+    const int nblocks = S[0].ctx->sm_count;
+    std::vector<cudaLaunchConfig_t> ccfg(n_shards);
+    cudaLaunchAttribute cattr[1];
+    cattr[0].id = cudaLaunchAttributeClusterDimension;
+    cattr[0].val.clusterDim.x = lay.csize;
+    cattr[0].val.clusterDim.y = 1;
+    cattr[0].val.clusterDim.z = 1;
+    for (int d = 0; d < n_shards; ++d) {
+        mfrec_ctx *ctx = S[d].ctx;
+        MF_CUDA(nullptr, cudaSetDevice(S[d].device));
+        if (lay.csize == 1) {
+            if (lay.smem > ctx->smem_optin)
+                return mfrec_set_error(nullptr, MFREC_ERR_UNSUPPORTED, "%s: k=%d: device %d cannot give one CTA %zu B of shared memory",
+                                       who, k, S[d].device, lay.smem);
+            MF_CUDA(nullptr, cudaFuncSetAttribute(als_solve_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.smem));
+        } else {
+            MF_CUDA(nullptr, cudaFuncSetAttribute(als_cluster_solve_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.smem));
+            cudaLaunchConfig_t &c = ccfg[d];
+            c = {};
+            c.gridDim = dim3(lay.csize, 1, 1);
+            c.blockDim = dim3(kClusterThreads, 1, 1);
+            c.dynamicSmemBytes = lay.smem;
+            c.stream = ctx->stream;
+            c.attrs = cattr;
+            c.numAttrs = 1;
+            int nclusters = 0;
+            MF_CUDA(nullptr, cudaOccupancyMaxActiveClusters(&nclusters, als_cluster_solve_multi_kernel, &c));
+            if (nclusters < 1)
+                return mfrec_set_error(nullptr, MFREC_ERR_UNSUPPORTED, "%s: k=%d: a cluster of %d CTAs with %zu B of shared memory each does not fit device %d",
+                                       who, k, lay.csize, lay.smem, S[d].device);
+        }
+    }
+    if (nbr_epochs == 0) return MFREC_OK;
+    const std::vector<int64_t> uoff = offsets_from_counts(users_row, n_users_row);
+    const std::vector<int64_t> ioff = offsets_from_counts(items_row, n_items_row);
+    const int64_t nuc = uoff[nau], nic = ioff[nai];
+    if ((nuc > 0 && !users_col) || (nic > 0 && !items_col))
+        return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "%s: NULL column array", who);
+    for (int64_t j = 0; j < nau; ++j)
+        if (uoff[j + 1] < uoff[j]) return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "%s: negative count", who);
+    for (int64_t j = 0; j < nai; ++j)
+        if (ioff[j + 1] < ioff[j]) return mfrec_set_error(nullptr, MFREC_ERR_BAD_ARG, "%s: negative count", who);
+    const std::vector<int64_t> cu = split_rows(uoff, nau, k, n_shards), ci = split_rows(ioff, nai, k, n_shards);
+    for (int a : devs)   // before the first launch
+        for (int b : devs) {
+            if (a == b) continue;
+            MF_CUDA(nullptr, cudaSetDevice(a));
+            const cudaError_t e = cudaDeviceEnablePeerAccess(b, 0);
+            if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+            else {
+                MF_CUDA(nullptr, e);
+                G.peers.emplace_back(a, b);
+            }
+        }
+    const char *times_path = getenv("MFREC_ALS_SHARD_TIMES");
+    // ---- per shard: its rows' structure and the validation of their neighbour ids --------------------
+    for (int d = 0; d < n_shards; ++d) {
+        AlsShard &s = S[d];
+        mfrec_ctx *ctx = s.ctx;
+        cudaStream_t st = ctx->stream;
+        MF_CUDA(nullptr, cudaSetDevice(s.device));
+        s.u0 = cu[d]; s.u1 = cu[d + 1]; s.i0 = ci[d]; s.i1 = ci[d + 1];
+        s.huoff.resize(s.u1 - s.u0 + 1);
+        s.hioff.resize(s.i1 - s.i0 + 1);
+        for (int64_t j = s.u0; j <= s.u1; ++j) s.huoff[j - s.u0] = uoff[j] - uoff[s.u0];
+        for (int64_t j = s.i0; j <= s.i1; ++j) s.hioff[j - s.i0] = ioff[j] - ioff[s.i0];
+        const int64_t nuc_s = s.huoff.back(), nic_s = s.hioff.back();
+        MF_CUDA(nullptr, cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+        if (times_path) {
+            s.tev.assign((size_t)4 * nbr_epochs, nullptr);
+            for (cudaEvent_t &e : s.tev) MF_CUDA(nullptr, cudaEventCreate(&e));
+        }
+        if (d == 0) MF_CUDA(nullptr, s.stage.alloc((size_t)k * std::max<int64_t>(nbr_users, nbr_items), st));
+        MF_CUDA(nullptr, s.U.alloc((size_t)k * nbr_items));
+        MF_CUDA(nullptr, s.V.alloc((size_t)k * nbr_users));
+        MF_CUDA(nullptr, s.part.alloc((size_t)nblocks * k * k, st));
+        MF_CUDA(nullptr, s.HH.alloc((size_t)k * k, st));
+        MF_CUDA(nullptr, s.uoff.alloc(s.huoff.size(), st));
+        MF_CUDA(nullptr, s.ioff.alloc(s.hioff.size(), st));
+        MF_CUDA(nullptr, s.ucol.alloc(nuc_s, st));
+        MF_CUDA(nullptr, s.icol.alloc(nic_s, st));
+        MF_CUDA(nullptr, s.bad.alloc(1, st));
+        MF_CUDA(nullptr, cudaMemsetAsync(s.bad.p, 0, 4, st));
+        MF_CUDA(nullptr, cudaMemcpyAsync(s.uoff.p, s.huoff.data(), s.huoff.size() * 8, cudaMemcpyHostToDevice, st));
+        MF_CUDA(nullptr, cudaMemcpyAsync(s.ioff.p, s.hioff.data(), s.hioff.size() * 8, cudaMemcpyHostToDevice, st));
+        if (nuc_s) MF_CUDA(nullptr, cudaMemcpyAsync(s.ucol.p, users_col + uoff[s.u0], (size_t)nuc_s * 4, cudaMemcpyHostToDevice, st));
+        if (nic_s) MF_CUDA(nullptr, cudaMemcpyAsync(s.icol.p, items_col + ioff[s.i0], (size_t)nic_s * 4, cudaMemcpyHostToDevice, st));
+        if (nuc_s) { validate_cols_kernel<<<ctx->sm_count, 256, 0, st>>>(s.ucol.p, nuc_s, nbr_items, s.bad.p); MF_LAUNCH_CHECK(ctx); }
+        if (nic_s) { validate_cols_kernel<<<ctx->sm_count, 256, 0, st>>>(s.icol.p, nic_s, nbr_users, s.bad.p); MF_LAUNCH_CHECK(ctx); }
+        MF_CUDA(nullptr, cudaMemcpyAsync(&s.h_bad, s.bad.p, 4, cudaMemcpyDeviceToHost, st));
+    }
+    for (int d = 0; d < n_shards; ++d) {
+        MF_CUDA(nullptr, cudaSetDevice(S[d].device));
+        MF_CUDA(nullptr, cudaStreamSynchronize(S[d].ctx->stream));
+    }
+    for (int d = 0; d < n_shards; ++d)
+        if (S[d].h_bad) return mfrec_set_error(nullptr, MFREC_ERR_INDEX, "%s: neighbour id out of range", who);
+    // ---- factors: [k][n] host -> [n][k] on shard 0 (one host transfer per side), then device to device
+    // into every other shard's copies (over NVLink between devices)
+    {
+        AlsShard &s0 = S[0];
+        cudaStream_t st = s0.ctx->stream;
+        MF_CUDA(nullptr, cudaSetDevice(s0.device));
+        MF_CUDA(nullptr, cudaMemcpyAsync(s0.stage.p, u, (size_t)k * nbr_items * 8, cudaMemcpyHostToDevice, st));
+        to_rows_f64_kernel<<<dim3((unsigned)ceil_div64(nbr_items, 32), (k + 31) / 32), 256, 0, st>>>(s0.stage.p, k, nbr_items, s0.U.p);
+        MF_LAUNCH_CHECK(s0.ctx);
+        MF_CUDA(nullptr, cudaMemcpyAsync(s0.stage.p, v, (size_t)k * nbr_users * 8, cudaMemcpyHostToDevice, st));
+        to_rows_f64_kernel<<<dim3((unsigned)ceil_div64(nbr_users, 32), (k + 31) / 32), 256, 0, st>>>(s0.stage.p, k, nbr_users, s0.V.p);
+        MF_LAUNCH_CHECK(s0.ctx);
+        MF_CUDA(nullptr, cudaEventRecord(s0.done, st));
+    }
+    for (int d = 1; d < n_shards; ++d) {   // (shard 0 overwrites its copies only after every shard's done event)
+        AlsShard &s = S[d];
+        cudaStream_t st = s.ctx->stream;
+        MF_CUDA(nullptr, cudaSetDevice(s.device));
+        MF_CUDA(nullptr, cudaStreamWaitEvent(st, S[0].done, 0));
+        MF_CUDA(nullptr, cudaMemcpyPeerAsync(s.U.p, s.device, S[0].U.p, S[0].device, (size_t)k * nbr_items * 8, st));
+        MF_CUDA(nullptr, cudaMemcpyPeerAsync(s.V.p, s.device, S[0].V.p, S[0].device, (size_t)k * nbr_users * 8, st));
+        MF_CUDA(nullptr, cudaEventRecord(s.done, st));
+    }
+    // ---- half-passes ----------------------------------------------------------------------------------
+    // every shard's stream first waits for every other shard's last solve (or upload): the Gram reads the
+    // side they stored into, and this pass overwrites the side they read
+    int hp = 0;
+    auto half_pass = [&](bool users) -> int {
+        for (int d = 0; d < n_shards; ++d) {
+            MF_CUDA(nullptr, cudaSetDevice(S[d].device));
+            for (int t = 0; t < n_shards; ++t)
+                if (t != d) MF_CUDA(nullptr, cudaStreamWaitEvent(S[d].ctx->stream, S[t].done, 0));
+        }
+        for (int d = 0; d < n_shards; ++d) {
+            AlsShard &s = S[d];
+            mfrec_ctx *ctx = s.ctx;
+            cudaStream_t st = ctx->stream;
+            MF_CUDA(nullptr, cudaSetDevice(s.device));
+            if (times_path) MF_CUDA(nullptr, cudaEventRecord(s.tev[2 * hp], st));
+            const double *X = users ? s.U.p : s.V.p;
+            MF_TRY(gram(ctx, X, users ? nbr_items : nbr_users, k, s.part.p, nblocks, s.HH.p));
+            const int64_t r0 = users ? s.u0 : s.i0, rows = (users ? s.u1 : s.i1) - r0;
+            const int64_t *doff = users ? s.uoff.p : s.ioff.p;
+            const int32_t *dcol = users ? s.ucol.p : s.icol.p;
+            AlsDst dst = {};
+            dst.n = n_shards;
+            for (int t = 0; t < n_shards; ++t) dst.p[t] = users ? S[t].V.p : S[t].U.p;
+            if (rows > 0) {
+                if (lay.csize == 1) {
+                    als_solve_multi_kernel<<<(unsigned)rows, 128, lay.smem, st>>>(X, s.HH.p, doff, dcol, k, (double)c_pos, reg, dst, r0, lay.kTile);
+                } else {
+                    if (rows * lay.csize > INT32_MAX)
+                        return mfrec_set_error(nullptr, MFREC_ERR_UNSUPPORTED, "%s: %lld rows x %d CTAs exceed one grid", who, (long long)rows, lay.csize);
+                    ccfg[d].gridDim = dim3((unsigned)(rows * lay.csize), 1, 1);
+                    MF_CUDA(nullptr, cudaLaunchKernelEx(&ccfg[d], als_cluster_solve_multi_kernel, X, (const double *)s.HH.p, doff, dcol, k,
+                                                        (double)c_pos, reg, dst, r0, lay.kTile, lay.csize));
+                }
+                MF_LAUNCH_CHECK(ctx);
+            }
+            if (times_path) MF_CUDA(nullptr, cudaEventRecord(s.tev[2 * hp + 1], st));
+            MF_CUDA(nullptr, cudaEventRecord(s.done, st));
+        }
+        ++hp;
+        return MFREC_OK;
+    };
+    for (int e = 0; e < nbr_epochs; ++e) {
+        MF_TRY(half_pass(true));
+        MF_TRY(half_pass(false));
+    }
+    // ---- result: shard 0's copies, once every shard's last stores have landed -------------------------
+    AlsShard &s0 = S[0];
+    cudaStream_t st = s0.ctx->stream;
+    MF_CUDA(nullptr, cudaSetDevice(s0.device));
+    for (int t = 1; t < n_shards; ++t) MF_CUDA(nullptr, cudaStreamWaitEvent(st, S[t].done, 0));
+    from_rows_f64_kernel<<<dim3((unsigned)ceil_div64(nbr_users, 32), (k + 31) / 32), 256, 0, st>>>(s0.V.p, k, nbr_users, s0.stage.p);
+    MF_LAUNCH_CHECK(s0.ctx);
+    MF_CUDA(nullptr, cudaMemcpyAsync(v, s0.stage.p, (size_t)k * nbr_users * 8, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(nullptr, cudaStreamSynchronize(st));
+    from_rows_f64_kernel<<<dim3((unsigned)ceil_div64(nbr_items, 32), (k + 31) / 32), 256, 0, st>>>(s0.U.p, k, nbr_items, s0.stage.p);
+    MF_LAUNCH_CHECK(s0.ctx);
+    MF_CUDA(nullptr, cudaMemcpyAsync(u, s0.stage.p, (size_t)k * nbr_items * 8, cudaMemcpyDeviceToHost, st));
+    MF_CUDA(nullptr, cudaStreamSynchronize(st));
+    if (times_path) {   // one JSON line per call: each shard's rows and milliseconds per half-pass
+        for (AlsShard &s : S) {
+            MF_CUDA(nullptr, cudaSetDevice(s.device));
+            MF_CUDA(nullptr, cudaStreamSynchronize(s.ctx->stream));
+        }
+        FILE *f = fopen(times_path, "a");
+        if (f) {
+            fprintf(f, "{\"k\": %d, \"epochs\": %d, \"csize\": %d, \"shards\": [", k, nbr_epochs, lay.csize);
+            for (int d = 0; d < n_shards; ++d) {
+                const AlsShard &s = S[d];
+                fprintf(f, "%s{\"device\": %d, \"users\": [%lld, %lld], \"items\": [%lld, %lld], \"half_pass_ms\": [", d ? ", " : "",
+                        s.device, (long long)s.u0, (long long)s.u1, (long long)s.i0, (long long)s.i1);
+                for (int h = 0; h < hp; ++h) {
+                    float ms = 0.f;
+                    cudaEventElapsedTime(&ms, s.tev[2 * h], s.tev[2 * h + 1]);
+                    fprintf(f, "%s%.4f", h ? ", " : "", ms);
+                }
+                fprintf(f, "]}");
+            }
+            fprintf(f, "]}\n");
+            fclose(f);
+        }
+    }
     return MFREC_OK;
 }

@@ -54,7 +54,8 @@ options = {
     "seed": int(os.environ.get("MFREC_B200_SEED", "0")),
     "device": int(os.environ.get("MFREC_B200_DEVICE", "-1")),
     # several CUDA devices, e.g. [0, 1, 2, 3] (MFREC_B200_DEVICES=0,1,2,3): train_linear_kernel /
-    # train_logistic_kernel calls that train both sides run as a DSGD ring over them
+    # train_logistic_kernel calls that train both sides run as a DSGD ring over them, and als_wrmf
+    # (WRMFRecommender.train) splits each ALS half-pass's rows over them (bit-identical to one device)
     "devices": [int(x) for x in os.environ.get("MFREC_B200_DEVICES", "").split(",") if x.strip()],
     # how the user-factor rows are kept in HBM while training: "f32" | "f16" | "bf16"
     # (mfrec_opts.storage in include/mfrec_b200.h: arithmetic stays float32; single device, both

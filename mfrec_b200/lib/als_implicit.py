@@ -2,8 +2,9 @@
 
 ``als_wrmf`` keeps the reference's signature (mfrec/lib/als_implicit.pyx:211-225); ``m`` and
 ``m_inv`` are scratch matrices there and are accepted and ignored here; ``u`` and ``v`` are updated
-in place; returns ``None``.  ``als_wrmf_dense`` (the dense-matrix development variant, :68-205) is
-out of scope."""
+in place; returns ``None``.  With more than one entry in ``options["devices"]`` the call is split
+over those devices (``mfrec_train_als_wrmf_multi``) and gives the one-device result bit for bit.
+``als_wrmf_dense`` (the dense-matrix development variant, :68-205) is out of scope."""
 import numpy as np
 
 from mfrec_b200 import _native
@@ -25,6 +26,11 @@ def als_wrmf(nbr_epochs, dim, u, v, m, m_inv, ratings_users_row, ratings_users_c
     if verbose:
         for epoch in range(int(nbr_epochs)):
             print('Epoch : ' + str(epoch))
+    if len(options["devices"]) > 1:
+        _native.train_als_wrmf_multi(options["devices"], int(nbr_epochs), dim, u, v, ratings_users_row,
+                                     ratings_users_col, ratings_items_row, ratings_items_col, int(nbr_users),
+                                     int(nbr_items), c_pos, k)
+        return None
     _native.train_als_wrmf(int(nbr_epochs), dim, u, v, ratings_users_row, ratings_users_col,
                            ratings_items_row, ratings_items_col, int(nbr_users), int(nbr_items), c_pos, k,
                            ctx=_native.default_context(options["device"]))

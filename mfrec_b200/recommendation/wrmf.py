@@ -45,7 +45,9 @@ class WRMFRecommender(MFRecommender):
         literal 0.015 and c_pos the literal 1 (the ``K`` attribute is not used there either).
         Note (a property of the reference, kept): the constant initialisation makes all features
         identical; round-off breaks the symmetry and from the third epoch on the factors depend on
-        the linear solver's rounding (tests/test_als_gpu.py)."""
+        the linear solver's rounding (tests/test_als_gpu.py).  With several devices in
+        ``mfrec_b200.lib.als_implicit.options["devices"]`` the rows of each half-pass are split over
+        them; the factors are the same bit for bit as on the first of them alone."""
         self.relationship_matrix_csc = self.relationship_matrix.T.tocsc()
         if initialize_model:
             self.svd_v = np.zeros([self.dimensionality, self.nbr_users]) + self.feature_init

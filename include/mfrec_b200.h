@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define MFREC_B200_ABI_VERSION 6
+#define MFREC_B200_ABI_VERSION 7
 
 typedef enum mfrec_status {
     MFREC_OK = 0,
@@ -462,6 +462,46 @@ int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *m, int predictor, 
                            const int32_t *rated_items, double mu, double min_rating,
                            double max_rating, int32_t N, int32_t *out_items, double *out_scores,
                            int32_t *out_counts, double stats[8]);
+
+/* ---- serving from several shards of one process ------------------------------------------------
+ * Both calls take n_shards (1..16) contexts and resident models, model s living on context s's device,
+ * all with equal k, ni, nu and kpad (the same factors uploaded once per shard).  Devices may repeat:
+ * every shard has its own context (contexts must be distinct: one in-flight call per context) and its
+ * own model.  Each shard runs the one-device call on its own host thread, context and stream, on a
+ * contiguous share of the work, and writes its own rows of the caller's outputs.  Host code only: no
+ * peer access, nothing is exchanged between devices.  Everything is validated before any launch, so
+ * a refused call leaves the outputs untouched; errors are reported on ctxs[0] (a shard's device error
+ * is copied there with the shard's number). */
+
+/* mfrec_model_topn_sweep over the shards; after n_shards the arguments of mfrec_model_topn_sweep.
+ * Every output row equals the one-device call's bit for bit: a user's result depends only on that
+ * user and the item side, and the path rule (the exact path below 128 users, for large N, ...) is
+ * applied once, to the whole user list; a share takes that path whatever its size.  The list
+ * (users == NULL: users 0 .. n_users-1) is cut into contiguous shares of near-equal count, at
+ * multiples of 512 users while every shard gets at least 512; a share may be empty.  Each share's
+ * rated-items CSR is rebased to start at 0.  The models must be in identity layout.  stats: as for
+ * mfrec_model_topn_sweep, merged: users redone, FLOPs and overflows summed; candidates per user
+ * averaged weighted by the shares' users; sweep and finish ms the slowest shard's; padded K and z are
+ * the same on every shard.  Fails with MFREC_ERR_UNSUPPORTED if two sweep CTAs could share an SM of a
+ * shard's device (each takes all of the SM's tensor memory); on a B200 neither registers nor shared
+ * memory allow it.  Debug only: with the environment variable MFREC_TOPN_SHARD_TIMES set to a file
+ * name, a call appends one JSON line to that file: the path and every shard's device, user range,
+ * sweep / finish ms and users redone. */
+int mfrec_model_topn_sweep_multi(mfrec_ctx *const *ctxs, const mfrec_model *const *models, int n_shards,
+                                 int predictor, const int32_t *users, int32_t n_users, int32_t n_candidates,
+                                 const int64_t *rated_indptr, const int32_t *rated_items, double mu,
+                                 double min_rating, double max_rating, int32_t N, int32_t *out_items,
+                                 double *out_scores, int32_t *out_counts, double stats[8]);
+
+/* mfrec_model_predict over the shards, for HOST arrays (pairs int32 [n][2], real nullable, out
+ * nullable float64 [n]): contiguous shares of near-equal count, every out[j] equal to the one-device
+ * call's (a pair's prediction does not depend on its position).  stats_out (nullable) = the shards'
+ * raw sums added in shard order.  A pair naming a row outside the model is MFREC_ERR_INDEX, reported
+ * after the launches as by mfrec_model_predict. */
+int mfrec_model_predict_multi(mfrec_ctx *const *ctxs, const mfrec_model *const *models, int n_shards,
+                              int predictor, const int32_t *pairs, const void *real, int real_is_f32,
+                              int64_t n, double mu, double min_rating, double max_rating, double *out,
+                              double stats_out[4]);
 
 #ifdef __cplusplus
 }

@@ -3,6 +3,7 @@
 There is no CPU path: if the shared library is missing, or no sm_100 device is visible when
 a compute call is made, an exception is raised -- nothing silently falls back.
 """
+import atexit
 import ctypes as C
 import os
 import threading
@@ -44,6 +45,7 @@ EXPORTS = (
     "mfrec_ring_connect_local", "mfrec_ring_epochs", "mfrec_ring_epochs_one_device", "mfrec_ring_wait",
     "mfrec_ring_sync_model", "mfrec_model_topn", "mfrec_model_topn_sweep", "mfrec_ratings_copies",
     "mfrec_train_kmf_multi", "mfrec_fold_in_kmf", "mfrec_fold_in_funk", "mfrec_train_als_wrmf_multi",
+    "mfrec_model_topn_sweep_multi", "mfrec_model_predict_multi",
 )
 
 
@@ -652,6 +654,117 @@ def _model_topn(self, predictor, users, n_candidates, rated_indptr, rated_items,
 
 
 Model.topn = _model_topn
+
+
+_shard_ctx = {}
+
+
+@atexit.register
+def _close_shard_contexts():
+    """Close the cached shard contexts while the module is still whole (a model that outlives them
+    keeps its device context alive until it is destroyed)."""
+    with _ctx_lock:
+        for ctxs in _shard_ctx.values():
+            for c in ctxs:
+                c.close()
+        _shard_ctx.clear()
+
+
+def shard_contexts(devices):
+    """One Context per entry of ``devices`` (a new one for every entry, also when ids repeat: a
+    context runs one call at a time), kept per device tuple so that a ModelSet rebuilt for new
+    factors reuses its streams and memory pools."""
+    key = tuple(int(d) for d in devices)
+    with _ctx_lock:
+        if key not in _shard_ctx:
+            _shard_ctx[key] = tuple(Context(d) for d in key)
+        return _shard_ctx[key]
+
+
+def _handles(objs):
+    return (C.c_void_p * len(objs))(*[o.handle for o in objs])
+
+
+class ModelSet(object):
+    """The same factors resident on several shards, one ``Model`` per entry of ``devices``, each on its
+    own Context.  Batched top-N (``topn(..., sweep=True)``) and host-array ``predict`` split their work
+    over the shards (``mfrec_model_topn_sweep_multi`` / ``mfrec_model_predict_multi``) and return what
+    one Model returns, bit for bit; everything else runs on the first shard."""
+
+    def __init__(self, devices, k, ni, nu, u=None, v=None, items_bias=None, users_bias=None):
+        ctxs = shard_contexts(devices)
+        if not ctxs:
+            raise ValueError("ModelSet needs at least one device")
+        self.k, self.ni, self.nu = int(k), int(ni), int(nu)
+        u, v = _as(u, np.float64), _as(v, np.float64)
+        ib, ub = _as(items_bias, np.float64), _as(users_bias, np.float64)
+        models, errors = [None] * len(ctxs), [None] * len(ctxs)
+
+        def build(s):   # the uploads of the shards overlap (ctypes drops the GIL during the call)
+            try:
+                models[s] = Model(k, ni, nu, u, v, ib, ub, ctx=ctxs[s])
+            except Exception as e:   # re-raised on the calling thread
+                errors[s] = e
+
+        threads = [threading.Thread(target=build, args=(s,)) for s in range(1, len(ctxs))]
+        for t in threads:
+            t.start()
+        build(0)
+        for t in threads:
+            t.join()
+        for e in errors:
+            if e is not None:
+                raise e
+        self.models = tuple(models)
+        self.devices = tuple(int(d) for d in devices)
+        self.ctx = ctxs[0]
+
+    def read(self):
+        return self.models[0].read()
+
+    def topn(self, predictor, users, n_candidates, rated_indptr, rated_items, N, mu=0.0, min_rating=1.0,
+             max_rating=5.0, sweep=False, out=None):
+        """``Model.topn``; with sweep=True the user list is split over the shards."""
+        if not sweep:
+            return self.models[0].topn(predictor, users, n_candidates, rated_indptr, rated_items, N, mu, min_rating,
+                                       max_rating, sweep=False, out=out)
+        users = None if users is None else _as(users, np.int32).reshape(-1)   # None: all users
+        n_users = self.nu if users is None else users.shape[0]
+        indptr = _as(rated_indptr, np.int64)
+        rated = _as(rated_items, np.int32)
+        if out is None:
+            items = np.full((n_users, N), -1, dtype=np.int32)
+            scores = np.zeros((n_users, N), dtype=np.float64)
+            counts = np.zeros(n_users, dtype=np.int32)
+        else:
+            items, scores, counts = out
+            assert items.shape == (n_users, N) and items.dtype == np.int32 and items.flags.c_contiguous
+            assert scores.shape == (n_users, N) and scores.dtype == np.float64 and scores.flags.c_contiguous
+            assert counts.shape == (n_users,) and counts.dtype == np.int32
+        stats = np.zeros(8, dtype=np.float64)
+        _check(lib().mfrec_model_topn_sweep_multi(
+            _handles([m.ctx for m in self.models]), _handles(self.models), C.c_int(len(self.models)),
+            C.c_int(PREDICTORS[predictor]), _ptr(users), C.c_int32(n_users), C.c_int32(n_candidates), _ptr(indptr),
+            _ptr(rated), C.c_double(mu), C.c_double(min_rating), C.c_double(max_rating), C.c_int32(N), _ptr(items),
+            _ptr(scores), _ptr(counts), _ptr(stats)), self.ctx.handle)
+        return items, scores, counts, stats
+
+    def predict(self, predictor, pairs, real=None, mu=0.0, min_rating=1.0, max_rating=5.0,
+                want_out=True, want_stats=False, device_ptrs=None, n=None, real_is_f32=False):
+        """``Model.predict``: host arrays are split over the shards; device pointers (which live on one
+        device) go to the first shard."""
+        if device_ptrs is not None:
+            return self.models[0].predict(predictor, pairs, real, mu, min_rating, max_rating, want_out, want_stats,
+                                          device_ptrs, n, real_is_f32)
+        stats = np.zeros(4, dtype=np.float64) if want_stats else None
+        pairs = _as(pairs, np.int32).reshape(-1, 2)
+        real = _as(real, np.float64)
+        out = np.zeros(pairs.shape[0], dtype=np.float64) if want_out else None
+        _check(lib().mfrec_model_predict_multi(
+            _handles([m.ctx for m in self.models]), _handles(self.models), C.c_int(len(self.models)),
+            C.c_int(PREDICTORS[predictor]), _ptr(pairs), _ptr(real), C.c_int(0), C.c_int64(pairs.shape[0]),
+            C.c_double(mu), C.c_double(min_rating), C.c_double(max_rating), _ptr(out), _ptr(stats)), self.ctx.handle)
+        return out, stats
 
 
 def copy_of_user(users, copies):

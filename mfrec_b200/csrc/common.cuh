@@ -8,6 +8,7 @@
 
 #include <cstdarg>
 #include <cstdio>
+#include <functional>
 #include <future>
 #include <memory>
 #include <string>
@@ -348,3 +349,12 @@ int mfrec_merge_copies(mfrec_ctx *ctx, float *Q, float *ib, int kpad, const int3
                        int32_t *abort_flag, unsigned long long wait_ns);
 int mfrec_download_vec(mfrec_ctx *ctx, const float *src, int32_t n, const int32_t *perm_dev,
                        double *host);
+
+// runtime.cu: serving from several shards of one process (mfrec_model_topn_sweep_multi,
+// mfrec_model_predict_multi).  mfrec_check_shards: 1 <= n_shards <= kMaxServeShards, no NULL entry,
+// every context distinct, each model on its context's device, equal k / kpad / ni / nu / storage;
+// errors on ctxs[0].  mfrec_run_shards: fn(s) for every shard, each on a host thread of its own
+// (shard 0 on the caller's); the first failing shard's status, its message copied to ctxs[0].
+constexpr int kMaxServeShards = 16;
+int mfrec_check_shards(mfrec_ctx *const *ctxs, const mfrec_model *const *models, int n_shards, const char *who);
+int mfrec_run_shards(mfrec_ctx *const *ctxs, int n_shards, const char *who, const std::function<int(int)> &fn);

@@ -541,3 +541,34 @@ extern "C" int mfrec_bias_stats(mfrec_ctx *ctx, const int32_t *ratings_index, co
     *mu_out = mu;
     return MFREC_OK;
 }
+
+// predict_kernel scores each pair from its own two rows with the same per-lane order wherever the pair
+// sits in the array (the four pairs of a warp iteration are reduced separately), so contiguous shares
+// of the pairs give every pair the one-device result.
+extern "C" int mfrec_model_predict_multi(mfrec_ctx *const *ctxs, const mfrec_model *const *models, int n_shards,
+                                         int predictor, const int32_t *pairs, const void *real, int real_is_f32,
+                                         int64_t n, double mu, double min_rating, double max_rating, double *out,
+                                         double stats_out[4])
+{
+    const char *who = "mfrec_model_predict_multi";
+    MF_TRY(mfrec_check_shards(ctxs, models, n_shards, who));
+    if (predictor < 0 || predictor > MFREC_PRED_DOT)
+        return mfrec_set_error(ctxs[0], MFREC_ERR_BAD_ARG, "%s: predictor=%d", who, predictor);
+    if (n < 0 || (n > 0 && !pairs)) return mfrec_set_error(ctxs[0], MFREC_ERR_BAD_ARG, "%s: n=%lld", who, (long long)n);
+    const size_t rsz = real_is_f32 ? 4 : 8;
+    std::vector<double> st((size_t)n_shards * 4, 0.0);
+    MF_TRY(mfrec_run_shards(ctxs, n_shards, who, [&](int s) -> int {
+        const int64_t a = n * s / n_shards, b = n * (s + 1) / n_shards;
+        if (a == b) return MFREC_OK;
+        return mfrec_model_predict(ctxs[s], models[s], predictor, pairs + 2 * a,
+                                   real ? static_cast<const char *>(real) + a * rsz : nullptr, real_is_f32, b - a, 0, mu,
+                                   min_rating, max_rating, out ? out + a : nullptr, stats_out ? &st[(size_t)s * 4] : nullptr);
+    }));
+    if (stats_out)
+        for (int j = 0; j < 4; ++j) {
+            double acc = 0.0;
+            for (int s = 0; s < n_shards; ++s) acc += st[(size_t)s * 4 + j];
+            stats_out[j] = acc;
+        }
+    return MFREC_OK;
+}

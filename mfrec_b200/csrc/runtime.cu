@@ -31,9 +31,8 @@ double Tracer::now()
 }
 Tracer::Tracer(const char *name, cudaStream_t stream) : st(stream), what(name)
 {
-    static int env = -1;
-    if (env < 0) env = getenv("MFREC_TRACE") ? 1 : 0;
-    on = env != 0;
+    static const bool env = getenv("MFREC_TRACE") != nullptr;   // (initialised once, also when shards start together)
+    on = env;
     t0 = last = on ? now() : 0.0;
 }
 void Tracer::lap(const char *stage)
@@ -604,5 +603,55 @@ extern "C" int mfrec_model_device_ptrs(const mfrec_model *m, void *ptrs[4], int6
     dims[0] = m->ni_rows;   // rows of Q / ib (item copies included): what a slab exchange addresses
     dims[1] = m->nu;
     dims[2] = m->kpad;
+    return MFREC_OK;
+}
+
+// ---- serving from several shards (mfrec_model_topn_sweep_multi, mfrec_model_predict_multi) ----------
+int mfrec_check_shards(mfrec_ctx *const *ctxs, const mfrec_model *const *models, int n_shards, const char *who)
+{
+    mfrec_ctx *c0 = ctxs && n_shards >= 1 ? ctxs[0] : nullptr;
+    if (!ctxs || !models || n_shards < 1)
+        return mfrec_set_error(c0, MFREC_ERR_BAD_ARG, "%s: no shards (n_shards=%d)", who, n_shards);
+    if (n_shards > kMaxServeShards)
+        return mfrec_set_error(c0, MFREC_ERR_UNSUPPORTED, "%s: %d shards, at most %d", who, n_shards, kMaxServeShards);
+    for (int s = 0; s < n_shards; ++s) {
+        if (!ctxs[s] || !models[s]) return mfrec_set_error(c0, MFREC_ERR_BAD_ARG, "%s: shard %d: NULL context or model", who, s);
+        for (int t = 0; t < s; ++t)
+            if (ctxs[t] == ctxs[s])
+                return mfrec_set_error(c0, MFREC_ERR_BAD_ARG, "%s: shards %d and %d share a context (one in-flight call per context)",
+                                       who, t, s);
+        const mfrec_model *m = models[s], *m0 = models[0];
+        if (m->device != ctxs[s]->device)
+            return mfrec_set_error(c0, MFREC_ERR_BAD_ARG, "%s: shard %d: model on device %d, context on device %d", who, s,
+                                   m->device, ctxs[s]->device);
+        if (m->k != m0->k || m->kpad != m0->kpad || m->ni != m0->ni || m->nu != m0->nu || m->p_kind != m0->p_kind)
+            return mfrec_set_error(c0, MFREC_ERR_BAD_ARG, "%s: shard %d: model k=%d ni=%d nu=%d kpad=%d differs from shard 0's "
+                                   "k=%d ni=%d nu=%d kpad=%d", who, s, m->k, m->ni, m->nu, m->kpad, m0->k, m0->ni, m0->nu,
+                                   m0->kpad);
+    }
+    return MFREC_OK;
+}
+
+int mfrec_run_shards(mfrec_ctx *const *ctxs, int n_shards, const char *who, const std::function<int(int)> &fn)
+{
+    std::vector<int> rc(n_shards, MFREC_OK);
+    std::vector<std::thread> threads;
+    std::vector<int> here;   // shards whose thread could not be started run on the calling thread
+    threads.reserve(n_shards);
+    for (int s = 1; s < n_shards; ++s) {
+        try {
+            threads.emplace_back([&rc, &fn, s] { rc[s] = fn(s); });
+        } catch (const std::system_error &) {
+            here.push_back(s);
+        }
+    }
+    rc[0] = fn(0);
+    for (int s : here) rc[s] = fn(s);
+    for (std::thread &t : threads) t.join();
+    for (int s = 0; s < n_shards; ++s)
+        if (rc[s] != MFREC_OK) {
+            const std::string msg = ctxs[s]->err;
+            return mfrec_set_error(ctxs[0], rc[s], "%s: shard %d (device %d): %s", who, s, ctxs[s]->device, msg.c_str());
+        }
     return MFREC_OK;
 }

@@ -27,6 +27,10 @@
 // O(users * (k^2 + C * k)) on the CUDA cores.
 #include <cuda_bf16.h>
 
+#include <algorithm>
+#include <cstdlib>
+#include <cstring>
+
 #include "common.cuh"
 
 namespace {
@@ -717,13 +721,30 @@ __global__ void __launch_bounds__(128, MFREC_FINISH_CTAS) topn_finish_kernel(con
     }
 }
 
+constexpr size_t sweep_smem_bytes(int KB, int NA, int ST)
+{
+    return (size_t)NA * KB * 16384 + (size_t)ST * KB * kBN * 128 + 256 + 1024;
+}
+
 template <int KB, int NA, int ST>
 int launch_sweep(mfrec_ctx *ctx, const SweepParams &prm, int grid)
 {
-    const size_t smem = (size_t)NA * KB * 16384 + (size_t)ST * KB * kBN * 128 + 256 + 1024;
+    const size_t smem = sweep_smem_bytes(KB, NA, ST);
     MF_CUDA(ctx, cudaFuncSetAttribute(topn_sweep_kernel<KB, NA, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     topn_sweep_kernel<KB, NA, ST><<<grid, kSweepThreads, smem, ctx->stream>>>(prm);
     MF_LAUNCH_CHECK(ctx);
+    return MFREC_OK;
+}
+
+// CTAs of one sweep instantiation that fit on one SM of the current device with its launch
+// configuration.  Every CTA allocates all 512 TMEM columns, so a second CTA on the same SM (from
+// another shard's stream, say) would wait in tcgen05.alloc until the first one finishes.
+template <int KB, int NA, int ST>
+int sweep_ctas_per_sm(mfrec_ctx *ctx, int *blocks)
+{
+    const size_t smem = sweep_smem_bytes(KB, NA, ST);
+    MF_CUDA(ctx, cudaFuncSetAttribute(topn_sweep_kernel<KB, NA, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MF_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, topn_sweep_kernel<KB, NA, ST>, kSweepThreads, smem));
     return MFREC_OK;
 }
 
@@ -767,11 +788,25 @@ extern "C" int mfrec_topn_sweep(mfrec_ctx *ctx, int predictor, int k, const doub
     return rc;
 }
 
-extern "C" int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *M, int predictor, const int32_t *users,
-                                      int32_t n_users, int32_t n_candidates, const int64_t *rated_indptr,
-                                      const int32_t *rated_items, double mu, double min_rating, double max_rating,
-                                      int32_t N, int32_t *out_items, double *out_scores, int32_t *out_counts,
-                                      double stats[8])
+namespace {
+
+// Which path a top-N call takes: the rule below (kPathAuto), or the one a multi-shard call chose for
+// the whole user list (a share of it may be smaller than the rule's 128 users).
+enum TopnPath { kPathAuto = 0, kPathSweep = 1, kPathExact = 2 };
+
+// The threshold filter pays off only when the top N is a thin slice of the candidates and the
+// candidate list has room for ~3N entries; everything else goes to the exact path.
+bool sweep_applies(int predictor, int k, int32_t N, int32_t n_candidates, int64_t n_users)
+{
+    const bool has_bias = predictor != MFREC_PRED_GD_RATING && predictor != MFREC_PRED_DOT;
+    const int KB = (k + (has_bias ? 1 : 0) + 63) / 64;
+    return !(8 * N > kCand || (int64_t)N * 16 > n_candidates || KB > 4 || n_users < 128);
+}
+
+int topn_sweep_on_model(mfrec_ctx *ctx, const mfrec_model *M, int predictor, const int32_t *users, int32_t n_users,
+                        int32_t n_candidates, const int64_t *rated_indptr, const int32_t *rated_items, double mu,
+                        double min_rating, double max_rating, int32_t N, int32_t *out_items, double *out_scores,
+                        int32_t *out_counts, double stats[8], int path)
 {
     if (!ctx || !M || !out_items || !out_scores || !out_counts)
         return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "mfrec_topn_sweep: NULL argument");
@@ -793,9 +828,7 @@ extern "C" int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *M, int 
     const bool has_bias = predictor != MFREC_PRED_GD_RATING && predictor != MFREC_PRED_DOT;
     const int ka = k + (has_bias ? 1 : 0);
     const int KB = (ka + 63) / 64;
-    // The threshold filter pays off only when the top N is a thin slice of the candidates and
-    // the candidate list has room for ~3N entries; everything else goes to the exact path.
-    if (8 * N > kCand || (int64_t)N * 16 > n_candidates || KB > 4 || n_users < 128) {
+    if (path == kPathExact || (path == kPathAuto && !sweep_applies(predictor, k, N, n_candidates, n_users))) {
         std::vector<int32_t> all;
         if (!users) {
             all.resize(n_users);
@@ -987,6 +1020,132 @@ extern "C" int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *M, int 
         stats[5] = (double)KB * 64;                                   // padded K the MMAs run over
         stats[6] = z;
         stats[7] = finish_ms;
+    }
+    return MFREC_OK;
+}
+
+}  // namespace
+
+extern "C" int mfrec_model_topn_sweep(mfrec_ctx *ctx, const mfrec_model *M, int predictor, const int32_t *users,
+                                      int32_t n_users, int32_t n_candidates, const int64_t *rated_indptr,
+                                      const int32_t *rated_items, double mu, double min_rating, double max_rating,
+                                      int32_t N, int32_t *out_items, double *out_scores, int32_t *out_counts,
+                                      double stats[8])
+{
+    return topn_sweep_on_model(ctx, M, predictor, users, n_users, n_candidates, rated_indptr, rated_items, mu,
+                               min_rating, max_rating, N, out_items, out_scores, out_counts, stats, kPathAuto);
+}
+
+// A user's result depends on that user and the item side only: the moments run on a fixed (ka, ka)
+// grid, z on N and n_candidates, thresholds / candidates / finish / certificate per user, and every
+// uncertified user is redone alone.  The one rule that spans users is the path choice, so it is made
+// here once, for the whole list, and every share takes that path whatever its size.
+extern "C" int mfrec_model_topn_sweep_multi(mfrec_ctx *const *ctxs, const mfrec_model *const *models, int n_shards,
+                                            int predictor, const int32_t *users, int32_t n_users, int32_t n_candidates,
+                                            const int64_t *rated_indptr, const int32_t *rated_items, double mu,
+                                            double min_rating, double max_rating, int32_t N, int32_t *out_items,
+                                            double *out_scores, int32_t *out_counts, double stats[8])
+{
+    const char *who = "mfrec_model_topn_sweep_multi";
+    MF_TRY(mfrec_check_shards(ctxs, models, n_shards, who));
+    mfrec_ctx *ctx = ctxs[0];
+    if (!out_items || !out_scores || !out_counts) return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "%s: NULL argument", who);
+    for (int s = 0; s < n_shards; ++s)
+        if (models[s]->user_perm || models[s]->item_perm)
+            return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "%s: shard %d: the model must be in identity layout (created without a ratings layout)",
+                                   who, s);
+    const int k = models[0]->k;
+    const int32_t ni = models[0]->ni, nu = models[0]->nu;
+    if (predictor < 0 || predictor > MFREC_PRED_DOT || n_users < 0 || N <= 0 || n_candidates < 0 || n_candidates > ni)
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "%s: predictor=%d n_users=%d N=%d n_candidates=%d", who, predictor,
+                               n_users, N, n_candidates);
+    if (users)
+        for (int32_t j = 0; j < n_users; ++j)
+            if (users[j] < 0 || users[j] >= nu)
+                return mfrec_set_error(ctx, MFREC_ERR_INDEX, "%s: user %d outside [0,%d)", who, users[j], nu);
+    if (!users && n_users > nu) return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "%s: n_users=%d > nu=%d", who, n_users, nu);
+    if (rated_indptr && n_users > 0 && rated_indptr[n_users] > 0 && !rated_items)
+        return mfrec_set_error(ctx, MFREC_ERR_BAD_ARG, "%s: rated_items is NULL", who);
+    const int path = sweep_applies(predictor, k, N, n_candidates, n_users) ? kPathSweep : kPathExact;
+    if (path == kPathSweep) {
+        // shards on one device run at the same time: each sweep CTA takes all 512 TMEM columns, so
+        // the launch configuration must keep it alone on its SM
+        const bool has_bias = predictor != MFREC_PRED_GD_RATING && predictor != MFREC_PRED_DOT;
+        const int KB = (k + (has_bias ? 1 : 0) + 63) / 64;
+        for (int s = 0; s < n_shards; ++s) {
+            MF_CUDA(ctx, cudaSetDevice(ctxs[s]->device));
+            int blocks = 0;
+            const int rc = KB == 1 ? sweep_ctas_per_sm<1, 4, 4>(ctx, &blocks)
+                         : KB == 2 ? sweep_ctas_per_sm<2, 4, 4>(ctx, &blocks)
+                         : KB == 3 ? sweep_ctas_per_sm<3, 2, 4>(ctx, &blocks)
+                                   : sweep_ctas_per_sm<4, 2, 2>(ctx, &blocks);
+            if (rc != MFREC_OK) return rc;
+            if (blocks != 1)
+                return mfrec_set_error(ctx, MFREC_ERR_UNSUPPORTED, "%s: %d sweep CTAs fit on one SM of device %d (each needs all of its tensor memory)",
+                                       who, blocks, ctxs[s]->device);
+        }
+    }
+    if (stats) memset(stats, 0, 8 * sizeof(double));
+    if (n_users == 0) return MFREC_OK;
+
+    // contiguous shares of near-equal count, cut at multiples of the 512-user sweep group where
+    // every shard still gets at least one group
+    constexpr int64_t kGroup = 512;
+    std::vector<int64_t> cut(n_shards + 1);
+    const int64_t n = n_users;
+    const int64_t n_groups = (n + kGroup - 1) / kGroup;
+    for (int s = 0; s <= n_shards; ++s)
+        cut[s] = n >= kGroup * n_shards ? std::min(n, n_groups * s / n_shards * kGroup) : n * s / n_shards;
+    std::vector<int32_t> iota;
+    if (!users) {
+        iota.resize(n_users);
+        for (int32_t j = 0; j < n_users; ++j) iota[j] = j;
+    }
+    const int32_t *uid = users ? users : iota.data();
+    std::vector<double> st((size_t)n_shards * 8, 0.0);
+    MF_TRY(mfrec_run_shards(ctxs, n_shards, who, [&](int s) -> int {
+        const int64_t a = cut[s], b = cut[s + 1];
+        if (a == b) return MFREC_OK;
+        // the share's rated CSR, rebased so that its indptr starts at 0
+        std::vector<int64_t> ip;
+        const int32_t *rated = nullptr;
+        if (rated_indptr) {
+            ip.resize(b - a + 1);
+            for (int64_t j = 0; j <= b - a; ++j) ip[j] = rated_indptr[a + j] - rated_indptr[a];
+            if (rated_items) rated = rated_items + rated_indptr[a];
+        }
+        return topn_sweep_on_model(ctxs[s], models[s], predictor, uid + a, (int32_t)(b - a), n_candidates,
+                                   rated_indptr ? ip.data() : nullptr, rated, mu, min_rating, max_rating, N,
+                                   out_items + a * N, out_scores + a * N, out_counts + a, &st[(size_t)s * 8], path);
+    }));
+    if (const char *path_env = getenv("MFREC_TOPN_SHARD_TIMES")) {   // debug: every shard's share and times
+        if (FILE *f = fopen(path_env, "a")) {
+            fprintf(f, "{\"path\": \"%s\", \"shards\": [", path == kPathSweep ? "sweep" : "exact");
+            for (int s = 0; s < n_shards; ++s) {
+                const double *x = &st[(size_t)s * 8];
+                fprintf(f, "%s{\"device\": %d, \"users\": [%lld, %lld], \"sweep_ms\": %.4f, \"finish_ms\": %.4f, \"redone\": %.0f}",
+                        s ? ", " : "", ctxs[s]->device, (long long)cut[s], (long long)cut[s + 1], x[2], x[7], x[0]);
+            }
+            fprintf(f, "]}\n");
+            fclose(f);
+        }
+    }
+    if (stats) {
+        double cand = 0.0;
+        for (int s = 0; s < n_shards; ++s) {
+            const int64_t ns = cut[s + 1] - cut[s];
+            if (ns == 0) continue;
+            const double *x = &st[(size_t)s * 8];
+            stats[0] += x[0];                          // users redone exactly
+            cand += x[1] * (double)ns;                 // candidates per user, weighted by the share's users
+            stats[2] = std::max(stats[2], x[2]);       // sweep ms: the slowest shard
+            stats[3] += x[3];                          // useful FLOPs
+            stats[4] += x[4];                          // overflowed candidate lists
+            stats[5] = x[5];                           // padded K and z: the same on every shard
+            stats[6] = x[6];
+            stats[7] = std::max(stats[7], x[7]);       // finish ms: the slowest shard
+        }
+        stats[1] = cand / (double)n_users;
     }
     return MFREC_OK;
 }

@@ -3,7 +3,7 @@
 import numpy as np
 
 from mfrec_b200 import _native
-from mfrec_b200.lib._buffers import buffer_arg
+from mfrec_b200.lib._buffers import buffer_arg, options
 from mfrec_b200.recommendation.base import BaseRecommender
 
 
@@ -83,13 +83,18 @@ class MFRecommender(BaseRecommender):
         """``mfrec_model`` of the current factors in identity layout, uploaded once and reused by
         predict / RMSE / top-N calls until the arrays change (their address, shape or sampled
         contents): ``test_predict_rating(nbr_samples=10)`` or one ``find_recommended_items`` call no
-        longer moves 0.5 GB of factors at Netflix shape."""
-        key = tuple(_native.array_fingerprint(a) for a in (self.svd_u, self.svd_v, self.items_bias, self.users_bias))
+        longer moves 0.5 GB of factors at Netflix shape.  With more than one entry in
+        ``options["devices"]`` it is a ``_native.ModelSet`` (one copy per listed device): batched top-N
+        and predictions are split over them, with the one-device results."""
+        devices = _serve_devices()
+        key = (devices,) + tuple(_native.array_fingerprint(a)
+                                 for a in (self.svd_u, self.svd_v, self.items_bias, self.users_bias))
         cached = getattr(self, '_model_cache', None)
         if cached is not None and cached[0] == key:
             return cached[1]
         k, ni = self.svd_u.shape
-        model = _native.Model(k, ni, self.svd_v.shape[1], self.svd_u, self.svd_v, self.items_bias, self.users_bias)
+        args = (k, ni, self.svd_v.shape[1], self.svd_u, self.svd_v, self.items_bias, self.users_bias)
+        model = _native.ModelSet(devices, *args) if devices else _native.Model(*args)
         self._model_cache = (key, model)
         return model
 
@@ -155,23 +160,26 @@ class MFRecommender(BaseRecommender):
         row of the similarity matrix is one top-N query.  cosine / Pearson: rows (centred for Pearson)
         scaled to unit length, score = dot.  euclidean: item side -2 x_i with bias |x_i|^2, user side
         x_q with bias |x_q|^2, so the linear predictor gives |x_i - x_q|^2.  Cached per (rows,
-        method): repeated queries upload nothing."""
-        key = (tag, method, _native.array_fingerprint(rows))
+        method, devices): repeated queries upload nothing.  Several devices in ``options["devices"]``:
+        a ``_native.ModelSet``, as for ``_resident_model``."""
+        devices = _serve_devices()
+        key = (tag, method, devices, _native.array_fingerprint(rows))
         cache = getattr(self, '_sim_cache', None)
         if cache is not None and cache[0] == key:
             return cache[1]
         x = np.array(rows, dtype=np.float64)
         if method == 'euclidean':
             sq = (x * x).sum(axis=1)
-            model = _native.Model(x.shape[1], x.shape[0], x.shape[0], np.ascontiguousarray(-2.0 * x.T),
-                                  np.ascontiguousarray(x.T), sq, sq)
+            args = (x.shape[1], x.shape[0], x.shape[0], np.ascontiguousarray(-2.0 * x.T), np.ascontiguousarray(x.T),
+                    sq, sq)
         else:
             if method == 'pearson':
                 x = x - x.mean(axis=1, keepdims=True)
             norm = np.sqrt((x * x).sum(axis=1, keepdims=True))
             x = np.divide(x, norm, out=np.zeros_like(x), where=norm > 0)
             xt = np.ascontiguousarray(x.T)                  # [d, n]: "item factors" and "user factors"
-            model = _native.Model(x.shape[1], x.shape[0], x.shape[0], xt, xt, None, None)
+            args = (x.shape[1], x.shape[0], x.shape[0], xt, xt, None, None)
+        model = _native.ModelSet(devices, *args) if devices else _native.Model(*args)
         self._sim_cache = (key, model)
         return model
 
@@ -242,6 +250,13 @@ class MFRecommender(BaseRecommender):
             if getattr(type(self), name, None) is target:
                 return name
         raise KeyError(predictor)
+
+
+def _serve_devices():
+    """The devices predictions and top-N are served from: ``options["devices"]`` when it lists more than
+    one (a ``_native.ModelSet``), else () (one ``_native.Model`` on the default context)."""
+    devices = tuple(int(d) for d in options["devices"])
+    return devices if len(devices) > 1 else ()
 
 
 # ---- batched fold-in: argument checks shared by KMFRecommender and GDRecommender ------------------

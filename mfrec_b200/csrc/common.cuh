@@ -309,6 +309,9 @@ static inline int mfrec_kpad(int k)
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// most shards one call of a multi-shard entry point takes (ALS training, serving)
+constexpr int kMaxShards = 16;
+
 // sgd.cu
 size_t mfrec_sgd_smem_bytes(int tile_rows, int kpad, int W, int p_elem_bytes = 4);
 
@@ -351,10 +354,9 @@ int mfrec_download_vec(mfrec_ctx *ctx, const float *src, int32_t n, const int32_
                        double *host);
 
 // runtime.cu: serving from several shards of one process (mfrec_model_topn_sweep_multi,
-// mfrec_model_predict_multi).  mfrec_check_shards: 1 <= n_shards <= kMaxServeShards, no NULL entry,
+// mfrec_model_predict_multi).  mfrec_check_shards: 1 <= n_shards <= kMaxShards, no NULL entry,
 // every context distinct, each model on its context's device, equal k / kpad / ni / nu / storage;
 // errors on ctxs[0].  mfrec_run_shards: fn(s) for every shard, each on a host thread of its own
 // (shard 0 on the caller's); the first failing shard's status, its message copied to ctxs[0].
-constexpr int kMaxServeShards = 16;
 int mfrec_check_shards(mfrec_ctx *const *ctxs, const mfrec_model *const *models, int n_shards, const char *who);
 int mfrec_run_shards(mfrec_ctx *const *ctxs, int n_shards, const char *who, const std::function<int(int)> &fn);

@@ -612,8 +612,8 @@ int mfrec_check_shards(mfrec_ctx *const *ctxs, const mfrec_model *const *models,
     mfrec_ctx *c0 = ctxs && n_shards >= 1 ? ctxs[0] : nullptr;
     if (!ctxs || !models || n_shards < 1)
         return mfrec_set_error(c0, MFREC_ERR_BAD_ARG, "%s: no shards (n_shards=%d)", who, n_shards);
-    if (n_shards > kMaxServeShards)
-        return mfrec_set_error(c0, MFREC_ERR_UNSUPPORTED, "%s: %d shards, at most %d", who, n_shards, kMaxServeShards);
+    if (n_shards > kMaxShards)
+        return mfrec_set_error(c0, MFREC_ERR_UNSUPPORTED, "%s: %d shards, at most %d", who, n_shards, kMaxShards);
     for (int s = 0; s < n_shards; ++s) {
         if (!ctxs[s] || !models[s]) return mfrec_set_error(c0, MFREC_ERR_BAD_ARG, "%s: shard %d: NULL context or model", who, s);
         for (int t = 0; t < s; ++t)

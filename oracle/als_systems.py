@@ -183,7 +183,7 @@ def check_half_pass(X_fixed, Y_before, Y_after, row, col, c_pos, reg, nbr_rows, 
 
 
 # ---- the device's row-solver layout ------------------------------------------------------------------
-# A restatement of als_layout in mfrec_b200/csrc/als.cu (lines 511-539 when this was written) and of the
+# A restatement of als_layout in mfrec_b200/csrc/als.cu (lines 480-508 when this was written) and of the
 # sizes it uses (als_pitch, als_cluster_pitch, als_cluster_smem): from k and the device's shared memory
 # it picks C, the CTAs per row (1: als_solve_kernel, more: als_cluster_solve_kernel), and kTile, the
 # neighbour rows staged per step.  Keep the two in step.

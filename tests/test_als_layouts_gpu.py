@@ -141,8 +141,8 @@ def test_deterministic(k):
 
 @pytest.mark.parametrize("k", [72, 220, 232])
 def test_three_shards_on_one_device_bit_identical(k):
-    """The multi-shard kernels (als_solve_multi_kernel, als_cluster_solve_multi_kernel) in the layouts
-    no earlier test ran, against the one-device call."""
+    """Three shards on one device, each solution stored into three copies, in the layouts no earlier
+    test ran, against the one-device call (one shard, one copy)."""
     from mfrec_b200 import _native
     d = _device()
     p = A.implicit_problem(k, 300, 200, 4000, seed=k + 3, degrees=_edges(k), hot=60, duplicate=True)
